@@ -4,6 +4,11 @@ the metric (3D elasticity, config 5), strong scaling of both, and the smaller co
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (SciPy port)
+    python bench.py ... --dump-outputs DIR                   # also save a fixed sample of the computed field
+
+--dump-outputs DIR writes the temperature field the timed steps left in HBM (the state a caller of the stepper reads
+back), sampled at fixed, seeded vertex indices, as DIR/heat_temperature.npy (float64), so that two builds can be
+compared output for output: with the same arguments the inputs and the sampled indices are the same on every run.
 
 One "step" = one backward-Euler time step (a full linear solve to rtol 1e-10) of the heat equation on the
 unit-cube-per-GPU 512^3 P1 mesh (135 M dofs per GPU; weak scaling stacks slabs along z).
@@ -49,6 +54,8 @@ ELAST_STEP_BYTES = 80.0 + 122.0 * 8.0 / 7.0
 ELAST_STEP_BYTES_R1 = 80.0 + 146.0 * 8.0 / 7.0
 SWEEP_BYTES = {0: 16, 1: 24, 2: 24, 3: 32}
 SWEEP_NAME = {0: "apply (+fused dots)", 1: "residual", 2: "chebyshev sweep (restart)", 3: "chebyshev sweep (with x_prev)"}
+DUMP_SAMPLES = 1 << 21          # --dump-outputs: vertices kept of the 135 M of heat3d_512 (16 MB of float64)
+DUMP_SEED = 20261020
 
 
 def measured_peaks():
@@ -310,6 +317,28 @@ def run_native(args):
                         "frac": ach / peak})
         return out, nd
 
+    def dump_field(name, local, n):
+        """Sample a nodal field held as z-slabs (this rank's part of the natural vertex order) at fixed, seeded global
+        vertex indices; rank 0 writes the sample as DIR/<name>.npy."""
+        plane = (n[0] + 1) * (n[1] + 1)
+        nglob = plane * (n[2] + 1)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(nglob, min(DUMP_SAMPLES, nglob), replace=False))
+        z0, nzl, _ = _lib.slab_partition(3, n, rank, world)
+        if local.size != nzl * plane:
+            raise RuntimeError(f"rank {rank} holds {local.size} vertices, its slab has {nzl * plane}")
+        lo = z0 * plane
+        mine = (idx >= lo) & (idx < lo + local.size)
+        vals = np.zeros(idx.size)
+        vals[mine] = local[idx[mine] - lo]
+        if dist is not None:          # each index lies in exactly one slab, so the sum over ranks is exact
+            import torch
+            t = torch.from_numpy(vals).cuda()
+            dist.all_reduce(t)
+            vals = t.cpu().numpy()
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), vals)
+
     # ---- 1. headline: heat, weak scaling (inputs resident in HBM) ----
     n_w = [w["n"][0], w["n"][1], w["n"][2] * world]
     L_w = [1.0, 1.0, 1.0 * world]
@@ -336,7 +365,9 @@ def run_native(args):
     # the upload of request k+1 and the download of result k-1 run on copy streams while request k is solved.
     # (2) serial, for comparison: set_state / step / get_state, the result being the next step's input.
     hbuf = _lib.PinnedArray(hs.nloc)
-    hs.get_state(hbuf.array)
+    hs.get_state(hbuf.array)                            # the state after the timed steps
+    if args.dump_outputs:
+        dump_field("heat_temperature", hbuf.array, n_w)
     e_steps = max(1, args.steps)
     h_in = [_lib.PinnedArray(hs.nloc) for _ in range(2)]
     h_out = [_lib.PinnedArray(hs.nloc) for _ in range(2)]
@@ -539,7 +570,13 @@ def _main(emit_restore):
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-cg-leg", action="store_true")
     ap.add_argument("--cg-cells", type=int, default=128)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of the field the timed steps computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
     if args.warmup < 3 and args.impl == "native":
         args.warmup = 3
     args.emit_restore = emit_restore

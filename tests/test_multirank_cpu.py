@@ -159,11 +159,12 @@ def test_requested_gpus_beyond_the_visible_devices_is_refused(monkeypatch):
 
 def test_tool_pool_reports_a_rank_without_a_device_instead_of_hanging(monkeypatch):
     """Pool start-up handshake: every worker says whether it holds a device context BEFORE rank 0 enters the NCCL
-    communicator set-up.  Here (no GPU) the spawned rank cannot create its context: the pool must raise with the rank's
-    own message and reap the worker - not block in the collective."""
+    communicator set-up.  Here the spawned rank sees no GPU and cannot create its context: the pool must raise with the
+    rank's own message and reap the worker - not block in the collective."""
     import time
 
     from pde_solver_b200 import _lib, multi
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")          # the worker inherits it, also on a machine with GPUs
 
     class FakeContext:                       # rank 0 'has' a device; its comm_init must never be reached
         def __init__(self, device):
