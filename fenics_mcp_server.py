@@ -256,7 +256,7 @@ def solve_heat_3D_spherical(
         r_inner=r_inner, r_outer=r_outer, nr=nr, ntheta=ntheta, nphi=nphi, diffusivity=diffusivity,
         T_boundary=T_boundary, T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"])
+        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
     return _save(field, data_dir, "heat_3d_spherical")
 
 
@@ -272,7 +272,7 @@ def solve_heat_1D_cylindrical(
         r_inner=r_inner, r_outer=r_outer, nr=nr, diffusivity=diffusivity, T_inner=T_inner, T_outer=T_outer,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"])
+        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
     return _save(field, data_dir, "heat_1d_cylindrical")
 
 
@@ -288,7 +288,7 @@ def solve_heat_1D_spherical(
         r_inner=r_inner, r_outer=r_outer, nr=nr, diffusivity=diffusivity, T_inner=T_inner, T_outer=T_outer,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"])
+        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
     return _save(field, data_dir, "heat_1d_spherical")
 
 
@@ -304,7 +304,7 @@ def solve_heat_2D_cylindrical(
         r_inner=r_inner, r_outer=r_outer, z_length=z_length, nr=nr, nz=nz, diffusivity=diffusivity,
         T_boundary=T_boundary, T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"])
+        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
     return _save(field, data_dir, "heat_2d_cylindrical")
 
 
@@ -320,7 +320,7 @@ def solve_heat_2D_spherical(
         r_inner=r_inner, r_outer=r_outer, nr=nr, ntheta=ntheta, diffusivity=diffusivity, T_boundary=T_boundary,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"])
+        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
     return _save(field, data_dir, "heat_2d_spherical")
 
 

@@ -196,8 +196,18 @@ typedef struct pde_wheat_params {
   double initial_amplitude;
   double initial_wavenumber;
 } pde_wheat_params;
+/* o->precond: PDE_PRECOND_GMG runs GMG-PCG with Galerkin coarse operators (P^T A P) while every axis halves evenly;
+ * st->levels and st->true_relres (||b - A x||/||b|| of the last solve, full assembled stencil) are filled.  A grid
+ * with an odd cell count falls back to Jacobi-PCG (levels = 1).  PDE_PRECOND_JACOBI and PDE_PRECOND_AUTO run
+ * Jacobi-PCG (true_relres = NaN). */
 int pde_wheat_solve(pde_ctx* ctx, const pde_wheat_params* p, const pde_solver_opts* o,
                     double* values_out /* [nsnap][nverts] */, double* times_out, pde_stats* st);
+/* Operator of multigrid level `level` of the GMG path: n_out = cells per user axis of that level (0 for absent axes),
+ * coef_out = [nk][nverts] in natural vertex order, nk = 3 / 7 / 15 (1-D / 2-D / 3-D): entry [k][i] = a(i, i + d_k)
+ * with d_k the Kuhn offsets in internal axes (x, y, z; 2-D: x, z) in the order {0, +x, -x, +y, -y, +z, -z, +xy, -xy,
+ * +xz, -xz, +yz, -yz, +xyz, -xyz} restricted to the present axes.  Rows and columns of Dirichlet vertices are zero.
+ * coef_out = NULL only fills n_out.  Non-zero if the level does not exist. */
+int pde_wheat_level_coefs(pde_ctx* ctx, const pde_wheat_params* p, int level, int32_t n_out[3], double* coef_out);
 
 /* ---- elasticity: _solve_elasticity_{1,2,3}d_static :1470-1587, 1593-1743, 1749-1892 ---- */
 typedef struct pde_elast_params {

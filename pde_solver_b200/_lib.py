@@ -94,7 +94,7 @@ def lib():
                      "pde_heat_open", "pde_heat_set_state", "pde_heat_step", "pde_heat_get_state",
                      "pde_heat_advance_batch", "pde_halo_check",
                      "pde_heat_close", "pde_elasticity_solve", "pde_op_table", "pde_op_apply", "pde_op_bench", "pde_op_sweep", "pde_op_bench_mode", "pde_comm_info", "pde_device_count",
-                     "pde_op_solve", "pde_version", "pde_host_alloc", "pde_host_free", "pde_slab_partition", "pde_op_manufactured", "pde_halo_bench", "pde_wheat_solve",
+                     "pde_op_solve", "pde_version", "pde_host_alloc", "pde_host_free", "pde_slab_partition", "pde_op_manufactured", "pde_halo_bench", "pde_wheat_solve", "pde_wheat_level_coefs",
                      "pde_mesh_coords_box"):
             getattr(L, name).restype = C.c_int
         _lib = L

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libpde_b200.so")
-SOURCES = ["tables.cpp", "kernels.cu", "stencil3d.cu", "elast3d.cu", "heat2.cu", "solver.cu", "weighted.cu", "comm.cu", "cabi.cu"]
+SOURCES = ["tables.cpp", "kernels.cu", "stencil3d.cu", "elast3d.cu", "heat2.cu", "solver.cu", "weighted.cu", "wmg.cu", "comm.cu", "cabi.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"] + os.environ.get("PDE_B200_NVCC_FLAGS", "").split()
 

@@ -157,9 +157,7 @@ int project_trig_ic(pde_ctx* c, const Grid& g, const BcDev& bc, int dim, const i
 }
 
 // ---- multigrid ---------------------------------------------------------------------------------
-#define PDE_DENSE_MAX 768
-
-static long long count_free_and_index(const Grid& g, const BcDev& bc, int ncomp, std::vector<long long>* idx,
+long long count_free_and_index(const Grid& g, const BcDev& bc, int ncomp, std::vector<long long>* idx,
                                       std::vector<int>* dofid) {
   long long n = 0;
   if (dofid) dofid->assign((size_t)g.nn[0] * g.nn[1] * g.nzl * ncomp, -1);
@@ -177,7 +175,7 @@ static long long count_free_and_index(const Grid& g, const BcDev& bc, int ncomp,
   return n;
 }
 
-static int dense_inverse_spd(std::vector<double>& A, int n) {
+int dense_inverse_spd(std::vector<double>& A, int n) {
   // Cholesky A = L L^T (in place, lower), then A^-1 = L^-T L^-1
   for (int j = 0; j < n; ++j) {
     double d = A[(size_t)j * n + j];

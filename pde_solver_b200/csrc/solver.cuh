@@ -73,4 +73,11 @@ int project_trig_ic(pde_ctx* c, const Grid& g, const BcDev& bc, int dim, const i
                     const double* lo_user, double amp, double kw, int use_sin, const pde_solver_opts& o, double* u,
                     double* rhs);
 int read_scal(pde_ctx* c, int slot, int count, double* out);
+// coarsest multigrid levels with at most this many free dofs are solved with a dense inverse
+#define PDE_DENSE_MAX 768
+// free dofs of a grid; idx: their flat field indices, dofid: node -> dof number (-1: Dirichlet)
+long long count_free_and_index(const Grid& g, const BcDev& bc, int ncomp, std::vector<long long>* idx,
+                               std::vector<int>* dofid);
+// in-place inverse of a dense SPD matrix (Cholesky); non-zero if it is not positive definite
+int dense_inverse_spd(std::vector<double>& A, int n);
 int choose_precond(const pde_solver_opts& o, pde_ctx* c, long long ndofs, const Hierarchy& h);

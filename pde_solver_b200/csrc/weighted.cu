@@ -6,17 +6,20 @@
 // cell and integrates exactly; the weight is separable, so its vertex / edge-midpoint values come from one table
 // per axis on the half-step lattice.  The operator is no longer a constant stencil: k_wassemble writes the 15
 // (7 / 3) stencil coefficients of every node once, k_vapply applies them, and a Jacobi-PCG with device-side
-// scalars solves the systems (these tools run modest grids; multigrid is not needed).
+// scalars solves the systems.  Jacobi needs O(1/h) iterations, so precond = GMG switches to Galerkin multigrid
+// (wmg.cu: symmetric half-coefficient storage, P^T A P coarse operators) when every axis halves evenly; the full
+// stencil stays allocated for the true residual of that path.
 //
 // The cylinder / composite-core branches of _solve_heat_3d_raw (:512-572, 642-645) run through the same kernels: the
 // reference's deployment has no mshr (neither Dockerfile nor requirements.txt install it), so its "cylinder" is
 // BoxMesh((0,-R,-R),(Lx,R,R)) with every term weighted by Expression("sqrt(x[1]^2+x[2]^2)", degree=2)
 // (weight_kind 1: not separable, evaluated from the y/z coordinate tables), and a composite core is a DG0
 // diffusivity: core_diffusivity on the cells whose vertices and midpoint all have sqrt(y^2+z^2) < core_radius.
+#include <chrono>
 #include <cmath>
 #include <cstring>
 
-#include "solver.cuh"
+#include "wmg.cuh"
 
 struct WeightInts {
   int nk, nv;          // weight basis functions (P1: nv, P2: nv + edges), simplex vertices
@@ -322,9 +325,8 @@ static int wpcg(WheatState& s, double bn2, const pde_solver_opts& o, pde_stats* 
   return 0;
 }
 
-extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o_in, double* values_out,
-                               double* times_out, pde_stats* st_out) {
-  if (!c || !p || !values_out || !times_out) PDE_FAIL("null argument");
+// validates p, lays out the grid (L: user box lengths) and assembles coefA / coefM / loadv into s
+static int wheat_assemble(pde_ctx* c, const pde_wheat_params* p, WheatState& s, double L[3]) {
   if (c->world > 1) PDE_FAIL("pde_wheat_solve: the curvilinear tools run on one GPU");
   CUDA_OK(cudaSetDevice(c->device));
   if (p->dim < 1 || p->dim > 3) PDE_FAIL("dim must be 1, 2 or 3");
@@ -335,14 +337,11 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
   if (p->has_core && !(p->core_diffusivity > 0)) PDE_FAIL("core_diffusivity must be > 0");
   if (!p->steady && !(p->dt > 0)) PDE_FAIL("dt must be > 0");
   if (!(p->diffusivity > 0)) PDE_FAIL("diffusivity must be > 0");
-  pde_solver_opts o;
-  if (o_in) o = *o_in; else pde_solver_opts_default(&o);
-  double L[3] = {1, 1, 1};
+  for (int k = 0; k < 3; ++k) L[k] = 1.0;
   for (int k = 0; k < p->dim; ++k) {
     L[k] = p->hi[k] - p->lo[k];
     if (!(L[k] > 0)) PDE_FAIL("hi must exceed lo on every axis");
   }
-  WheatState s;
   s.c = c;
   PDE_OK(make_grid(p->dim, p->n, L, 0, 1, &s.g));
   user_bc_to_dev(p->dim, &p->bc, &s.bc);
@@ -380,7 +379,7 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
   build_simplex_geom(p->dim, g.h, &sg);
   WeightInts wi;
   build_weight_ints(p->dim, p->weight_degree, &wi);
-  const double kappa = p->diffusivity, f = p->source_value;
+  const double kappa = p->diffusivity;
   const double alpha = p->steady ? 0.0 : 1.0, beta = p->steady ? kappa : p->dt * kappa;
   RowLaunch rl = row_launch(c, g);
   k_wassemble<<<rl.grid, rl.block, 0, c->stream>>>(g, sg, wi, alpha, beta, tabs[0], tabs[1] ? tabs[1] : tabs[0],
@@ -390,11 +389,42 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
                                                    s.coefA.p, s.coefM.p, s.loadv.p);
   c->launches++;
   CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o_in, double* values_out,
+                               double* times_out, pde_stats* st_out) {
+  if (!c || !p || !values_out || !times_out) PDE_FAIL("null argument");
+  pde_solver_opts o;
+  if (o_in) o = *o_in; else pde_solver_opts_default(&o);
+  WheatState s;
+  double L[3];
+  PDE_OK(wheat_assemble(c, p, s, L));
+  const Grid& g = s.g;
+  const double f = p->source_value;
+  // GMG only on request (PDE_PRECOND_AUTO keeps Jacobi here); a grid that does not coarsen runs Jacobi
+  WHierarchy mg;
+  bool use_mg = false;
+  double setup_ms = 0.0;
+  if (o.precond == PDE_PRECOND_GMG) {
+    CUDA_OK(cudaStreamSynchronize(c->stream));
+    const auto t0 = std::chrono::steady_clock::now();
+    PDE_OK(mg.build(c, g, s.bc, s.coefA.p));
+    CUDA_OK(cudaStreamSynchronize(c->stream));
+    setup_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    use_mg = mg.levels() >= 2;
+    if (!use_mg) mg.release();
+  }
   pde_stats st;
   std::memset(&st, 0, sizeof(st));
   st.ndofs = (long long)g.nn[0] * g.nn[1] * g.nzg;
   st.converged = 1;
   st.true_relres = NAN;
+  st.setup_ms = setup_ms;
+  const bool verify = use_mg && o.verify_residual >= 0;
+  auto solve = [&](double bn2) -> int {
+    return use_mg ? wmg_pcg(c, mg, s.u.p, s.r.p, s.p.p, s.q.p, bn2, o, &st) : wpcg(s, bn2, o, &st);
+  };
   const long long nloc = st.ndofs;
   double* dense = nullptr;
   CUDA_OK(cudaMalloc(&dense, sizeof(double) * nloc));
@@ -417,12 +447,21 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
     PDE_OK(launch_fill_ic(c, g, s.bc, s.u.p, v0, 1));
   }
   long long snap = 0;
+  // GMG path: ||b - A x|| / ||b|| of the last solve with the full assembled stencil (also checks the packed operator)
+  Field un;
+  struct UnRel { Field* f; ~UnRel() { f->release(); } } unrel{&un};
   if (p->steady) {
     // r0 = f m_w - k K_w u_lift  (A = k K_w)
     PDE_OK(vapply(s, s.coefA, s.u.p, s.r.p, 0.0, -1.0, f, S_XY));
     double bn2;
     PDE_OK(read_scal(c, S_YY, 1, &bn2));
-    PDE_OK(wpcg(s, bn2, o, &st));
+    PDE_OK(solve(bn2));
+    if (verify) {
+      PDE_OK(vapply(s, s.coefA, s.u.p, s.q.p, 0.0, -1.0, f, S_XY));
+      double rr;
+      PDE_OK(read_scal(c, S_YY, 1, &rr));
+      st.true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
+    }
     PDE_OK(snapshot(values_out));
     times_out[0] = 0.0;
   } else {
@@ -430,12 +469,24 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
     times_out[snap++] = 0.0;
     const int stride = p->snapshot_stride > 0 ? p->snapshot_stride : 1;
     for (int step = 0; step < p->num_steps; ++step) {
+      const bool last = verify && step == p->num_steps - 1;
+      if (last) {
+        PDE_OK(un.alloc(c, g, 1));
+        PDE_OK(launch_copy(c, g, 1, un.p, s.u.p));
+      }
       // b = M_w u_n + dt f m_w (its norm is the stopping scale); warm start x0 = u_n: r0 = b - A u_n
       PDE_OK(vapply(s, s.coefM, s.u.p, s.r.p, 0.0, 1.0, p->dt * f, S_XY));
       double bn2;
       PDE_OK(read_scal(c, S_YY, 1, &bn2));
       PDE_OK(vapply(s, s.coefA, s.u.p, s.r.p, 1.0, -1.0, 0.0, -1));
-      PDE_OK(wpcg(s, bn2, o, &st));
+      PDE_OK(solve(bn2));
+      if (last) {
+        PDE_OK(vapply(s, s.coefM, un.p, s.q.p, 0.0, 1.0, p->dt * f, -1));
+        PDE_OK(vapply(s, s.coefA, s.u.p, s.q.p, 1.0, -1.0, 0.0, S_XY));
+        double rr;
+        PDE_OK(read_scal(c, S_YY, 1, &rr));
+        st.true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
+      }
       if ((step + 1) % stride == 0) {
         PDE_OK(snapshot(values_out + snap * nloc));
         times_out[snap++] = (step + 1) * p->dt;
@@ -449,5 +500,19 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
   st.solve_ms = ms;
   st.launches = c->launches - l0;
   if (st_out) *st_out = st;
+  return 0;
+}
+
+extern "C" int pde_wheat_level_coefs(pde_ctx* c, const pde_wheat_params* p, int level, int32_t n_out[3],
+                                     double* coef_out) {
+  if (!c || !p || !n_out) PDE_FAIL("null argument");
+  WheatState s;
+  double L[3];
+  PDE_OK(wheat_assemble(c, p, s, L));
+  WHierarchy mg;
+  PDE_OK(mg.build(c, s.g, s.bc, s.coefA.p));
+  if (level < 0 || level >= mg.levels()) PDE_FAIL("no such multigrid level");
+  for (int q = 0; q < 3; ++q) n_out[q] = q < p->dim ? p->n[q] >> level : 0;
+  if (coef_out) PDE_OK(wmg_level_coefs(c, mg, level, coef_out));
   return 0;
 }

@@ -194,7 +194,7 @@ def _solve_heat_3d_raw(Lx: float, Ly: float, Lz: float, nx: int, ny: int, nz: in
         return _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady,
                                 source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
                                 geometry_type, cylinder_radius, T_left, T_right, T_side, core_radius,
-                                core_diffusivity, rtol, snapshot_stride, as_arrays)
+                                core_diffusivity, rtol, snapshot_stride, as_arrays, precond)
     bc = mesh.heat_bc(3, T_boundary=T_boundary, T_left=T_left, T_right=T_right, T_side=T_side)
     coords, values, times = _heat(3, [Lx, Ly, Lz], [nx, ny, nz], diffusivity, T_initial, dt, num_steps, steady,
                                   source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
@@ -217,7 +217,7 @@ def _solve_heat_3d_raw(Lx: float, Ly: float, Lz: float, nx: int, ny: int, nz: in
 def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady, source_type,
                      source_value, initial_type, initial_amplitude, initial_wavenumber, geometry_type,
                      cylinder_radius, T_left, T_right, T_side, core_radius, core_diffusivity, rtol, snapshot_stride,
-                     as_arrays, ctx=None):
+                     as_arrays, precond="jacobi", ctx=None):
     """Cylinder / composite-core branches of _solve_heat_3d_raw (:512-572, 576-605, 642-645) as the reference's
     deployment runs them (no mshr in Dockerfile / requirements.txt, so MSHR_AVAILABLE is False): the "cylinder" is
     BoxMesh((0,-R,-R),(Lx,R,R), nx, int(ny*2R), int(nz*2R)) with every term weighted by
@@ -271,7 +271,7 @@ def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial,
     values = np.empty((nsnap, nv), dtype=np.float64)
     times = np.empty(nsnap, dtype=np.float64)
     st = _lib.Stats()
-    o = _lib.make_opts(rtol=rtol, precond="jacobi")
+    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
     _lib.check(_lib.lib().pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
                                           C.byref(st)))
     _record(st.as_dict(), "heat solve (weighted box)")
@@ -379,8 +379,15 @@ _CURVI = {
 }
 
 
+def _wheat_precond(precond):
+    """Weighted operators: "gmg" selects Galerkin multigrid; "auto" still means Jacobi-PCG for them."""
+    if precond not in _lib.PRECOND:
+        raise ValueError(f"precond must be one of {sorted(_lib.PRECOND)}, got {precond!r}")
+    return "gmg" if precond == "gmg" else "jacobi"
+
+
 def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                 snapshot_stride=1, ctx=None):
+                 snapshot_stride=1, ctx=None, precond="jacobi"):
     ctx = ctx or _lib.default_context()
     dim, rpow, wsin, wdeg = _CURVI[kind]
     p = _lib.WheatParams()
@@ -402,7 +409,7 @@ def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, ste
     values = np.empty((nsnap, nv), dtype=np.float64)
     times = np.empty(nsnap, dtype=np.float64)
     st = _lib.Stats()
-    o = _lib.make_opts(rtol=rtol, precond="jacobi")
+    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
     _lib.check(_lib.lib().pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
                                           C.byref(st)))
     _record(st.as_dict(), "curvilinear heat solve")
@@ -429,10 +436,12 @@ def _solve_heat_1d_cylindrical_raw(r_inner: float, r_outer: float, nr: int, diff
                                    T_outer: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                    source_type: str = "none", source_value: float = 0.0,
                                    initial_type: str = "constant", initial_amplitude: float = 1.0, *,
-                                   rtol: float = 1e-10, as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                   rtol: float = 1e-10, precond: str = "jacobi",
+                                   as_arrays: Optional[bool] = None) -> TimeSeriesField:
     """1D radial heat equation in cylindrical coordinates, weight r (:769-920)."""
     X, values, times = _curvilinear("1d_cylindrical", [r_inner], [r_outer], [nr], _radial_bc(r_inner, T_inner, T_outer),
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol)
+                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    precond=precond)
     order = np.argsort(X[:, 0], kind="stable")
     meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annulus", r_inner, r_outer, source_type,
                        source_value, steady)
@@ -442,11 +451,12 @@ def _solve_heat_1d_cylindrical_raw(r_inner: float, r_outer: float, nr: int, diff
 def _solve_heat_1d_spherical_raw(r_inner: float, r_outer: float, nr: int, diffusivity: float, T_inner: float,
                                  T_outer: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
-                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10,
+                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
                                  as_arrays: Optional[bool] = None) -> TimeSeriesField:
     """1D radial heat equation in spherical coordinates, weight r^2 (:926-1057)."""
     X, values, times = _curvilinear("1d_spherical", [r_inner], [r_outer], [nr], _radial_bc(r_inner, T_inner, T_outer),
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol)
+                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    precond=precond)
     order = np.argsort(X[:, 0], kind="stable")
     meta = _curvi_meta("spherical", "sphere" if r_inner < 1e-10 else "spherical_shell", r_inner, r_outer, source_type,
                        source_value, steady)
@@ -457,11 +467,13 @@ def _solve_heat_2d_cylindrical_raw(r_inner: float, r_outer: float, z_length: flo
                                    diffusivity: float, T_boundary: float, T_initial: float, dt: float, num_steps: int,
                                    steady: bool = False, source_type: str = "none", source_value: float = 0.0,
                                    initial_type: str = "constant", initial_amplitude: float = 1.0, *,
-                                   rtol: float = 1e-10, as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                   rtol: float = 1e-10, precond: str = "jacobi",
+                                   as_arrays: Optional[bool] = None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, z) plane, weight r (:1063-1185)."""
     bc = _lib.make_bc({f: T_boundary for f in range(4)})
     X, values, times = _curvilinear("2d_cylindrical", [r_inner, 0.0], [r_outer, z_length], [nr, nz], bc, diffusivity,
-                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol)
+                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    precond=precond)
     coords = np.zeros((X.shape[0], 3))
     coords[:, 0], coords[:, 2] = X[:, 0], X[:, 1]                 # (r, 0, z)
     meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annular_cylinder", r_inner, r_outer,
@@ -472,12 +484,13 @@ def _solve_heat_2d_cylindrical_raw(r_inner: float, r_outer: float, z_length: flo
 def _solve_heat_2d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta: int, diffusivity: float,
                                  T_boundary: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
-                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10,
+                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
                                  as_arrays: Optional[bool] = None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, theta) plane, weight r^2 sin(theta) (:1191-1320)."""
     bc = _lib.make_bc({f: T_boundary for f in range(4)})
     X, values, times = _curvilinear("2d_spherical", [r_inner, 0.0], [r_outer, float(np.pi)], [nr, ntheta], bc,
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol)
+                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    precond=precond)
     coords = np.zeros((X.shape[0], 3))
     coords[:, 0] = X[:, 0] * np.sin(X[:, 1])                      # phi = 0: (r sin(theta), 0, r cos(theta))
     coords[:, 2] = X[:, 0] * np.cos(X[:, 1])
@@ -489,13 +502,13 @@ def _solve_heat_2d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta
 def _solve_heat_3d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta: int, nphi: int, diffusivity: float,
                                  T_boundary: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
-                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10,
+                                 initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
                                  as_arrays: Optional[bool] = None) -> TimeSeriesField:
     """3D heat equation in (r, theta, phi), weight r^2 sin(theta) (:1326-1464)."""
     bc = _lib.make_bc({f: T_boundary for f in range(6)})
     X, values, times = _curvilinear("3d_spherical", [r_inner, 0.0, 0.0], [r_outer, float(np.pi), float(2.0 * np.pi)],
                                     [nr, ntheta, nphi], bc, diffusivity, T_initial, dt, num_steps, steady, source_type,
-                                    source_value, rtol)
+                                    source_value, rtol, precond=precond)
     coords = np.empty((X.shape[0], 3))
     coords[:, 0] = X[:, 0] * np.sin(X[:, 1]) * np.cos(X[:, 2])
     coords[:, 1] = X[:, 0] * np.sin(X[:, 1]) * np.sin(X[:, 2])
