@@ -21,7 +21,9 @@ BoxMesh((0,-R,-R),(Lx,R,R)) with the radial weight sqrt(y^2+z^2), DG0 core diffu
 Solver knobs the reference does not have come from the environment so existing callers are
 unaffected: PDE_B200_RTOL (default 1e-10), PDE_B200_PRECOND (auto|gmg|jacobi),
 PDE_B200_SNAPSHOT_STRIDE (default 1 = every step, as the reference), PDE_B200_STREAM (npz|xdmf: stream the
-snapshots to a file beside the pickle instead of holding them all in memory)."""
+snapshots to a file beside the pickle instead of holding them all in memory).  All eight heat tools honour the
+stride and streaming; the curvilinear tools write their coordinate-space lattice (e.g. (r, theta, phi)) and the
+cylinder branch of solve_heat_3D the BoxMesh (0,-R,-R)-(Lx,R,R) it solves on.  Steady solves do not stream."""
 import json
 import os
 import pickle
@@ -39,6 +41,7 @@ from mcp.server.fastmcp import FastMCP  # noqa: E402
 
 import pde_solver_b200 as _p  # noqa: E402
 from pde_solver_b200.fields import PlotResult, SolveResult, TimeSeriesField  # noqa: E402,F401
+from pde_solver_b200.solvers import curvilinear_grid, heat_3d_grid  # noqa: E402
 
 mcp = FastMCP("FEniCS-Heat")
 
@@ -52,7 +55,7 @@ def _stride():
     return max(1, int(os.environ.get("PDE_B200_SNAPSHOT_STRIDE", "1")))
 
 
-def _stream(data_dir: str, stem: str, dim: int, n, L):
+def _stream(data_dir: str, stem: str, dim: int, n, L, origin=None, meta=None):
     """PDE_B200_STREAM=npz|xdmf: snapshots go to <data_dir>/<stem>_<uuid8>.<ext> one at a time (the pickle
     then keeps only the first and last one).  Returns (writer or None, uuid8)."""
     tag = uuid.uuid4().hex[:8]
@@ -61,7 +64,15 @@ def _stream(data_dir: str, stem: str, dim: int, n, L):
         return None, tag
     from pde_solver_b200 import io as _io
     Path(data_dir).mkdir(parents=True, exist_ok=True)
-    return _io.open_writer(fmt, str(Path(data_dir) / f"{stem}_{tag}.{fmt}"), dim, n, L, name="temperature"), tag
+    return _io.open_writer(fmt, str(Path(data_dir) / f"{stem}_{tag}.{fmt}"), dim, n, L, name="temperature",
+                           meta=meta, origin=origin), tag
+
+
+def _stream_grid(data_dir: str, stem: str, grid, system=None):
+    """_stream for the lattice grid = (n, lo, hi) a solver builds: L = hi - lo, origin = lo."""
+    n, lo, hi = grid
+    meta = {"coordinate_system": system} if system else None
+    return _stream(data_dir, stem, len(n), n, [h - l for l, h in zip(lo, hi)], origin=lo, meta=meta)
 
 
 def _save(field: TimeSeriesField, data_dir: str, stem: str, tag: Optional[str] = None, writer=None) -> SolveResult:
@@ -69,7 +80,7 @@ def _save(field: TimeSeriesField, data_dir: str, stem: str, tag: Optional[str] =
     data_path = Path(data_dir)
     data_path.mkdir(parents=True, exist_ok=True)
     if writer is not None:
-        # steady solves and the cylinder / composite-core branch never stream: do not publish an empty series
+        # steady solves never stream: do not publish an empty series
         written = len(writer.times)
         path = writer.close()
         if written > 0:
@@ -173,7 +184,9 @@ def solve_heat_3D(
 ) -> SolveResult:
     """3D heat equation on the box [0,Lx]x[0,Ly]x[0,Lz]: uniform Dirichlet value T_boundary, or the
     directional values T_left (x=0) / T_right (x=Lx) / T_side (remaining faces)."""
-    writer, tag = _stream(data_dir, "heat_3d", 3, [nx, ny, nz], [Lx, Ly, Lz])
+    # the cylinder branch solves on BoxMesh (0,-R,-R)-(Lx,R,R) with its own node counts
+    writer, tag = _stream_grid(data_dir, "heat_3d", heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type,
+                                                                 cylinder_radius))
     field = _p._solve_heat_3d_raw(
         Lx=Lx, Ly=Ly, Lz=Lz, nx=nx, ny=ny, nz=nz, diffusivity=diffusivity, T_boundary=T_boundary,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
@@ -252,12 +265,15 @@ def solve_heat_3D_spherical(
     source_value: float = 0.0, initial_type: str = "constant", initial_amplitude: float = 1.0,
 ) -> SolveResult:
     """3D heat equation in spherical coordinates (r, theta, phi) on [r_inner, r_outer] x [0, pi] x [0, 2 pi]."""
+    writer, tag = _stream_grid(data_dir, "heat_3d_spherical",
+                               curvilinear_grid("3d_spherical", r_inner, r_outer, [nr, ntheta, nphi]),
+                               "spherical (r, theta, phi)")
     field = _p._solve_heat_3d_spherical_raw(
         r_inner=r_inner, r_outer=r_outer, nr=nr, ntheta=ntheta, nphi=nphi, diffusivity=diffusivity,
         T_boundary=T_boundary, T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
-    return _save(field, data_dir, "heat_3d_spherical")
+        snapshot_stride=_stride(), stream_to=writer, **_knobs())
+    return _save(field, data_dir, "heat_3d_spherical", tag, writer)
 
 
 @mcp.tool()
@@ -268,12 +284,14 @@ def solve_heat_1D_cylindrical(
     initial_amplitude: float = 1.0,
 ) -> SolveResult:
     """1D radial heat equation in cylindrical coordinates on (r_inner, r_outer)."""
+    writer, tag = _stream_grid(data_dir, "heat_1d_cylindrical",
+                               curvilinear_grid("1d_cylindrical", r_inner, r_outer, [nr]), "cylindrical (r)")
     field = _p._solve_heat_1d_cylindrical_raw(
         r_inner=r_inner, r_outer=r_outer, nr=nr, diffusivity=diffusivity, T_inner=T_inner, T_outer=T_outer,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
-    return _save(field, data_dir, "heat_1d_cylindrical")
+        snapshot_stride=_stride(), stream_to=writer, **_knobs())
+    return _save(field, data_dir, "heat_1d_cylindrical", tag, writer)
 
 
 @mcp.tool()
@@ -284,12 +302,14 @@ def solve_heat_1D_spherical(
     initial_amplitude: float = 1.0,
 ) -> SolveResult:
     """1D radial heat equation in spherical coordinates on (r_inner, r_outer)."""
+    writer, tag = _stream_grid(data_dir, "heat_1d_spherical", curvilinear_grid("1d_spherical", r_inner, r_outer, [nr]),
+                               "spherical (r)")
     field = _p._solve_heat_1d_spherical_raw(
         r_inner=r_inner, r_outer=r_outer, nr=nr, diffusivity=diffusivity, T_inner=T_inner, T_outer=T_outer,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
-    return _save(field, data_dir, "heat_1d_spherical")
+        snapshot_stride=_stride(), stream_to=writer, **_knobs())
+    return _save(field, data_dir, "heat_1d_spherical", tag, writer)
 
 
 @mcp.tool()
@@ -300,12 +320,15 @@ def solve_heat_2D_cylindrical(
     source_value: float = 0.0, initial_type: str = "constant", initial_amplitude: float = 1.0,
 ) -> SolveResult:
     """2D axisymmetric heat equation in cylindrical coordinates (r, z)."""
+    writer, tag = _stream_grid(data_dir, "heat_2d_cylindrical",
+                               curvilinear_grid("2d_cylindrical", r_inner, r_outer, [nr, nz], z_length),
+                               "cylindrical (r, z)")
     field = _p._solve_heat_2d_cylindrical_raw(
         r_inner=r_inner, r_outer=r_outer, z_length=z_length, nr=nr, nz=nz, diffusivity=diffusivity,
         T_boundary=T_boundary, T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
-    return _save(field, data_dir, "heat_2d_cylindrical")
+        snapshot_stride=_stride(), stream_to=writer, **_knobs())
+    return _save(field, data_dir, "heat_2d_cylindrical", tag, writer)
 
 
 @mcp.tool()
@@ -316,12 +339,14 @@ def solve_heat_2D_spherical(
     initial_type: str = "constant", initial_amplitude: float = 1.0,
 ) -> SolveResult:
     """2D axisymmetric heat equation in spherical coordinates (r, theta)."""
+    writer, tag = _stream_grid(data_dir, "heat_2d_spherical",
+                               curvilinear_grid("2d_spherical", r_inner, r_outer, [nr, ntheta]), "spherical (r, theta)")
     field = _p._solve_heat_2d_spherical_raw(
         r_inner=r_inner, r_outer=r_outer, nr=nr, ntheta=ntheta, diffusivity=diffusivity, T_boundary=T_boundary,
         T_initial=T_initial, dt=dt, num_steps=num_steps, steady=steady, source_type=source_type,
         source_value=source_value, initial_type=initial_type, initial_amplitude=initial_amplitude,
-        rtol=_knobs()["rtol"], precond=_knobs()["precond"])
-    return _save(field, data_dir, "heat_2d_spherical")
+        snapshot_stride=_stride(), stream_to=writer, **_knobs())
+    return _save(field, data_dir, "heat_2d_spherical", tag, writer)
 
 
 # ─────────────────────────────── plot tools (consumers of the .pkl) ───────────────────────────────

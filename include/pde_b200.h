@@ -170,7 +170,9 @@ int pde_heat_close(pde_heat_state* s);
  *   a = w u v dx + dt k w grad(u).grad(v) dx,  L = w u_n v dx + dt w f v dx,
  *   w = x0^weight_rpow * (weight_sin_axis1 ? sin(x1) : 1), an Expression of degree weight_degree (1 or 2).
  * The initial state of the curvilinear tools is the constant T_initial (every initial_type falls back to it);
- * the 3D cylinder / composite-core branches honour initial_type like the box solver. */
+ * the 3D cylinder / composite-core branches honour initial_type like the box solver.  PDE_IC_ARRAY is refused:
+ * a host initial field goes through the resident stepper (pde_wheat_open + pde_wheat_set_state), which also serves
+ * runs whose snapshots do not fit in host memory (one pde_wheat_get_state per kept snapshot). */
 typedef struct pde_wheat_params {
   int32_t dim;
   int32_t n[3];
@@ -202,6 +204,18 @@ typedef struct pde_wheat_params {
  * Jacobi-PCG (true_relres = NaN). */
 int pde_wheat_solve(pde_ctx* ctx, const pde_wheat_params* p, const pde_solver_opts* o,
                     double* values_out /* [nsnap][nverts] */, double* times_out, pde_stats* st);
+/* resident stepper of the same solve: state stays in HBM between calls, pde_wheat_solve is open + step(1) per step
+ * + get_state per kept snapshot.  open assembles, builds the GMG hierarchy (o->precond as above) and sets the
+ * initial state from initial_type (num_steps and snapshot_stride are not used).  set_state loads a host field and
+ * re-applies the Dirichlet values.  step runs nsteps backward-Euler steps (steady: the one solve, from the current
+ * state as starting guess); st covers this call, true_relres its last step.  One GPU only. */
+typedef struct pde_wheat_state pde_wheat_state;
+int pde_wheat_open(pde_ctx* ctx, const pde_wheat_params* p, const pde_solver_opts* o, pde_wheat_state** out);
+int pde_wheat_set_state(pde_wheat_state* s, const double* u_host /* [nverts] natural order */);
+int pde_wheat_step(pde_wheat_state* s, int nsteps, pde_stats* st);
+int pde_wheat_get_state(pde_wheat_state* s, double* u_host /* [nverts] natural order */);
+int64_t pde_wheat_local_nverts(pde_wheat_state* s);
+int pde_wheat_close(pde_wheat_state* s);
 /* Operator of multigrid level `level` of the GMG path: n_out = cells per user axis of that level (0 for absent axes),
  * coef_out = [nk][nverts] in natural vertex order, nk = 3 / 7 / 15 (1-D / 2-D / 3-D): entry [k][i] = a(i, i + d_k)
  * with d_k the Kuhn offsets in internal axes (x, y, z; 2-D: x, z) in the order {0, +x, -x, +y, -y, +z, -z, +xy, -xy,

@@ -87,6 +87,7 @@ def lib():
         L.pde_last_error.restype = C.c_char_p
         L.pde_ctx_launch_count.restype = C.c_int64
         L.pde_heat_local_nverts.restype = C.c_int64
+        L.pde_wheat_local_nverts.restype = C.c_int64
         L.pde_solver_opts_default.restype = None
         for name in ("pde_ctx_create", "pde_ctx_destroy", "pde_ctx_sync", "pde_timer_start", "pde_timer_stop",
                      "pde_nccl_unique_id", "pde_comm_init", "pde_mesh_counts", "pde_mesh_coords",
@@ -95,6 +96,7 @@ def lib():
                      "pde_heat_advance_batch", "pde_halo_check",
                      "pde_heat_close", "pde_elasticity_solve", "pde_op_table", "pde_op_apply", "pde_op_bench", "pde_op_sweep", "pde_op_bench_mode", "pde_comm_info", "pde_device_count",
                      "pde_op_solve", "pde_version", "pde_host_alloc", "pde_host_free", "pde_slab_partition", "pde_op_manufactured", "pde_halo_bench", "pde_wheat_solve", "pde_wheat_level_coefs",
+                     "pde_wheat_open", "pde_wheat_set_state", "pde_wheat_step", "pde_wheat_get_state", "pde_wheat_close",
                      "pde_mesh_coords_box"):
             getattr(L, name).restype = C.c_int
         _lib = L

@@ -94,17 +94,6 @@ struct DevMem {
   }
 };
 
-static int d2h(pde_ctx* c, void* dst, const void* src, size_t bytes) {
-  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
-  CUDA_OK(cudaStreamSynchronize(c->stream));
-  return 0;
-}
-static int h2d(pde_ctx* c, void* dst, const void* src, size_t bytes) {
-  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, c->stream));
-  CUDA_OK(cudaStreamSynchronize(c->stream));
-  return 0;
-}
-
 extern "C" int pde_halo_bench(pde_ctx* c, int dim, const int32_t n[3], int ncomp, int reps, double* ms_per_exchange,
                               int64_t* bytes_sent) {
   if (!c) PDE_FAIL("null context");

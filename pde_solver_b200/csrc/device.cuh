@@ -157,6 +157,18 @@ static inline RowLaunch row_launch(const pde_ctx* c, const Grid& g) {
   r.grid = dim3((unsigned)blocks, 1, 1);
   return r;
 }
+// blocking host <-> device copies on the context's stream
+static inline int d2h(pde_ctx* c, void* dst, const void* src, size_t bytes) {
+  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_OK(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+static inline int h2d(pde_ctx* c, void* dst, const void* src, size_t bytes) {
+  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, c->stream));
+  CUDA_OK(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+
 static inline int flat_blocks(const pde_ctx* c, long long n_items, int threads) {
   long long blocks = (n_items + threads - 1) / threads;
   long long cap = (long long)c->sm_count * 8;

@@ -18,6 +18,8 @@
 #include <chrono>
 #include <cmath>
 #include <cstring>
+#include <memory>
+#include <new>
 
 #include "wmg.cuh"
 
@@ -392,66 +394,82 @@ static int wheat_assemble(pde_ctx* c, const pde_wheat_params* p, WheatState& s, 
   return 0;
 }
 
-extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o_in, double* values_out,
-                               double* times_out, pde_stats* st_out) {
-  if (!c || !p || !values_out || !times_out) PDE_FAIL("null argument");
-  pde_solver_opts o;
-  if (o_in) o = *o_in; else pde_solver_opts_default(&o);
-  WheatState s;
-  double L[3];
-  PDE_OK(wheat_assemble(c, p, s, L));
-  const Grid& g = s.g;
-  const double f = p->source_value;
-  // GMG only on request (PDE_PRECOND_AUTO keeps Jacobi here); a grid that does not coarsen runs Jacobi
+// Resident stepper: the assembled operator, the multigrid hierarchy and the field stay on the device between calls.
+// pde_wheat_solve runs on the same pieces (wheat_setup, wheat_init_state, wheat_advance, wheat_get_state).
+struct pde_wheat_state : WheatState {
+  pde_wheat_params prm{};
+  pde_solver_opts o{};
+  double L[3] = {1.0, 1.0, 1.0};
   WHierarchy mg;
   bool use_mg = false;
-  double setup_ms = 0.0;
-  if (o.precond == PDE_PRECOND_GMG) {
+  double setup_ms = 0.0;   // host time of the hierarchy set-up
+  Field un;                // u_n of a verified step (true residual), allocated on first use
+  double* dense = nullptr; // [nloc] natural-order staging buffer of the host copies
+  long long nloc = 0;
+  ~pde_wheat_state() {
+    un.release();
+    if (dense) cudaFree(dense);
+  }
+};
+
+// everything before the initial state: checks, assembly, the GMG hierarchy (PDE_PRECOND_AUTO keeps Jacobi here; a
+// grid that does not coarsen runs Jacobi), the staging buffer
+static int wheat_setup(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o_in, pde_wheat_state* s) {
+  if (p->initial_type == PDE_IC_ARRAY) PDE_FAIL("initial_type array: load the field with pde_wheat_set_state");
+  s->prm = *p;
+  if (o_in) s->o = *o_in; else pde_solver_opts_default(&s->o);
+  PDE_OK(wheat_assemble(c, p, *s, s->L));
+  if (s->o.precond == PDE_PRECOND_GMG) {
     CUDA_OK(cudaStreamSynchronize(c->stream));
     const auto t0 = std::chrono::steady_clock::now();
-    PDE_OK(mg.build(c, g, s.bc, s.coefA.p));
+    PDE_OK(s->mg.build(c, s->g, s->bc, s->coefA.p));
     CUDA_OK(cudaStreamSynchronize(c->stream));
-    setup_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    use_mg = mg.levels() >= 2;
-    if (!use_mg) mg.release();
+    s->setup_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    s->use_mg = s->mg.levels() >= 2;
+    if (!s->use_mg) s->mg.release();
   }
-  pde_stats st;
-  std::memset(&st, 0, sizeof(st));
-  st.ndofs = (long long)g.nn[0] * g.nn[1] * g.nzg;
-  st.converged = 1;
-  st.true_relres = NAN;
-  st.setup_ms = setup_ms;
-  const bool verify = use_mg && o.verify_residual >= 0;
-  auto solve = [&](double bn2) -> int {
-    return use_mg ? wmg_pcg(c, mg, s.u.p, s.r.p, s.p.p, s.q.p, bn2, o, &st) : wpcg(s, bn2, o, &st);
-  };
-  const long long nloc = st.ndofs;
-  double* dense = nullptr;
-  CUDA_OK(cudaMalloc(&dense, sizeof(double) * nloc));
-  struct DenseRel { double* p; ~DenseRel() { cudaFree(p); } } denserel{dense};
-  auto snapshot = [&](double* dst) -> int {
-    PDE_OK(launch_pack(c, g, 1, s.u.p, dense, 0));
-    CUDA_OK(cudaMemcpyAsync(dst, dense, sizeof(double) * nloc, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_OK(cudaStreamSynchronize(c->stream));
-    return 0;
-  };
-  CUDA_OK(cudaEventRecord(c->ev0, c->stream));
-  const long long l0 = c->launches;
-  // initial state / Dirichlet lift: every initial_type of the curvilinear tools falls back to the constant
-  // (:893-896 ...); the 3D cylinder / composite branches keep zero and the (unweighted) cosine / sine projection
-  if (!p->steady && (p->initial_type == PDE_IC_COSINE || p->initial_type == PDE_IC_SINE)) {
-    PDE_OK(project_trig_ic(c, g, s.bc, p->dim, p->n, L, p->lo, p->initial_amplitude, p->initial_wavenumber,
-                           p->initial_type == PDE_IC_SINE, o, s.u.p, s.r.p));
+  s->nloc = (long long)s->g.nn[0] * s->g.nn[1] * s->g.nzg;
+  CUDA_OK(cudaMalloc(&s->dense, sizeof(double) * s->nloc));
+  return 0;
+}
+
+// initial state / Dirichlet lift: every initial_type of the curvilinear tools falls back to the constant
+// (:893-896 ...); the 3D cylinder / composite branches keep zero and the (unweighted) cosine / sine projection
+static int wheat_init_state(pde_wheat_state& s) {
+  const pde_wheat_params& p = s.prm;
+  if (!p.steady && (p.initial_type == PDE_IC_COSINE || p.initial_type == PDE_IC_SINE)) {
+    PDE_OK(project_trig_ic(s.c, s.g, s.bc, p.dim, p.n, s.L, p.lo, p.initial_amplitude, p.initial_wavenumber,
+                           p.initial_type == PDE_IC_SINE, s.o, s.u.p, s.r.p));
   } else {
-    const double v0 = (p->steady || p->initial_type == PDE_IC_ZERO) ? 0.0 : p->T_initial;
-    PDE_OK(launch_fill_ic(c, g, s.bc, s.u.p, v0, 1));
+    const double v0 = (p.steady || p.initial_type == PDE_IC_ZERO) ? 0.0 : p.T_initial;
+    PDE_OK(launch_fill_ic(s.c, s.g, s.bc, s.u.p, v0, 1));
   }
-  long long snap = 0;
-  // GMG path: ||b - A x|| / ||b|| of the last solve with the full assembled stencil (also checks the packed operator)
-  Field un;
-  struct UnRel { Field* f; ~UnRel() { f->release(); } } unrel{&un};
-  if (p->steady) {
-    // r0 = f m_w - k K_w u_lift  (A = k K_w)
+  return 0;
+}
+
+static void wheat_stats(const pde_wheat_state& s, pde_stats* st) {
+  std::memset(st, 0, sizeof(*st));
+  st->ndofs = s.nloc;
+  st->converged = 1;
+  st->true_relres = NAN;
+  st->setup_ms = s.setup_ms;
+}
+
+// nsteps backward-Euler steps (steady: the one solve, u is the starting guess), accumulated into st.  verify_last: on
+// the GMG path (verify_residual >= 0), ||b - A x|| / ||b|| of the last step with the full assembled stencil (this also
+// checks the packed operator)
+static int wheat_advance(pde_wheat_state& s, int nsteps, bool verify_last, pde_stats* st) {
+  pde_ctx* c = s.c;
+  const Grid& g = s.g;
+  const pde_wheat_params& p = s.prm;
+  const double f = p.source_value;
+  const bool verify = verify_last && s.use_mg && s.o.verify_residual >= 0;
+  auto solve = [&](double bn2) -> int {
+    return s.use_mg ? wmg_pcg(c, s.mg, s.u.p, s.r.p, s.p.p, s.q.p, bn2, s.o, st) : wpcg(s, bn2, s.o, st);
+  };
+  if (p.steady) {
+    if (nsteps < 1) return 0;
+    // r0 = f m_w - k K_w u  (A = k K_w)
     PDE_OK(vapply(s, s.coefA, s.u.p, s.r.p, 0.0, -1.0, f, S_XY));
     double bn2;
     PDE_OK(read_scal(c, S_YY, 1, &bn2));
@@ -460,35 +478,125 @@ extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_
       PDE_OK(vapply(s, s.coefA, s.u.p, s.q.p, 0.0, -1.0, f, S_XY));
       double rr;
       PDE_OK(read_scal(c, S_YY, 1, &rr));
-      st.true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
+      st->true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
     }
-    PDE_OK(snapshot(values_out));
+    return 0;
+  }
+  for (int step = 0; step < nsteps; ++step) {
+    const bool last = verify && step == nsteps - 1;
+    if (last) {
+      if (!s.un.p) PDE_OK(s.un.alloc(c, g, 1));
+      PDE_OK(launch_copy(c, g, 1, s.un.p, s.u.p));
+    }
+    // b = M_w u_n + dt f m_w (its norm is the stopping scale); warm start x0 = u_n: r0 = b - A u_n
+    PDE_OK(vapply(s, s.coefM, s.u.p, s.r.p, 0.0, 1.0, p.dt * f, S_XY));
+    double bn2;
+    PDE_OK(read_scal(c, S_YY, 1, &bn2));
+    PDE_OK(vapply(s, s.coefA, s.u.p, s.r.p, 1.0, -1.0, 0.0, -1));
+    PDE_OK(solve(bn2));
+    if (last) {
+      PDE_OK(vapply(s, s.coefM, s.un.p, s.q.p, 0.0, 1.0, p.dt * f, -1));
+      PDE_OK(vapply(s, s.coefA, s.u.p, s.q.p, 1.0, -1.0, 0.0, S_XY));
+      double rr;
+      PDE_OK(read_scal(c, S_YY, 1, &rr));
+      st->true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
+    }
+  }
+  return 0;
+}
+
+static int wheat_get_state(pde_wheat_state& s, double* dst) {
+  PDE_OK(launch_pack(s.c, s.g, 1, s.u.p, s.dense, 0));
+  return d2h(s.c, dst, s.dense, sizeof(double) * s.nloc);
+}
+
+extern "C" int pde_wheat_close(pde_wheat_state* s) {
+  if (!s) return 0;
+  cudaSetDevice(s->c->device);
+  cudaStreamSynchronize(s->c->stream);
+  delete s;
+  return 0;
+}
+
+extern "C" int pde_wheat_open(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o, pde_wheat_state** out) {
+  if (!c || !p || !out) PDE_FAIL("null argument");
+  pde_wheat_state* s = new (std::nothrow) pde_wheat_state();
+  if (!s) PDE_FAIL("out of host memory");
+  s->c = c;
+  int rc = wheat_setup(c, p, o, s);
+  if (!rc) rc = wheat_init_state(*s);
+  if (rc) {
+    pde_wheat_close(s);
+    return rc;
+  }
+  *out = s;
+  return 0;
+}
+
+extern "C" int64_t pde_wheat_local_nverts(pde_wheat_state* s) { return s ? s->nloc : 0; }
+
+extern "C" int pde_wheat_set_state(pde_wheat_state* s, const double* u_host) {
+  if (!s || !u_host) PDE_FAIL("null argument");
+  pde_ctx* c = s->c;
+  CUDA_OK(cudaSetDevice(c->device));
+  PDE_OK(h2d(c, s->dense, u_host, sizeof(double) * s->nloc));
+  PDE_OK(launch_unpack(c, s->g, 1, s->dense, s->u.p, 0));
+  return launch_apply_bc_values(c, s->g, s->bc, s->u.p);
+}
+
+extern "C" int pde_wheat_get_state(pde_wheat_state* s, double* u_host) {
+  if (!s || !u_host) PDE_FAIL("null argument");
+  CUDA_OK(cudaSetDevice(s->c->device));
+  return wheat_get_state(*s, u_host);
+}
+
+extern "C" int pde_wheat_step(pde_wheat_state* s, int nsteps, pde_stats* st_out) {
+  if (!s) PDE_FAIL("null state");
+  if (nsteps < 0) PDE_FAIL("nsteps must be >= 0");
+  pde_ctx* c = s->c;
+  CUDA_OK(cudaSetDevice(c->device));
+  pde_stats st;
+  wheat_stats(*s, &st);
+  const long long l0 = c->launches;
+  CUDA_OK(cudaEventRecord(c->ev0, c->stream));
+  PDE_OK(wheat_advance(*s, nsteps, true, &st));
+  CUDA_OK(cudaEventRecord(c->ev1, c->stream));
+  CUDA_OK(cudaEventSynchronize(c->ev1));
+  float ms = 0;
+  CUDA_OK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+  st.solve_ms = ms;
+  st.launches = c->launches - l0;
+  if (st_out) *st_out = st;
+  return 0;
+}
+
+// open, step(1) per step with a snapshot every snapshot_stride steps, close.  solve_ms is the device time from the
+// initial state to the last snapshot; the set-up (assembly, hierarchy) is not part of it.
+extern "C" int pde_wheat_solve(pde_ctx* c, const pde_wheat_params* p, const pde_solver_opts* o, double* values_out,
+                               double* times_out, pde_stats* st_out) {
+  if (!c || !p || !values_out || !times_out) PDE_FAIL("null argument");
+  std::unique_ptr<pde_wheat_state> s(new (std::nothrow) pde_wheat_state());
+  if (!s) PDE_FAIL("out of host memory");
+  s->c = c;
+  PDE_OK(wheat_setup(c, p, o, s.get()));
+  pde_stats st;
+  wheat_stats(*s, &st);
+  CUDA_OK(cudaEventRecord(c->ev0, c->stream));
+  const long long l0 = c->launches;
+  PDE_OK(wheat_init_state(*s));
+  if (p->steady) {
+    PDE_OK(wheat_advance(*s, 1, true, &st));
+    PDE_OK(wheat_get_state(*s, values_out));
     times_out[0] = 0.0;
   } else {
-    PDE_OK(snapshot(values_out));
+    long long snap = 0;
+    PDE_OK(wheat_get_state(*s, values_out));
     times_out[snap++] = 0.0;
     const int stride = p->snapshot_stride > 0 ? p->snapshot_stride : 1;
     for (int step = 0; step < p->num_steps; ++step) {
-      const bool last = verify && step == p->num_steps - 1;
-      if (last) {
-        PDE_OK(un.alloc(c, g, 1));
-        PDE_OK(launch_copy(c, g, 1, un.p, s.u.p));
-      }
-      // b = M_w u_n + dt f m_w (its norm is the stopping scale); warm start x0 = u_n: r0 = b - A u_n
-      PDE_OK(vapply(s, s.coefM, s.u.p, s.r.p, 0.0, 1.0, p->dt * f, S_XY));
-      double bn2;
-      PDE_OK(read_scal(c, S_YY, 1, &bn2));
-      PDE_OK(vapply(s, s.coefA, s.u.p, s.r.p, 1.0, -1.0, 0.0, -1));
-      PDE_OK(solve(bn2));
-      if (last) {
-        PDE_OK(vapply(s, s.coefM, un.p, s.q.p, 0.0, 1.0, p->dt * f, -1));
-        PDE_OK(vapply(s, s.coefA, s.u.p, s.q.p, 1.0, -1.0, 0.0, S_XY));
-        double rr;
-        PDE_OK(read_scal(c, S_YY, 1, &rr));
-        st.true_relres = bn2 > 0 ? std::sqrt(rr / bn2) : 0.0;
-      }
+      PDE_OK(wheat_advance(*s, 1, step == p->num_steps - 1, &st));
       if ((step + 1) % stride == 0) {
-        PDE_OK(snapshot(values_out + snap * nloc));
+        PDE_OK(wheat_get_state(*s, values_out + snap * s->nloc));
         times_out[snap++] = (step + 1) * p->dt;
       }
     }

@@ -7,7 +7,9 @@ one snapshot on the host.
     xdmf  <stem>.xdmf (temporal collection on a 3DCoRectMesh / 2DCoRectMesh, node-centred attribute)
           + <stem>.bin  (raw little-endian float64, one snapshot after another; XDMF "Binary" + Seek)
 
-Both describe the structured grid by origin / spacing / node counts instead of a coordinate list."""
+Both describe the structured grid by origin / spacing / node counts instead of a coordinate list.  The origin
+defaults to zeros; the weighted heat solves write their coordinate-space lattice (origin = lo, L = hi - lo, e.g.
+(r, theta, phi)) and name it in meta["coordinate_system"]."""
 import json
 import os
 import zipfile
@@ -15,10 +17,15 @@ import zipfile
 import numpy as np
 
 
+def _origin(dim, origin):
+    return [0.0] * int(dim) if origin is None else [float(v) for v in origin]
+
+
 class NpzSnapshotWriter:
-    def __init__(self, path, dim, n, L, meta=None):
+    def __init__(self, path, dim, n, L, meta=None, origin=None):
         self.path = str(path)
         self.dim, self.n, self.L = int(dim), [int(v) for v in n], [float(v) for v in L]
+        self.origin = _origin(dim, origin)
         self.meta = dict(meta or {})
         self.times = []
         self._zip = zipfile.ZipFile(self.path, "w", compression=zipfile.ZIP_STORED, allowZip64=True)
@@ -37,9 +44,10 @@ class NpzSnapshotWriter:
         self._put("times", np.asarray(self.times))
         self._put("shape_nodes", np.asarray([v + 1 for v in self.n], dtype=np.int64))
         self._put("extent", np.asarray(self.L))
+        self._put("origin", np.asarray(self.origin))
         with self._zip.open("meta.json", "w") as f:
-            f.write(json.dumps({"dim": self.dim, "n": self.n, "L": self.L, "order": "natural (x fastest)",
-                                **self.meta}, default=str).encode())
+            f.write(json.dumps({"dim": self.dim, "n": self.n, "L": self.L, "origin": self.origin,
+                                "order": "natural (x fastest)", **self.meta}, default=str).encode())
         self._zip.close()
         self._zip = None
         return self.path
@@ -52,11 +60,12 @@ class NpzSnapshotWriter:
 
 
 class XdmfSnapshotWriter:
-    def __init__(self, path, dim, n, L, name="u", meta=None):
+    def __init__(self, path, dim, n, L, name="u", meta=None, origin=None):
         stem = str(path)
         stem = stem[:-5] if stem.endswith(".xdmf") else stem
         self.xdmf_path, self.bin_path = stem + ".xdmf", stem + ".bin"
         self.dim, self.n, self.L = int(dim), [int(v) for v in n], [float(v) for v in L]
+        self.origin = _origin(dim, origin)
         self.name = name
         self.meta = dict(meta or {})
         self.times = []
@@ -79,8 +88,9 @@ class XdmfSnapshotWriter:
         # XDMF lists the slowest axis first (z y x); pad to at least 2-D for readers
         nodes = [v + 1 for v in self.n][::-1]
         spacing = [l / c for l, c in zip(self.L, self.n)][::-1]
+        origin = self.origin[::-1]
         if d == 1:
-            nodes, spacing = [1] + nodes, [1.0] + spacing
+            nodes, spacing, origin = [1] + nodes, [1.0] + spacing, [0.0] + origin
         dd = max(d, 2)
         topo = "3DCoRectMesh" if dd == 3 else "2DCoRectMesh"
         geo = "ORIGIN_DXDYDZ" if dd == 3 else "ORIGIN_DXDY"
@@ -93,7 +103,7 @@ class XdmfSnapshotWriter:
                     f'    <Topology TopologyType="{topo}" Dimensions="{dims}"/>',
                     f'    <Geometry GeometryType="{geo}">',
                     f'     <DataItem Dimensions="{dd}" NumberType="Float" Precision="8" Format="XML">'
-                    + " ".join("0" for _ in range(dd)) + "</DataItem>",
+                    + " ".join(f"{v:.17g}" for v in origin) + "</DataItem>",
                     f'     <DataItem Dimensions="{dd}" NumberType="Float" Precision="8" Format="XML">'
                     + " ".join(f"{v:.17g}" for v in spacing) + "</DataItem>", "    </Geometry>",
                     f'    <Attribute Name="{self.name}" AttributeType="Scalar" Center="Node">',
@@ -111,11 +121,11 @@ class XdmfSnapshotWriter:
         self.close()
 
 
-def open_writer(fmt, path, dim, n, L, name="u", meta=None):
+def open_writer(fmt, path, dim, n, L, name="u", meta=None, origin=None):
     if fmt == "npz":
-        return NpzSnapshotWriter(path, dim, n, L, meta=meta)
+        return NpzSnapshotWriter(path, dim, n, L, meta=meta, origin=origin)
     if fmt == "xdmf":
-        return XdmfSnapshotWriter(path, dim, n, L, name=name, meta=meta)
+        return XdmfSnapshotWriter(path, dim, n, L, name=name, meta=meta, origin=origin)
     raise ValueError("snapshot format must be 'npz' or 'xdmf'")
 
 

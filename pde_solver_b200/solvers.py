@@ -5,7 +5,7 @@ Reference: /root/reference/fenics_mcp_server.py
   _solve_elasticity_1d_static :1470-1587   _2d_ :1593-1743   _3d_ :1749-1892
 Each function only marshals arguments into the C ABI (include/pde_b200.h) and wraps the result;
 all arithmetic runs in hand-written CUDA.  Extra keyword-only arguments (rtol, precond,
-snapshot_stride, as_arrays) are additions the reference does not have; their defaults reproduce
+snapshot_stride, as_arrays, u0, stream_to) are additions the reference does not have; their defaults reproduce
 the reference's behaviour."""
 import ctypes as C
 import os
@@ -194,7 +194,8 @@ def _solve_heat_3d_raw(Lx: float, Ly: float, Lz: float, nx: int, ny: int, nz: in
         return _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady,
                                 source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
                                 geometry_type, cylinder_radius, T_left, T_right, T_side, core_radius,
-                                core_diffusivity, rtol, snapshot_stride, as_arrays, precond)
+                                core_diffusivity, rtol, snapshot_stride, as_arrays, precond, u0=u0,
+                                stream_to=stream_to)
     bc = mesh.heat_bc(3, T_boundary=T_boundary, T_left=T_left, T_right=T_right, T_side=T_side)
     coords, values, times = _heat(3, [Lx, Ly, Lz], [nx, ny, nz], diffusivity, T_initial, dt, num_steps, steady,
                                   source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
@@ -214,24 +215,26 @@ def _solve_heat_3d_raw(Lx: float, Ly: float, Lz: float, nx: int, ny: int, nz: in
     return _finish(coords, values, times, 3, meta, as_arrays, n=[nx, ny, nz])
 
 
+def heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type="box", cylinder_radius=None):
+    """(n, lo, hi) of the mesh a _solve_heat_3d_raw call builds: the cylinder is BoxMesh((0,-R,-R), (Lx,R,R), nx,
+    int(ny*2R), int(nz*2R)) (the reference without mshr), every other geometry the box [0,Lx]x[0,Ly]x[0,Lz]."""
+    if geometry_type == "cylinder" and cylinder_radius is not None:
+        R = float(cylinder_radius)
+        return [int(nx), int(ny * R * 2), int(nz * R * 2)], [0.0, -R, -R], [float(Lx), R, R]
+    return [int(nx), int(ny), int(nz)], [0.0, 0.0, 0.0], [float(Lx), float(Ly), float(Lz)]
+
+
 def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady, source_type,
                      source_value, initial_type, initial_amplitude, initial_wavenumber, geometry_type,
                      cylinder_radius, T_left, T_right, T_side, core_radius, core_diffusivity, rtol, snapshot_stride,
-                     as_arrays, precond="jacobi", ctx=None):
+                     as_arrays, precond="jacobi", ctx=None, u0=None, stream_to=None):
     """Cylinder / composite-core branches of _solve_heat_3d_raw (:512-572, 576-605, 642-645) as the reference's
     deployment runs them (no mshr in Dockerfile / requirements.txt, so MSHR_AVAILABLE is False): the "cylinder" is
     BoxMesh((0,-R,-R),(Lx,R,R), nx, int(ny*2R), int(nz*2R)) with every term weighted by
     Expression("sqrt(x[1]^2+x[2]^2)", degree=2); the core is a DG0 diffusivity marked by SubDomain.mark."""
-    ctx = ctx or _lib.default_context()
     cyl = geometry_type == "cylinder" and cylinder_radius is not None
     has_core = core_radius is not None and core_diffusivity is not None
-    if cyl:
-        R = float(cylinder_radius)
-        lo, hi = [0.0, -R, -R], [float(Lx), R, R]
-        n = [int(nx), int(ny * R * 2), int(nz * R * 2)]
-    else:
-        lo, hi = [0.0, 0.0, 0.0], [float(Lx), float(Ly), float(Lz)]
-        n = [int(nx), int(ny), int(nz)]
+    n, lo, hi = heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type, cylinder_radius)
     if min(n) < 1:
         raise ValueError(f"BoxMesh needs at least one cell per axis, got {n}")
     directional = T_left is not None or T_right is not None or T_side is not None
@@ -266,15 +269,8 @@ def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial,
     p.initial_amplitude = float(initial_amplitude)
     p.initial_wavenumber = float(initial_wavenumber)
     p.bc = bc
-    nv, _ = _lib.mesh_counts(3, n)
-    nsnap = 1 if steady else 1 + int(num_steps) // max(1, int(snapshot_stride))
-    values = np.empty((nsnap, nv), dtype=np.float64)
-    times = np.empty(nsnap, dtype=np.float64)
-    st = _lib.Stats()
-    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
-    _lib.check(_lib.lib().pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
-                                          C.byref(st)))
-    _record(st.as_dict(), "heat solve (weighted box)")
+    values, times = _wheat(ctx, p, rtol, precond, u0, stream_to, "heat solve (weighted box)")
+    ctx = ctx or _lib.default_context()
     coords = mesh.coordinates_box(3, n, lo, hi, ctx)
     box = geometry_type == "box"
     meta = {"name": "temperature", "unit": "°C", "pde": "heat",
@@ -379,6 +375,14 @@ _CURVI = {
 }
 
 
+def curvilinear_grid(kind, r_inner, r_outer, n, z_length=None):
+    """(n, lo, hi) of the coordinate-space mesh of a curvilinear tool: IntervalMesh(nr, r_inner, r_outer),
+    RectangleMesh to (r_outer, z_length) / (r_outer, pi), BoxMesh to (r_outer, pi, 2 pi)."""
+    rest = {"2d_cylindrical": [z_length], "2d_spherical": [float(np.pi)],
+            "3d_spherical": [float(np.pi), float(2.0 * np.pi)]}.get(kind, [])
+    return [int(k) for k in n], [r_inner] + [0.0] * len(rest), [r_outer] + rest
+
+
 def _wheat_precond(precond):
     """Weighted operators: "gmg" selects Galerkin multigrid; "auto" still means Jacobi-PCG for them."""
     if precond not in _lib.PRECOND:
@@ -386,9 +390,81 @@ def _wheat_precond(precond):
     return "gmg" if precond == "gmg" else "jacobi"
 
 
-def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                 snapshot_stride=1, ctx=None, precond="jacobi"):
+def _wheat(ctx, p, rtol, precond, u0, writer, what):
+    """(values, times) of the weighted solve p.  A plain call is one pde_wheat_solve.  With a host initial field u0
+    (natural vertex order) or a snapshot writer it runs on the resident stepper (pde_wheat_open / set_state / step /
+    get_state), as _heat_streaming does for the box: every kept snapshot goes through one pinned buffer to the writer,
+    which leaves the first and last one in the result.  Steady solves never stream; u0 is their starting guess."""
+    nv = int(np.prod([int(p.n[q]) + 1 for q in range(int(p.dim))]))
+    if u0 is not None:
+        u0 = np.ascontiguousarray(u0, dtype=np.float64)
+        if u0.shape != (nv,):
+            raise ValueError(f"u0 must hold one value per mesh vertex ({nv}), got shape {u0.shape}")
     ctx = ctx or _lib.default_context()
+    steady = bool(p.steady)
+    if steady:
+        writer = None
+    stride = max(1, int(p.snapshot_stride))
+    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
+    L = _lib.lib()
+    if u0 is None and writer is None:
+        nsnap = 1 if steady else 1 + int(p.num_steps) // stride
+        values = np.empty((nsnap, nv), dtype=np.float64)
+        times = np.empty(nsnap, dtype=np.float64)
+        st = _lib.Stats()
+        _lib.check(L.pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
+                                     C.byref(st)))
+        _record(st.as_dict(), what)
+        return values, times
+    h = C.c_void_p()
+    _lib.check(L.pde_wheat_open(ctx.handle, C.byref(p), C.byref(o), C.byref(h)))
+    buf = _lib.PinnedArray(nv) if writer is not None else None
+    acc = {"iters_total": 0, "solves": 0, "converged": 1, "solve_ms": 0.0, "launches": 0}
+    kept, times = [], []
+
+    def keep(t):
+        out = buf.array if writer is not None else np.empty(nv, dtype=np.float64)
+        _lib.check(L.pde_wheat_get_state(h, _lib.ptr(out)))
+        times.append(t)
+        if writer is None:
+            kept.append(out)
+            return
+        writer.append(t, out)
+        if len(kept) < 2:
+            kept.append(out.copy())
+        else:
+            kept[1][:] = out
+
+    try:
+        if u0 is not None:
+            _lib.check(L.pde_wheat_set_state(h, _lib.ptr(u0)))
+        if not steady:
+            keep(0.0)
+        st = _lib.Stats()
+        for step in range(1 if steady else int(p.num_steps)):
+            _lib.check(L.pde_wheat_step(h, 1, C.byref(st)))
+            d = st.as_dict()
+            for k in ("iters_total", "solves", "solve_ms", "launches"):
+                acc[k] += d[k]
+            acc["converged"] &= d["converged"]
+            acc.update(ndofs=d["ndofs"], levels=d["levels"], final_relres=d["final_relres"], setup_ms=d["setup_ms"],
+                       true_relres=d["true_relres"])
+            if steady:
+                keep(0.0)
+            elif (step + 1) % stride == 0:
+                keep((step + 1) * p.dt)
+    finally:
+        L.pde_wheat_close(h)
+        if buf is not None:
+            buf.free()
+    _record(acc, what + (" (streaming)" if writer is not None else ""))
+    if writer is not None:
+        return np.stack([kept[0], kept[-1]]), np.array([times[0], times[-1]])
+    return np.stack(kept), np.array(times)
+
+
+def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                 snapshot_stride=1, ctx=None, precond="jacobi", u0=None, stream_to=None):
     dim, rpow, wsin, wdeg = _CURVI[kind]
     p = _lib.WheatParams()
     p.dim = dim
@@ -404,15 +480,8 @@ def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, ste
     p.source_value = float(source_value) if source_type == "constant" else 0.0
     p.T_initial = float(T_initial)
     p.bc = bc
-    nv, _ = _lib.mesh_counts(dim, n)
-    nsnap = 1 if steady else 1 + int(num_steps) // max(1, int(snapshot_stride))
-    values = np.empty((nsnap, nv), dtype=np.float64)
-    times = np.empty(nsnap, dtype=np.float64)
-    st = _lib.Stats()
-    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
-    _lib.check(_lib.lib().pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
-                                          C.byref(st)))
-    _record(st.as_dict(), "curvilinear heat solve")
+    values, times = _wheat(ctx, p, rtol, precond, u0, stream_to, "curvilinear heat solve")
+    ctx = ctx or _lib.default_context()
     X = mesh.coordinates_box(dim, n, lo, hi, ctx)
     return X, values, times
 
@@ -436,12 +505,13 @@ def _solve_heat_1d_cylindrical_raw(r_inner: float, r_outer: float, nr: int, diff
                                    T_outer: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                    source_type: str = "none", source_value: float = 0.0,
                                    initial_type: str = "constant", initial_amplitude: float = 1.0, *,
-                                   rtol: float = 1e-10, precond: str = "jacobi",
-                                   as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                   rtol: float = 1e-10, precond: str = "jacobi", snapshot_stride: int = 1,
+                                   as_arrays: Optional[bool] = None, u0=None, stream_to=None) -> TimeSeriesField:
     """1D radial heat equation in cylindrical coordinates, weight r (:769-920)."""
-    X, values, times = _curvilinear("1d_cylindrical", [r_inner], [r_outer], [nr], _radial_bc(r_inner, T_inner, T_outer),
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    precond=precond)
+    n, lo, hi = curvilinear_grid("1d_cylindrical", r_inner, r_outer, [nr])
+    X, values, times = _curvilinear("1d_cylindrical", lo, hi, n, _radial_bc(r_inner, T_inner, T_outer), diffusivity,
+                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
     order = np.argsort(X[:, 0], kind="stable")
     meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annulus", r_inner, r_outer, source_type,
                        source_value, steady)
@@ -452,11 +522,13 @@ def _solve_heat_1d_spherical_raw(r_inner: float, r_outer: float, nr: int, diffus
                                  T_outer: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
                                  initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
-                                 as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                 snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
+                                 stream_to=None) -> TimeSeriesField:
     """1D radial heat equation in spherical coordinates, weight r^2 (:926-1057)."""
-    X, values, times = _curvilinear("1d_spherical", [r_inner], [r_outer], [nr], _radial_bc(r_inner, T_inner, T_outer),
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    precond=precond)
+    n, lo, hi = curvilinear_grid("1d_spherical", r_inner, r_outer, [nr])
+    X, values, times = _curvilinear("1d_spherical", lo, hi, n, _radial_bc(r_inner, T_inner, T_outer), diffusivity,
+                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
+                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
     order = np.argsort(X[:, 0], kind="stable")
     meta = _curvi_meta("spherical", "sphere" if r_inner < 1e-10 else "spherical_shell", r_inner, r_outer, source_type,
                        source_value, steady)
@@ -467,13 +539,14 @@ def _solve_heat_2d_cylindrical_raw(r_inner: float, r_outer: float, z_length: flo
                                    diffusivity: float, T_boundary: float, T_initial: float, dt: float, num_steps: int,
                                    steady: bool = False, source_type: str = "none", source_value: float = 0.0,
                                    initial_type: str = "constant", initial_amplitude: float = 1.0, *,
-                                   rtol: float = 1e-10, precond: str = "jacobi",
-                                   as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                   rtol: float = 1e-10, precond: str = "jacobi", snapshot_stride: int = 1,
+                                   as_arrays: Optional[bool] = None, u0=None, stream_to=None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, z) plane, weight r (:1063-1185)."""
     bc = _lib.make_bc({f: T_boundary for f in range(4)})
-    X, values, times = _curvilinear("2d_cylindrical", [r_inner, 0.0], [r_outer, z_length], [nr, nz], bc, diffusivity,
-                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    precond=precond)
+    n, lo, hi = curvilinear_grid("2d_cylindrical", r_inner, r_outer, [nr, nz], z_length)
+    X, values, times = _curvilinear("2d_cylindrical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
+                                    source_type, source_value, rtol,
+                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
     coords = np.zeros((X.shape[0], 3))
     coords[:, 0], coords[:, 2] = X[:, 0], X[:, 1]                 # (r, 0, z)
     meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annular_cylinder", r_inner, r_outer,
@@ -485,12 +558,14 @@ def _solve_heat_2d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta
                                  T_boundary: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
                                  initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
-                                 as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                 snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
+                                 stream_to=None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, theta) plane, weight r^2 sin(theta) (:1191-1320)."""
     bc = _lib.make_bc({f: T_boundary for f in range(4)})
-    X, values, times = _curvilinear("2d_spherical", [r_inner, 0.0], [r_outer, float(np.pi)], [nr, ntheta], bc,
-                                    diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    precond=precond)
+    n, lo, hi = curvilinear_grid("2d_spherical", r_inner, r_outer, [nr, ntheta])
+    X, values, times = _curvilinear("2d_spherical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
+                                    source_type, source_value, rtol,
+                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
     coords = np.zeros((X.shape[0], 3))
     coords[:, 0] = X[:, 0] * np.sin(X[:, 1])                      # phi = 0: (r sin(theta), 0, r cos(theta))
     coords[:, 2] = X[:, 0] * np.cos(X[:, 1])
@@ -503,12 +578,14 @@ def _solve_heat_3d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta
                                  T_boundary: float, T_initial: float, dt: float, num_steps: int, steady: bool = False,
                                  source_type: str = "none", source_value: float = 0.0, initial_type: str = "constant",
                                  initial_amplitude: float = 1.0, *, rtol: float = 1e-10, precond: str = "jacobi",
-                                 as_arrays: Optional[bool] = None) -> TimeSeriesField:
+                                 snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
+                                 stream_to=None) -> TimeSeriesField:
     """3D heat equation in (r, theta, phi), weight r^2 sin(theta) (:1326-1464)."""
     bc = _lib.make_bc({f: T_boundary for f in range(6)})
-    X, values, times = _curvilinear("3d_spherical", [r_inner, 0.0, 0.0], [r_outer, float(np.pi), float(2.0 * np.pi)],
-                                    [nr, ntheta, nphi], bc, diffusivity, T_initial, dt, num_steps, steady, source_type,
-                                    source_value, rtol, precond=precond)
+    n, lo, hi = curvilinear_grid("3d_spherical", r_inner, r_outer, [nr, ntheta, nphi])
+    X, values, times = _curvilinear("3d_spherical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
+                                    source_type, source_value, rtol,
+                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
     coords = np.empty((X.shape[0], 3))
     coords[:, 0] = X[:, 0] * np.sin(X[:, 1]) * np.cos(X[:, 2])
     coords[:, 1] = X[:, 0] * np.sin(X[:, 1]) * np.sin(X[:, 2])
