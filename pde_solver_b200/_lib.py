@@ -341,41 +341,67 @@ class PinnedArray:
             self.ptr = C.c_void_p()
 
 
-class HeatStepper:
-    """Device-resident backward-Euler stepper (pde_heat_open/step/close): state stays in HBM."""
+def heat_params(dim, n, L, diffusivity, dt, T_initial=0.0, bc=None, source_value=0.0, steady=False, num_steps=0,
+                snapshot_stride=1, initial_type="constant", initial_amplitude=0.0, initial_wavenumber=0.0):
+    """HeatParams (pde_heat_params) of a box heat problem; the defaults are those of a bare HeatStepper."""
+    p = HeatParams()
+    p.dim = int(dim)
+    p.n = i3(n)
+    p.L = d3(L)
+    p.diffusivity = float(diffusivity)
+    p.dt = float(dt)
+    p.num_steps = int(num_steps)
+    p.steady = 1 if steady else 0
+    p.source_value = float(source_value)
+    p.initial_type = IC.get(initial_type, IC["constant"])
+    p.snapshot_stride = int(snapshot_stride)
+    p.T_initial = float(T_initial)
+    p.initial_amplitude = float(initial_amplitude)
+    p.initial_wavenumber = float(initial_wavenumber)
+    p.bc = bc if bc is not None else Bc()
+    return p
 
-    def __init__(self, ctx, dim, n, L, diffusivity, dt, T_initial=0.0, bc=None, source_value=0.0, steady=False,
-                 opts=None):
-        p = HeatParams()
-        p.dim = int(dim)
-        p.n = i3(n)
-        p.L = d3(L)
-        p.diffusivity = float(diffusivity)
-        p.dt = float(dt)
-        p.num_steps = 0
-        p.steady = 1 if steady else 0
-        p.source_value = float(source_value)
-        p.initial_type = IC["constant"]
-        p.snapshot_stride = 1
-        p.T_initial = float(T_initial)
-        p.bc = bc if bc is not None else Bc()
+
+class Stepper:
+    """Device-resident backward-Euler stepper of one solver family (pde_<kind>_open / set_state / step / get_state /
+    close): the state stays in HBM between steps."""
+
+    def __init__(self, kind, ctx, params, opts=None):
+        self.kind = kind
         self.ctx = ctx
         self.handle = C.c_void_p()
         o = opts if opts is not None else make_opts()
-        check(lib().pde_heat_open(ctx.handle, C.byref(p), C.byref(o), C.byref(self.handle)))
-        self.nloc = int(lib().pde_heat_local_nverts(self.handle))
+        check(self._fn("open")(ctx.handle, C.byref(params), C.byref(o), C.byref(self.handle)))
+        self.nloc = int(self._fn("local_nverts")(self.handle))
+
+    def _fn(self, name):
+        return getattr(lib(), f"pde_{self.kind}_{name}")
 
     def step(self, nsteps=1):
         st = Stats()
-        check(lib().pde_heat_step(self.handle, int(nsteps), C.byref(st)))
+        check(self._fn("step")(self.handle, int(nsteps), C.byref(st)))
         return st.as_dict()
 
     def set_state(self, u):
-        check(lib().pde_heat_set_state(self.handle, ptr(u)))
+        check(self._fn("set_state")(self.handle, ptr(u)))
 
     def get_state(self, out):
-        check(lib().pde_heat_get_state(self.handle, ptr(out)))
+        check(self._fn("get_state")(self.handle, ptr(out)))
         return out
+
+    def close(self):
+        if self.handle:
+            self._fn("close")(self.handle)
+            self.handle = C.c_void_p()
+
+
+class HeatStepper(Stepper):
+    """Stepper of the box heat solve (pde_heat_*)."""
+
+    def __init__(self, ctx, dim, n, L, diffusivity, dt, T_initial=0.0, bc=None, source_value=0.0, steady=False,
+                 opts=None):
+        super().__init__("heat", ctx, heat_params(dim, n, L, diffusivity, dt, T_initial=T_initial, bc=bc,
+                                                  source_value=source_value, steady=steady), opts)
 
     def advance_batch(self, inputs, outputs):
         """Independent one-step advances inputs[k] -> outputs[k] (host arrays of nloc float64, ideally pinned):
@@ -389,7 +415,9 @@ class HeatStepper:
         check(lib().pde_heat_advance_batch(self.handle, n, pin, pout, C.byref(st)))
         return st.as_dict()
 
-    def close(self):
-        if self.handle:
-            lib().pde_heat_close(self.handle)
-            self.handle = C.c_void_p()
+
+class WheatStepper(Stepper):
+    """Stepper of the coordinate-weighted heat solve (pde_wheat_*) for a filled WheatParams."""
+
+    def __init__(self, ctx, params, opts=None):
+        super().__init__("wheat", ctx, params, opts)

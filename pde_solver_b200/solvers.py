@@ -65,82 +65,81 @@ def _heat(dim, L, n, diffusivity, T_initial, dt, num_steps, steady, source_type,
     """stream_to: an io.*SnapshotWriter.  Snapshots then go to the writer one at a time (device-resident
     stepper, one pinned host buffer) and only the first and last are returned."""
     ctx = ctx or _lib.default_context()
-    p = _lib.HeatParams()
-    p.dim = dim
-    p.n = _lib.i3(n)
-    p.L = _lib.d3(L)
-    p.diffusivity = float(diffusivity)
-    p.dt = float(dt)
-    p.num_steps = int(num_steps)
-    p.steady = 1 if steady else 0
-    p.source_value = float(source_value) if source_type == "constant" else 0.0
-    if u0 is not None:
-        p.initial_type = _lib.IC["array"]
-    else:
-        p.initial_type = _lib.IC.get(initial_type, _lib.IC["constant"])
-    p.snapshot_stride = int(snapshot_stride)
-    p.T_initial = float(T_initial)
-    p.initial_amplitude = float(initial_amplitude)
-    p.initial_wavenumber = float(initial_wavenumber)
-    p.bc = bc
+    p = _lib.heat_params(dim, n, L, diffusivity, dt, T_initial=T_initial, bc=bc,
+                         source_value=source_value if source_type == "constant" else 0.0, steady=steady,
+                         num_steps=num_steps, snapshot_stride=snapshot_stride,
+                         initial_type="array" if u0 is not None else initial_type,
+                         initial_amplitude=initial_amplitude, initial_wavenumber=initial_wavenumber)
     nv, _ = _lib.mesh_counts(dim, n)
-    if stream_to is not None and not steady:
-        return _heat_streaming(ctx, p, dim, n, L, rtol, precond, u0, stream_to)
-    nsnap = 1 if steady else 1 + int(num_steps) // max(1, int(snapshot_stride))
     o = _lib.make_opts(rtol=rtol, precond=precond)
+    u0a = np.ascontiguousarray(u0, dtype=np.float64) if u0 is not None else None
+    if stream_to is not None and not steady:
+        values, times = _run_stepper(_lib.Stepper("heat", ctx, p, o), p, u0a, stream_to, "heat solve")
+        return mesh.coordinates(dim, n, L, ctx), values, times
     if dim == 3 and u0 is None and multi.usable(int(n[2])):
         # PDE_B200_GPUS=N: the same call on N z-slabs, one worker process per GPU (multi.py)
-        stats, values, times = multi.heat_solve(p, o, nsnap, nv)
+        stats, values, times = multi.heat_solve(p, o, _nsnap(p), nv)
         _record(stats, "heat solve")
-        return mesh.coordinates(dim, n, L, ctx), values, times
-    values = np.empty((nsnap, nv), dtype=np.float64)
-    times = np.empty(nsnap, dtype=np.float64)
+    else:
+        values, times = _solve_in_memory(_lib.lib().pde_heat_solve, ctx, p, o, nv, "heat solve", _lib.ptr(u0a))
+    return mesh.coordinates(dim, n, L, ctx), values, times
+
+
+def _nsnap(p):
+    return 1 if p.steady else 1 + int(p.num_steps) // max(1, int(p.snapshot_stride))
+
+
+def _solve_in_memory(fn, ctx, p, o, nv, what, *u0):
+    """(values, times) of one pde_heat_solve / pde_wheat_solve call, every kept snapshot in host memory."""
+    values = np.empty((_nsnap(p), nv), dtype=np.float64)
+    times = np.empty(_nsnap(p), dtype=np.float64)
     st = _lib.Stats()
-    u0a = np.ascontiguousarray(u0, dtype=np.float64) if u0 is not None else None
-    _lib.check(_lib.lib().pde_heat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(u0a), _lib.ptr(values),
-                                         _lib.ptr(times), C.byref(st)))
-    _record(st.as_dict(), "heat solve")
-    coords = mesh.coordinates(dim, n, L, ctx)
-    return coords, values, times
+    _lib.check(fn(ctx.handle, C.byref(p), C.byref(o), *u0, _lib.ptr(values), _lib.ptr(times), C.byref(st)))
+    _record(st.as_dict(), what)
+    return values, times
 
 
-def _heat_streaming(ctx, p, dim, n, L, rtol, precond, u0, writer):
-    """Backward-Euler loop on the resident stepper (pde_heat_open/step/get_state): every kept snapshot is
-    copied to one pinned buffer and handed to the writer; host memory use is one snapshot."""
-    nv, _ = _lib.mesh_counts(dim, n)
-    st_h = C.c_void_p()
-    o = _lib.make_opts(rtol=rtol, precond=precond)
-    _lib.check(_lib.lib().pde_heat_open(ctx.handle, C.byref(p), C.byref(o), C.byref(st_h)))
-    buf = _lib.PinnedArray(nv)
+def _run_stepper(stepper, p, u0, writer, what):
+    """(values, times) of the solve p on a resident stepper, which it closes.  u0 (natural vertex order) replaces
+    the initial field.  A transient run keeps the state at t = 0 and after every snapshot_stride-th step: with a
+    writer every kept state goes through one pinned buffer to the writer and only the first and last are returned
+    (host memory use is one snapshot); without one every kept state is returned.  A steady run (never with a writer)
+    takes its one solve, u0 being the starting guess, and keeps the result at t = 0."""
+    steady, stride = bool(p.steady), max(1, int(p.snapshot_stride))
     acc = {"iters_total": 0, "solves": 0, "converged": 1, "solve_ms": 0.0, "launches": 0}
+    kept, times, buf = [], [], None
+
+    def keep(t):
+        out = buf.array if buf is not None else np.empty(stepper.nloc, dtype=np.float64)
+        stepper.get_state(out)
+        times.append(t)
+        if writer is not None:
+            writer.append(t, out)
+        kept.append(out.copy() if writer is not None and not kept else out)
+
     try:
+        if writer is not None:
+            buf = _lib.PinnedArray(stepper.nloc)
         if u0 is not None:
-            _lib.check(_lib.lib().pde_heat_set_state(st_h, _lib.ptr(np.ascontiguousarray(u0, dtype=np.float64))))
-        _lib.check(_lib.lib().pde_heat_get_state(st_h, _lib.ptr(buf.array)))
-        first = buf.array.copy()
-        writer.append(0.0, buf.array)
-        stride = max(1, int(p.snapshot_stride))
-        st = _lib.Stats()
-        times = [0.0]
-        for step in range(int(p.num_steps)):
-            _lib.check(_lib.lib().pde_heat_step(st_h, 1, C.byref(st)))
-            d = st.as_dict()
+            stepper.set_state(u0)
+        if not steady:
+            keep(0.0)
+        for step in range(1 if steady else int(p.num_steps)):
+            d = stepper.step(1)
             for k in ("iters_total", "solves", "solve_ms", "launches"):
                 acc[k] += d[k]
             acc["converged"] &= d["converged"]
-            acc.update(ndofs=d["ndofs"], levels=d["levels"], final_relres=d["final_relres"], setup_ms=d["setup_ms"],
-                       true_relres=d["true_relres"])
-            if (step + 1) % stride == 0:
-                _lib.check(_lib.lib().pde_heat_get_state(st_h, _lib.ptr(buf.array)))
-                times.append((step + 1) * p.dt)
-                writer.append(times[-1], buf.array)
-        last = buf.array.copy()
+            acc.update({k: d[k] for k in ("ndofs", "levels", "final_relres", "setup_ms", "true_relres")})
+            if steady or (step + 1) % stride == 0:
+                keep(0.0 if steady else (step + 1) * p.dt)
+        if writer is not None:      # the first kept state and the pinned buffer, which holds the last
+            kept, times = [kept[0], kept[-1].copy()], [times[0], times[-1]]
     finally:
-        _lib.lib().pde_heat_close(st_h)
-        buf.free()
-    _record(acc, "heat solve (streaming)")
-    coords = mesh.coordinates(dim, n, L, ctx)
-    return coords, np.stack([first, last]), np.array([times[0], times[-1]])
+        stepper.close()
+        if buf is not None:
+            buf.free()
+    _record(acc, what + (" (streaming)" if writer is not None else ""))
+    return np.stack(kept), np.array(times)
 
 
 def _solve_heat_1d_raw(length: float, nx: int, diffusivity: float, T_left: float, T_right: float,
@@ -189,30 +188,45 @@ def _solve_heat_3d_raw(Lx: float, Ly: float, Lz: float, nx: int, ny: int, nz: in
                        stream_to=None) -> TimeSeriesField:
     """3D heat equation on the box [0,Lx]x[0,Ly]x[0,Lz]; uniform or directional Dirichlet values."""
     cyl = geometry_type == "cylinder" and cylinder_radius is not None
-    has_core = core_radius is not None and core_diffusivity is not None
-    if cyl or has_core:
-        return _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady,
-                                source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
-                                geometry_type, cylinder_radius, T_left, T_right, T_side, core_radius,
-                                core_diffusivity, rtol, snapshot_stride, as_arrays, precond, u0=u0,
-                                stream_to=stream_to)
-    bc = mesh.heat_bc(3, T_boundary=T_boundary, T_left=T_left, T_right=T_right, T_side=T_side)
-    coords, values, times = _heat(3, [Lx, Ly, Lz], [nx, ny, nz], diffusivity, T_initial, dt, num_steps, steady,
-                                  source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
-                                  bc, rtol, precond, snapshot_stride, u0, stream_to=stream_to)
-    use_directional_bc = (T_left is not None or T_right is not None or T_side is not None)
+    core = (core_radius, core_diffusivity) if core_radius is not None and core_diffusivity is not None else None
+    special = cyl or core is not None
+    directional = T_left is not None or T_right is not None or T_side is not None
+    if special and directional and geometry_type == "cylinder":
+        # side_boundary_cylinder (:594-598) asks for near(r, R) on boundary facets away from the x ends; on the
+        # BoxMesh no facet has all vertices and its midpoint at r == R, so DOLFIN's topological search finds none
+        # and T_side constrains nothing; left / right are the x-end faces
+        bc = _lib.make_bc({f: v for f, v in ((0, T_left), (1, T_right)) if v is not None})
+    else:
+        bc = mesh.heat_bc(3, T_boundary=T_boundary, T_left=T_left, T_right=T_right, T_side=T_side)
+    if special:
+        coords, values, times = _heat_3d_special(
+            Lx=Lx, Ly=Ly, Lz=Lz, nx=nx, ny=ny, nz=nz, geometry_type=geometry_type, cylinder_radius=cylinder_radius,
+            cyl=cyl, core=core, bc=bc, diffusivity=diffusivity, T_initial=T_initial, dt=dt, num_steps=num_steps,
+            steady=steady, source_type=source_type, source_value=source_value, initial_type=initial_type,
+            initial_amplitude=initial_amplitude, initial_wavenumber=initial_wavenumber, rtol=rtol, precond=precond,
+            snapshot_stride=snapshot_stride, u0=u0, stream_to=stream_to)
+    else:
+        coords, values, times = _heat(3, [Lx, Ly, Lz], [nx, ny, nz], diffusivity, T_initial, dt, num_steps, steady,
+                                      source_type, source_value, initial_type, initial_amplitude, initial_wavenumber,
+                                      bc, rtol, precond, snapshot_stride, u0, stream_to=stream_to)
+    box = geometry_type == "box"
+    # the cylinder / core branch reports the cylinder's diameter as Ly and Lz whenever a radius is given
+    D = cylinder_radius * 2 if special and not box and cylinder_radius else None
     meta = {"name": "temperature", "unit": "°C", "pde": "heat",
-            "coordinate_system": "cartesian" if geometry_type == "box" else "cylindrical",
-            "Lx": Lx, "Ly": Ly, "Lz": Lz, "geometry_type": geometry_type, "source_type": source_type,
+            "coordinate_system": "cartesian" if box else "cylindrical", "Lx": Lx, "Ly": Ly if D is None else D,
+            "Lz": Lz if D is None else D, "geometry_type": geometry_type, "source_type": source_type,
             "source_value": source_value, "steady": steady}
-    if use_directional_bc:
-        for k, v in (("T_left", T_left), ("T_right", T_right), ("T_side", T_side)):
-            if v is not None:
-                meta[k] = v
+    if cyl:
+        meta["cylinder_radius"] = cylinder_radius
+    if directional:
+        meta.update({k: v for k, v in (("T_left", T_left), ("T_right", T_right), ("T_side", T_side)) if v is not None})
     else:
         meta["T_boundary"] = T_boundary
-    meta["diffusivity"] = diffusivity
-    return _finish(coords, values, times, 3, meta, as_arrays, n=[nx, ny, nz])
+    if core is not None:
+        meta.update(core_radius=core_radius, core_diffusivity=core_diffusivity, base_diffusivity=diffusivity)
+    else:
+        meta["diffusivity"] = diffusivity
+    return _finish(coords, values, times, 3, meta, as_arrays, n=None if special else [nx, ny, nz])
 
 
 def heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type="box", cylinder_radius=None):
@@ -224,40 +238,39 @@ def heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type="box", cylinder_radius=No
     return [int(nx), int(ny), int(nz)], [0.0, 0.0, 0.0], [float(Lx), float(Ly), float(Lz)]
 
 
-def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial, dt, num_steps, steady, source_type,
-                     source_value, initial_type, initial_amplitude, initial_wavenumber, geometry_type,
-                     cylinder_radius, T_left, T_right, T_side, core_radius, core_diffusivity, rtol, snapshot_stride,
-                     as_arrays, precond="jacobi", ctx=None, u0=None, stream_to=None):
+def _heat_3d_special(*, Lx, Ly, Lz, nx, ny, nz, geometry_type, cylinder_radius, cyl, core, bc, diffusivity, T_initial,
+                     dt, num_steps, steady, source_type, source_value, initial_type, initial_amplitude,
+                     initial_wavenumber, rtol, precond, snapshot_stride, u0, stream_to):
     """Cylinder / composite-core branches of _solve_heat_3d_raw (:512-572, 576-605, 642-645) as the reference's
     deployment runs them (no mshr in Dockerfile / requirements.txt, so MSHR_AVAILABLE is False): the "cylinder" is
     BoxMesh((0,-R,-R),(Lx,R,R), nx, int(ny*2R), int(nz*2R)) with every term weighted by
-    Expression("sqrt(x[1]^2+x[2]^2)", degree=2); the core is a DG0 diffusivity marked by SubDomain.mark."""
-    cyl = geometry_type == "cylinder" and cylinder_radius is not None
-    has_core = core_radius is not None and core_diffusivity is not None
+    Expression("sqrt(x[1]^2+x[2]^2)", degree=2); the core is a DG0 diffusivity marked by SubDomain.mark.
+    core: (radius, diffusivity) or None.  Returns (coords, values, times)."""
     n, lo, hi = heat_3d_grid(Lx, Ly, Lz, nx, ny, nz, geometry_type, cylinder_radius)
     if min(n) < 1:
         raise ValueError(f"BoxMesh needs at least one cell per axis, got {n}")
-    directional = T_left is not None or T_right is not None or T_side is not None
-    if not directional:
-        bc = mesh.heat_bc(3, T_boundary=T_boundary)
-    elif geometry_type == "cylinder":
-        # side_boundary_cylinder (:594-598) asks for near(r, R) on boundary facets away from the x ends; on the
-        # BoxMesh no facet has all vertices and its midpoint at r == R, so DOLFIN's topological search finds none
-        # and T_side constrains nothing; left / right are the x-end faces
-        bc = _lib.make_bc({f: v for f, v in ((0, T_left), (1, T_right)) if v is not None})
-    else:
-        bc = mesh.heat_bc(3, T_left=T_left, T_right=T_right, T_side=T_side)
+    p = _wheat_params(3, n, lo, hi, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value,
+                      snapshot_stride, weight=(0, 0, 2 if cyl else 1), weight_kind=1 if cyl else 0, core=core,
+                      initial_type=initial_type, initial_amplitude=initial_amplitude,
+                      initial_wavenumber=initial_wavenumber)
+    values, times = _wheat(p, rtol, precond, u0, stream_to, "heat solve (weighted box)")
+    return mesh.coordinates_box(3, n, lo, hi), values, times
+
+
+def _wheat_params(dim, n, lo, hi, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value,
+                  snapshot_stride, weight=(0, 0, 1), weight_kind=0, core=None, initial_type="constant",
+                  initial_amplitude=0.0, initial_wavenumber=0.0):
+    """WheatParams (pde_wheat_params).  weight: (r-power, sin(x1) factor, Expression degree) of a curvilinear
+    weight; weight_kind 1 is the cylinder's sqrt(x1^2 + x2^2); core: (radius, diffusivity) of a DG0 core or None."""
     p = _lib.WheatParams()
-    p.dim = 3
+    p.dim = dim
     p.n = _lib.i3(n)
     p.lo = _lib.d3(lo, 0.0)
     p.hi = _lib.d3(hi, 1.0)
-    p.weight_rpow, p.weight_sin_axis1 = 0, 0
-    p.weight_degree = 2 if cyl else 1
-    p.weight_kind = 1 if cyl else 0
-    p.has_core = 1 if has_core else 0
-    p.core_radius = float(core_radius) if has_core else 0.0
-    p.core_diffusivity = float(core_diffusivity) if has_core else 0.0
+    p.weight_rpow, p.weight_sin_axis1, p.weight_degree = weight
+    p.weight_kind = weight_kind
+    p.has_core = 1 if core is not None else 0
+    p.core_radius, p.core_diffusivity = (float(core[0]), float(core[1])) if core is not None else (0.0, 0.0)
     p.steady = 1 if steady else 0
     p.diffusivity = float(diffusivity)
     p.dt = float(dt)
@@ -269,29 +282,7 @@ def _heat_3d_special(Lx, Ly, Lz, nx, ny, nz, diffusivity, T_boundary, T_initial,
     p.initial_amplitude = float(initial_amplitude)
     p.initial_wavenumber = float(initial_wavenumber)
     p.bc = bc
-    values, times = _wheat(ctx, p, rtol, precond, u0, stream_to, "heat solve (weighted box)")
-    ctx = ctx or _lib.default_context()
-    coords = mesh.coordinates_box(3, n, lo, hi, ctx)
-    box = geometry_type == "box"
-    meta = {"name": "temperature", "unit": "°C", "pde": "heat",
-            "coordinate_system": "cartesian" if box else "cylindrical", "Lx": Lx,
-            "Ly": Ly if box else (cylinder_radius * 2 if cylinder_radius else Ly),
-            "Lz": Lz if box else (cylinder_radius * 2 if cylinder_radius else Lz),
-            "geometry_type": geometry_type, "source_type": source_type, "source_value": source_value,
-            "steady": steady}
-    if cyl:
-        meta["cylinder_radius"] = cylinder_radius
-    if directional:
-        for k, v in (("T_left", T_left), ("T_right", T_right), ("T_side", T_side)):
-            if v is not None:
-                meta[k] = v
-    else:
-        meta["T_boundary"] = T_boundary
-    if has_core:
-        meta.update(core_radius=core_radius, core_diffusivity=core_diffusivity, base_diffusivity=diffusivity)
-    else:
-        meta["diffusivity"] = diffusivity
-    return _finish(coords, values, times, 3, meta, as_arrays)
+    return p
 
 
 def _elasticity(dim, L, n, E, nu, body, quantity, plane_stress=True, area=1.0, rtol=1e-10, precond="auto",
@@ -368,10 +359,31 @@ def _solve_elasticity_3d_static(Lx: float, Ly: float, Lz: float, nx: int, ny: in
 # ----------------------------------------------------------------------------------------------------------
 # Curvilinear heat tools (reference :769-1464): the same loop on the coordinate-space mesh with one scalar weight
 # ----------------------------------------------------------------------------------------------------------
+def _cylindrical_rz(X):
+    coords = np.zeros((X.shape[0], 3))
+    coords[:, 0], coords[:, 2] = X[:, 0], X[:, 1]                 # (r, 0, z)
+    return coords
+
+
+def _spherical_xyz(X):
+    coords = np.zeros((X.shape[0], 3))
+    if X.shape[1] == 2:                                           # phi = 0: (r sin(theta), 0, r cos(theta))
+        coords[:, 0] = X[:, 0] * np.sin(X[:, 1])
+    else:
+        coords[:, 0] = X[:, 0] * np.sin(X[:, 1]) * np.cos(X[:, 2])
+        coords[:, 1] = X[:, 0] * np.sin(X[:, 1]) * np.sin(X[:, 2])
+    coords[:, 2] = X[:, 0] * np.cos(X[:, 1])
+    return coords
+
+
 _CURVI = {
-    # kind: (dim, weight r-power, sin(x1) factor, weight Expression degree)
-    "1d_cylindrical": (1, 1, 0, 1), "1d_spherical": (1, 2, 0, 2), "2d_cylindrical": (2, 1, 0, 1),
-    "2d_spherical": (2, 2, 1, 2), "3d_spherical": (3, 2, 1, 2),
+    # kind: (dim, weight r-power, sin(x1) factor, weight Expression degree, coordinate system, geometry_type without
+    #        and with an inner radius, map of the coordinate-space vertices to (x, y, z))
+    "1d_cylindrical": (1, 1, 0, 1, "cylindrical", "cylinder", "annulus", lambda X: _embed3(X, 1)),
+    "1d_spherical": (1, 2, 0, 2, "spherical", "sphere", "spherical_shell", lambda X: _embed3(X, 1)),
+    "2d_cylindrical": (2, 1, 0, 1, "cylindrical", "cylinder", "annular_cylinder", _cylindrical_rz),
+    "2d_spherical": (2, 2, 1, 2, "spherical", "sphere", "spherical_shell", _spherical_xyz),
+    "3d_spherical": (3, 2, 1, 2, "spherical", "sphere", "spherical_shell", _spherical_xyz),
 }
 
 
@@ -383,115 +395,46 @@ def curvilinear_grid(kind, r_inner, r_outer, n, z_length=None):
     return [int(k) for k in n], [r_inner] + [0.0] * len(rest), [r_outer] + rest
 
 
-def _wheat_precond(precond):
-    """Weighted operators: "gmg" selects Galerkin multigrid; "auto" still means Jacobi-PCG for them."""
-    if precond not in _lib.PRECOND:
-        raise ValueError(f"precond must be one of {sorted(_lib.PRECOND)}, got {precond!r}")
-    return "gmg" if precond == "gmg" else "jacobi"
-
-
-def _wheat(ctx, p, rtol, precond, u0, writer, what):
+def _wheat(p, rtol, precond, u0, writer, what):
     """(values, times) of the weighted solve p.  A plain call is one pde_wheat_solve.  With a host initial field u0
-    (natural vertex order) or a snapshot writer it runs on the resident stepper (pde_wheat_open / set_state / step /
-    get_state), as _heat_streaming does for the box: every kept snapshot goes through one pinned buffer to the writer,
-    which leaves the first and last one in the result.  Steady solves never stream; u0 is their starting guess."""
+    (natural vertex order) or a snapshot writer it runs on the resident stepper (_run_stepper).  Steady solves never
+    stream; u0 is their starting guess."""
     nv = int(np.prod([int(p.n[q]) + 1 for q in range(int(p.dim))]))
     if u0 is not None:
         u0 = np.ascontiguousarray(u0, dtype=np.float64)
         if u0.shape != (nv,):
             raise ValueError(f"u0 must hold one value per mesh vertex ({nv}), got shape {u0.shape}")
-    ctx = ctx or _lib.default_context()
-    steady = bool(p.steady)
-    if steady:
+    ctx = _lib.default_context()
+    if p.steady:
         writer = None
-    stride = max(1, int(p.snapshot_stride))
-    o = _lib.make_opts(rtol=rtol, precond=_wheat_precond(precond))
-    L = _lib.lib()
-    if u0 is None and writer is None:
-        nsnap = 1 if steady else 1 + int(p.num_steps) // stride
-        values = np.empty((nsnap, nv), dtype=np.float64)
-        times = np.empty(nsnap, dtype=np.float64)
-        st = _lib.Stats()
-        _lib.check(L.pde_wheat_solve(ctx.handle, C.byref(p), C.byref(o), _lib.ptr(values), _lib.ptr(times),
-                                     C.byref(st)))
-        _record(st.as_dict(), what)
-        return values, times
-    h = C.c_void_p()
-    _lib.check(L.pde_wheat_open(ctx.handle, C.byref(p), C.byref(o), C.byref(h)))
-    buf = _lib.PinnedArray(nv) if writer is not None else None
-    acc = {"iters_total": 0, "solves": 0, "converged": 1, "solve_ms": 0.0, "launches": 0}
-    kept, times = [], []
-
-    def keep(t):
-        out = buf.array if writer is not None else np.empty(nv, dtype=np.float64)
-        _lib.check(L.pde_wheat_get_state(h, _lib.ptr(out)))
-        times.append(t)
-        if writer is None:
-            kept.append(out)
-            return
-        writer.append(t, out)
-        if len(kept) < 2:
-            kept.append(out.copy())
-        else:
-            kept[1][:] = out
-
-    try:
-        if u0 is not None:
-            _lib.check(L.pde_wheat_set_state(h, _lib.ptr(u0)))
-        if not steady:
-            keep(0.0)
-        st = _lib.Stats()
-        for step in range(1 if steady else int(p.num_steps)):
-            _lib.check(L.pde_wheat_step(h, 1, C.byref(st)))
-            d = st.as_dict()
-            for k in ("iters_total", "solves", "solve_ms", "launches"):
-                acc[k] += d[k]
-            acc["converged"] &= d["converged"]
-            acc.update(ndofs=d["ndofs"], levels=d["levels"], final_relres=d["final_relres"], setup_ms=d["setup_ms"],
-                       true_relres=d["true_relres"])
-            if steady:
-                keep(0.0)
-            elif (step + 1) % stride == 0:
-                keep((step + 1) * p.dt)
-    finally:
-        L.pde_wheat_close(h)
-        if buf is not None:
-            buf.free()
-    _record(acc, what + (" (streaming)" if writer is not None else ""))
-    if writer is not None:
-        return np.stack([kept[0], kept[-1]]), np.array([times[0], times[-1]])
-    return np.stack(kept), np.array(times)
+    if precond not in _lib.PRECOND:
+        raise ValueError(f"precond must be one of {sorted(_lib.PRECOND)}, got {precond!r}")
+    # "gmg" selects Galerkin multigrid; "auto" still means Jacobi-PCG for the weighted operators
+    o = _lib.make_opts(rtol=rtol, precond="gmg" if precond == "gmg" else "jacobi")
+    if u0 is not None or writer is not None:
+        return _run_stepper(_lib.WheatStepper(ctx, p, o), p, u0, writer, what)
+    return _solve_in_memory(_lib.lib().pde_wheat_solve, ctx, p, o, nv, what)
 
 
-def _curvilinear(kind, lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                 snapshot_stride=1, ctx=None, precond="jacobi", u0=None, stream_to=None):
-    dim, rpow, wsin, wdeg = _CURVI[kind]
-    p = _lib.WheatParams()
-    p.dim = dim
-    p.n = _lib.i3(n)
-    p.lo = _lib.d3(lo, 0.0)
-    p.hi = _lib.d3(hi, 1.0)
-    p.weight_rpow, p.weight_sin_axis1, p.weight_degree = rpow, wsin, wdeg
-    p.steady = 1 if steady else 0
-    p.diffusivity = float(diffusivity)
-    p.dt = float(dt)
-    p.num_steps = int(num_steps)
-    p.snapshot_stride = int(snapshot_stride)
-    p.source_value = float(source_value) if source_type == "constant" else 0.0
-    p.T_initial = float(T_initial)
-    p.bc = bc
-    values, times = _wheat(ctx, p, rtol, precond, u0, stream_to, "curvilinear heat solve")
-    ctx = ctx or _lib.default_context()
-    X = mesh.coordinates_box(dim, n, lo, hi, ctx)
-    return X, values, times
-
-
-def _curvi_meta(system, geometry, r_inner, r_outer, source_type, source_value, steady, **extra):
+def _curvilinear(kind, r_inner, r_outer, n, bc, diffusivity, T_initial, dt, num_steps, steady, source_type,
+                 source_value, *, rtol, precond, snapshot_stride, as_arrays, u0, stream_to, z_length=None):
+    """One curvilinear tool: the weighted solve on the coordinate-space mesh of curvilinear_grid, its vertices mapped
+    to (x, y, z); the 1-D tools sort the vertices by r as the reference does."""
+    dim, rpow, wsin, wdeg, system, solid, hollow, to_xyz = _CURVI[kind]
+    n, lo, hi = curvilinear_grid(kind, r_inner, r_outer, n, z_length)
+    p = _wheat_params(dim, n, lo, hi, bc, diffusivity, T_initial, dt, num_steps, steady, source_type, source_value,
+                      snapshot_stride, weight=(rpow, wsin, wdeg))
+    values, times = _wheat(p, rtol, precond, u0, stream_to, "curvilinear heat solve")
+    X = mesh.coordinates_box(dim, n, lo, hi)
+    if dim == 1:
+        order = np.argsort(X[:, 0], kind="stable")
+        X, values = X[order], values[:, order]
     meta = {"name": "temperature", "unit": "°C", "pde": "heat", "coordinate_system": system,
-            "geometry_type": geometry, "r_inner": r_inner, "r_outer": r_outer}
-    meta.update(extra)
+            "geometry_type": solid if r_inner < 1e-10 else hollow, "r_inner": r_inner, "r_outer": r_outer}
+    if z_length is not None:
+        meta["z_length"] = z_length
     meta.update({"source_type": source_type, "source_value": source_value, "steady": steady})
-    return meta
+    return _finish(to_xyz(X), values, times, dim, meta, as_arrays)
 
 
 def _radial_bc(r_inner, T_inner, T_outer):
@@ -508,14 +451,9 @@ def _solve_heat_1d_cylindrical_raw(r_inner: float, r_outer: float, nr: int, diff
                                    rtol: float = 1e-10, precond: str = "jacobi", snapshot_stride: int = 1,
                                    as_arrays: Optional[bool] = None, u0=None, stream_to=None) -> TimeSeriesField:
     """1D radial heat equation in cylindrical coordinates, weight r (:769-920)."""
-    n, lo, hi = curvilinear_grid("1d_cylindrical", r_inner, r_outer, [nr])
-    X, values, times = _curvilinear("1d_cylindrical", lo, hi, n, _radial_bc(r_inner, T_inner, T_outer), diffusivity,
-                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
-    order = np.argsort(X[:, 0], kind="stable")
-    meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annulus", r_inner, r_outer, source_type,
-                       source_value, steady)
-    return _finish(_embed3(X[order], 1), values[:, order], times, 1, meta, as_arrays)
+    return _curvilinear("1d_cylindrical", r_inner, r_outer, [nr], _radial_bc(r_inner, T_inner, T_outer), diffusivity,
+                        T_initial, dt, num_steps, steady, source_type, source_value, rtol=rtol, precond=precond,
+                        snapshot_stride=snapshot_stride, as_arrays=as_arrays, u0=u0, stream_to=stream_to)
 
 
 def _solve_heat_1d_spherical_raw(r_inner: float, r_outer: float, nr: int, diffusivity: float, T_inner: float,
@@ -525,14 +463,9 @@ def _solve_heat_1d_spherical_raw(r_inner: float, r_outer: float, nr: int, diffus
                                  snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
                                  stream_to=None) -> TimeSeriesField:
     """1D radial heat equation in spherical coordinates, weight r^2 (:926-1057)."""
-    n, lo, hi = curvilinear_grid("1d_spherical", r_inner, r_outer, [nr])
-    X, values, times = _curvilinear("1d_spherical", lo, hi, n, _radial_bc(r_inner, T_inner, T_outer), diffusivity,
-                                    T_initial, dt, num_steps, steady, source_type, source_value, rtol,
-                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
-    order = np.argsort(X[:, 0], kind="stable")
-    meta = _curvi_meta("spherical", "sphere" if r_inner < 1e-10 else "spherical_shell", r_inner, r_outer, source_type,
-                       source_value, steady)
-    return _finish(_embed3(X[order], 1), values[:, order], times, 1, meta, as_arrays)
+    return _curvilinear("1d_spherical", r_inner, r_outer, [nr], _radial_bc(r_inner, T_inner, T_outer), diffusivity,
+                        T_initial, dt, num_steps, steady, source_type, source_value, rtol=rtol, precond=precond,
+                        snapshot_stride=snapshot_stride, as_arrays=as_arrays, u0=u0, stream_to=stream_to)
 
 
 def _solve_heat_2d_cylindrical_raw(r_inner: float, r_outer: float, z_length: float, nr: int, nz: int,
@@ -542,16 +475,10 @@ def _solve_heat_2d_cylindrical_raw(r_inner: float, r_outer: float, z_length: flo
                                    rtol: float = 1e-10, precond: str = "jacobi", snapshot_stride: int = 1,
                                    as_arrays: Optional[bool] = None, u0=None, stream_to=None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, z) plane, weight r (:1063-1185)."""
-    bc = _lib.make_bc({f: T_boundary for f in range(4)})
-    n, lo, hi = curvilinear_grid("2d_cylindrical", r_inner, r_outer, [nr, nz], z_length)
-    X, values, times = _curvilinear("2d_cylindrical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
-                                    source_type, source_value, rtol,
-                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
-    coords = np.zeros((X.shape[0], 3))
-    coords[:, 0], coords[:, 2] = X[:, 0], X[:, 1]                 # (r, 0, z)
-    meta = _curvi_meta("cylindrical", "cylinder" if r_inner < 1e-10 else "annular_cylinder", r_inner, r_outer,
-                       source_type, source_value, steady, z_length=z_length)
-    return _finish(coords, values, times, 2, meta, as_arrays)
+    return _curvilinear("2d_cylindrical", r_inner, r_outer, [nr, nz], _lib.make_bc({f: T_boundary for f in range(4)}),
+                        diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol=rtol,
+                        precond=precond, snapshot_stride=snapshot_stride, as_arrays=as_arrays, u0=u0,
+                        stream_to=stream_to, z_length=z_length)
 
 
 def _solve_heat_2d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta: int, diffusivity: float,
@@ -561,17 +488,10 @@ def _solve_heat_2d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta
                                  snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
                                  stream_to=None) -> TimeSeriesField:
     """2D axisymmetric heat equation in the (r, theta) plane, weight r^2 sin(theta) (:1191-1320)."""
-    bc = _lib.make_bc({f: T_boundary for f in range(4)})
-    n, lo, hi = curvilinear_grid("2d_spherical", r_inner, r_outer, [nr, ntheta])
-    X, values, times = _curvilinear("2d_spherical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
-                                    source_type, source_value, rtol,
-                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
-    coords = np.zeros((X.shape[0], 3))
-    coords[:, 0] = X[:, 0] * np.sin(X[:, 1])                      # phi = 0: (r sin(theta), 0, r cos(theta))
-    coords[:, 2] = X[:, 0] * np.cos(X[:, 1])
-    meta = _curvi_meta("spherical", "sphere" if r_inner < 1e-10 else "spherical_shell", r_inner, r_outer, source_type,
-                       source_value, steady)
-    return _finish(coords, values, times, 2, meta, as_arrays)
+    return _curvilinear("2d_spherical", r_inner, r_outer, [nr, ntheta], _lib.make_bc({f: T_boundary for f in range(4)}),
+                        diffusivity, T_initial, dt, num_steps, steady, source_type, source_value, rtol=rtol,
+                        precond=precond, snapshot_stride=snapshot_stride, as_arrays=as_arrays, u0=u0,
+                        stream_to=stream_to)
 
 
 def _solve_heat_3d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta: int, nphi: int, diffusivity: float,
@@ -581,15 +501,7 @@ def _solve_heat_3d_spherical_raw(r_inner: float, r_outer: float, nr: int, ntheta
                                  snapshot_stride: int = 1, as_arrays: Optional[bool] = None, u0=None,
                                  stream_to=None) -> TimeSeriesField:
     """3D heat equation in (r, theta, phi), weight r^2 sin(theta) (:1326-1464)."""
-    bc = _lib.make_bc({f: T_boundary for f in range(6)})
-    n, lo, hi = curvilinear_grid("3d_spherical", r_inner, r_outer, [nr, ntheta, nphi])
-    X, values, times = _curvilinear("3d_spherical", lo, hi, n, bc, diffusivity, T_initial, dt, num_steps, steady,
-                                    source_type, source_value, rtol,
-                                    snapshot_stride=snapshot_stride, precond=precond, u0=u0, stream_to=stream_to)
-    coords = np.empty((X.shape[0], 3))
-    coords[:, 0] = X[:, 0] * np.sin(X[:, 1]) * np.cos(X[:, 2])
-    coords[:, 1] = X[:, 0] * np.sin(X[:, 1]) * np.sin(X[:, 2])
-    coords[:, 2] = X[:, 0] * np.cos(X[:, 1])
-    meta = _curvi_meta("spherical", "sphere" if r_inner < 1e-10 else "spherical_shell", r_inner, r_outer, source_type,
-                       source_value, steady)
-    return _finish(coords, values, times, 3, meta, as_arrays)
+    return _curvilinear("3d_spherical", r_inner, r_outer, [nr, ntheta, nphi],
+                        _lib.make_bc({f: T_boundary for f in range(6)}), diffusivity, T_initial, dt, num_steps, steady,
+                        source_type, source_value, rtol=rtol, precond=precond, snapshot_stride=snapshot_stride,
+                        as_arrays=as_arrays, u0=u0, stream_to=stream_to)

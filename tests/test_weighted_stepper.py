@@ -305,30 +305,8 @@ def _params(P, name):
     return p
 
 
-class _Stepper:
-    def __init__(self, P, p, precond):
-        self.L = P._lib
-        self.h = C.c_void_p()
-        o = self.L.make_opts(precond=precond)
-        self.L.check(self.L.lib().pde_wheat_open(self.L.default_context().handle, C.byref(p), C.byref(o),
-                                                 C.byref(self.h)))
-        self.nv = int(self.L.lib().pde_wheat_local_nverts(self.h))
-
-    def step(self, k):
-        st = self.L.Stats()
-        self.L.check(self.L.lib().pde_wheat_step(self.h, int(k), C.byref(st)))
-        return st.as_dict()
-
-    def set_state(self, u):
-        self.L.check(self.L.lib().pde_wheat_set_state(self.h, self.L.ptr(np.ascontiguousarray(u, dtype=np.float64))))
-
-    def get_state(self):
-        out = np.empty(self.nv)
-        self.L.check(self.L.lib().pde_wheat_get_state(self.h, self.L.ptr(out)))
-        return out
-
-    def close(self):
-        self.L.lib().pde_wheat_close(self.h)
+def _stepper(P, p, precond):
+    return P._lib.WheatStepper(P._lib.default_context(), p, P._lib.make_opts(precond=precond))
 
 
 @pytest.mark.gpu
@@ -336,17 +314,17 @@ class _Stepper:
 @pytest.mark.parametrize("name", ["2d_spherical", "cylinder_core"])
 def test_set_state_restarts_cleanly(P, name, precond):
     p = _params(P, name)
-    a = _Stepper(P, p, precond)
-    b = _Stepper(P, p, precond)
+    a = _stepper(P, p, precond)
+    b = _stepper(P, p, precond)
     try:
-        assert a.nv == (33 * 33 if name == "2d_spherical" else 9 * 17 * 17)
-        u0 = np.random.default_rng(11).standard_normal(a.nv)
+        assert a.nloc == (33 * 33 if name == "2d_spherical" else 9 * 17 * 17)
+        u0 = np.random.default_rng(11).standard_normal(a.nloc)
         a.step(3)
         a.set_state(u0)
         a.step(2)
         b.set_state(u0)
         b.step(2)
-        assert np.array_equal(a.get_state(), b.get_state())
+        assert np.array_equal(a.get_state(np.empty(a.nloc)), b.get_state(np.empty(b.nloc)))
     finally:
         a.close()
         b.close()
@@ -364,7 +342,7 @@ def test_set_state_restarts_cleanly(P, name, precond):
 @pytest.mark.parametrize("name", ["2d_spherical", "cylinder_core"])
 def test_streamed_gmg_stats(P, name, tmp_path):
     from pde_solver_b200 import io
-    s = _Stepper(P, _params(P, name), "gmg")
+    s = _stepper(P, _params(P, name), "gmg")
     try:
         per_step = [s.step(1)["iters_total"] for _ in range(6)]
     finally:
