@@ -286,6 +286,32 @@ int pde_op_solve(pde_ctx* ctx, const pde_op_params* p, const pde_solver_opts* o,
 int pde_op_manufactured(pde_ctx* ctx, const pde_op_params* p, const pde_solver_opts* o, double* rel_l2_error,
                         pde_stats* st);
 
+/* ---- multigrid V-cycle test entry points ---------------------------------------------------------------------
+ * The V-cycle is a fixed linear map z = B b.  These entries build the hierarchy the solver builds, apply B to a host
+ * vector `ncycles` times and return it, so that tests can compare B with a model of it vector by vector. */
+#define PDE_MG_MAX_LEVELS 16
+/* paths bits: fused kernels a level actually ran (k_sweep / generic FIRST2 pass of the first two pre-smoothing
+ * sweeps, k_heat_post2, round-1 k_post2, k_heat_post2 residual + restriction) */
+enum { PDE_MG_FIRST2 = 1, PDE_MG_HEAT_POST2 = 2, PDE_MG_POST2_R1 = 4, PDE_MG_RESID_RESTRICT = 8 };
+typedef struct pde_mg_info {
+  int32_t levels, n_dense;
+  int32_t graph;                        /* 1: the last cycle replayed a captured CUDA graph */
+  int32_t reserved;
+  int32_t n[PDE_MG_MAX_LEVELS][3];      /* cells per user axis of each level (0 for absent axes) */
+  double lmax[PDE_MG_MAX_LEVELS];       /* Chebyshev upper bound each level used */
+  uint32_t paths[PDE_MG_MAX_LEVELS];    /* PDE_MG_* bits, accumulated over the cycles of the call */
+} pde_mg_info;
+/* Box operators (heat / elasticity): the hierarchy of pde_op_solve's GMG path (nu and ratio from o, with the same
+ * environment overrides), run ncycles >= 1 times on the same b with the fused b.z of the PCG.  This always runs the
+ * hierarchy's cycle, a one-level hierarchy included.  b, z_first (cycle 1), z_last (cycle ncycles): host arrays
+ * [ncomp][nverts], natural order; bz (may be NULL): the fused b.z of the last cycle (free rows).  One GPU only. */
+int pde_op_vcycle(pde_ctx* ctx, const pde_op_params* p, const pde_solver_opts* o, int32_t ncycles, const double* b,
+                  double* z_first, double* z_last, double* bz, pde_mg_info* info);
+/* The same for the weighted operators of pde_wheat_solve (the steady / backward-Euler matrix of p) and their Galerkin
+ * hierarchy; paths stay 0, graph is 0.  Non-zero if the grid does not coarsen (the solve runs Jacobi-PCG then). */
+int pde_wheat_vcycle(pde_ctx* ctx, const pde_wheat_params* p, int32_t ncycles, const double* b, double* z_first,
+                     double* z_last, double* bz, pde_mg_info* info);
+
 #ifdef __cplusplus
 }
 #endif

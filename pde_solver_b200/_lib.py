@@ -63,6 +63,22 @@ class OpParams(C.Structure):
                 ("bc", Bc), ("variant", C.c_int32)]
 
 
+MG_MAX_LEVELS = 16
+MG_PATHS = {"first2": 1, "heat_post2": 2, "post2_r1": 4, "resid_restrict": 8}
+
+
+class MgInfo(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("n_dense", C.c_int32), ("graph", C.c_int32), ("reserved", C.c_int32),
+                ("n", (C.c_int32 * 3) * MG_MAX_LEVELS), ("lmax", C.c_double * MG_MAX_LEVELS),
+                ("paths", C.c_uint32 * MG_MAX_LEVELS)]
+
+    def as_dict(self):
+        nl = self.levels
+        return {"levels": nl, "n_dense": self.n_dense, "graph": self.graph,
+                "n": [list(self.n[l]) for l in range(nl)], "lmax": [self.lmax[l] for l in range(nl)],
+                "paths": [int(self.paths[l]) for l in range(nl)]}
+
+
 PRECOND = {"jacobi": 0, "gmg": 1, "auto": 2}
 IC = {"constant": 0, "zero": 1, "cosine": 2, "sine": 3, "array": 4}
 OP = {"heat": 0, "mass": 1, "stiffness": 2, "elasticity": 3}
@@ -97,7 +113,7 @@ def lib():
                      "pde_heat_close", "pde_elasticity_solve", "pde_op_table", "pde_op_apply", "pde_op_bench", "pde_op_sweep", "pde_op_bench_mode", "pde_comm_info", "pde_device_count",
                      "pde_op_solve", "pde_version", "pde_host_alloc", "pde_host_free", "pde_slab_partition", "pde_op_manufactured", "pde_halo_bench", "pde_wheat_solve", "pde_wheat_level_coefs",
                      "pde_wheat_open", "pde_wheat_set_state", "pde_wheat_step", "pde_wheat_get_state", "pde_wheat_close",
-                     "pde_mesh_coords_box"):
+                     "pde_mesh_coords_box", "pde_op_vcycle", "pde_wheat_vcycle"):
             getattr(L, name).restype = C.c_int
         _lib = L
     return _lib
@@ -287,6 +303,27 @@ def op_solve(ctx, p, b, opts=None):
     o = opts if opts is not None else make_opts()
     check(lib().pde_op_solve(ctx.handle, C.byref(p), C.byref(o), ptr(b), ptr(x), C.byref(st)))
     return x, st.as_dict()
+
+
+def _vcycle(fn, b, ncycles):
+    b = np.ascontiguousarray(b, dtype=np.float64)
+    z_first, z_last = np.empty_like(b), np.empty_like(b)
+    bz = C.c_double()
+    info = MgInfo()
+    check(fn(int(ncycles), ptr(b), ptr(z_first), ptr(z_last), C.byref(bz), C.byref(info)))
+    return z_first, z_last, bz.value, info.as_dict()
+
+
+def op_vcycle(ctx, p, b, opts=None, ncycles=3):
+    """The GMG V-cycle of op_solve applied `ncycles` times to b [ncomp][nverts] (see pde_op_vcycle in
+    include/pde_b200.h); returns (z of cycle 1, z of the last cycle, fused b.z of the last cycle, info dict)."""
+    o = C.byref(opts) if opts is not None else None
+    return _vcycle(lambda *a: lib().pde_op_vcycle(ctx.handle, C.byref(p), o, *a), b, ncycles)
+
+
+def wheat_vcycle(ctx, p, b, ncycles=3):
+    """As op_vcycle for the weighted operators of WheatParams and their Galerkin hierarchy."""
+    return _vcycle(lambda *a: lib().pde_wheat_vcycle(ctx.handle, C.byref(p), *a), b, ncycles)
 
 
 def comm_info(ctx):

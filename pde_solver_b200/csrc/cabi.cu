@@ -800,6 +800,19 @@ extern "C" int pde_op_bench_mode(pde_ctx* c, const pde_op_params* p, int mode, i
   return 0;
 }
 
+// the GMG hierarchy of the operator solves: levels from the operator, smoother degree and ratio from o and the
+// environment
+static int build_hierarchy(pde_ctx* c, OpGuard& G, const pde_op_params* p, const pde_solver_opts& o) {
+  double p0 = p->kind == PDE_OP_ELASTICITY ? p->lam : (p->kind == PDE_OP_MASS ? 1.0 : (p->kind == PDE_OP_STIFFNESS ? 0.0 : p->alpha));
+  double p1 = p->kind == PDE_OP_ELASTICITY ? p->mu : (p->kind == PDE_OP_MASS ? 0.0 : (p->kind == PDE_OP_STIFFNESS ? 1.0 : p->beta));
+  PDE_OK(G.mg.build(c, G.A, p->kind == PDE_OP_ELASTICITY ? PDE_OP_ELASTICITY : PDE_OP_HEAT, p0, p1));
+  G.mg.nu = o.cheby_degree > 0 ? o.cheby_degree : 2;
+  G.mg.ratio = o.cheby_ratio > 1 ? o.cheby_ratio : 8.0;
+  if (const char* e = getenv("PDE_B200_CHEBY_DEGREE")) G.mg.nu = atoi(e) > 0 ? atoi(e) : G.mg.nu;
+  if (const char* e = getenv("PDE_B200_CHEBY_RATIO")) G.mg.ratio = atof(e) > 1 ? atof(e) : G.mg.ratio;
+  return 0;
+}
+
 static int solve_with(pde_ctx* c, OpGuard& G, const pde_op_params* p, const pde_solver_opts& o, double* x, double* r,
                       double bn2, pde_stats* st) {
   const int nc = G.A.tab.ncomp;
@@ -813,13 +826,7 @@ static int solve_with(pde_ctx* c, OpGuard& G, const pde_op_params* p, const pde_
   int rc = 0;
   do {
     if (o.precond != PDE_PRECOND_JACOBI) {
-      double p0 = p->kind == PDE_OP_ELASTICITY ? p->lam : (p->kind == PDE_OP_MASS ? 1.0 : (p->kind == PDE_OP_STIFFNESS ? 0.0 : p->alpha));
-      double p1 = p->kind == PDE_OP_ELASTICITY ? p->mu : (p->kind == PDE_OP_MASS ? 0.0 : (p->kind == PDE_OP_STIFFNESS ? 1.0 : p->beta));
-      if ((rc = G.mg.build(c, G.A, p->kind == PDE_OP_ELASTICITY ? PDE_OP_ELASTICITY : PDE_OP_HEAT, p0, p1))) break;
-      G.mg.nu = o.cheby_degree > 0 ? o.cheby_degree : 2;
-      G.mg.ratio = o.cheby_ratio > 1 ? o.cheby_ratio : 8.0;
-      if (const char* e = getenv("PDE_B200_CHEBY_DEGREE")) G.mg.nu = atoi(e) > 0 ? atoi(e) : G.mg.nu;
-      if (const char* e = getenv("PDE_B200_CHEBY_RATIO")) G.mg.ratio = atof(e) > 1 ? atof(e) : G.mg.ratio;
+      if ((rc = build_hierarchy(c, G, p, o))) break;
       use_mg = choose_precond(o, c, ndofs, G.mg) == PDE_PRECOND_GMG;
     }
     if ((rc = G.w.alloc(c, G.A.g, nc))) break;
@@ -883,6 +890,55 @@ extern "C" int pde_op_solve(pde_ctx* c, const pde_op_params* p, const pde_solver
   PDE_OK(launch_pack(c, g, nc, G.x.p, (double*)dense.p, 0));
   PDE_OK(d2h(c, x, dense.p, sizeof(double) * nloc * nc));
   if (st_out) *st_out = st;
+  return 0;
+}
+
+// Test entry: the V-cycle of pde_op_solve's GMG path applied ncycles times to one host vector (see the header).  The
+// cycles after the first replay the CUDA graph of the levels below level 0 where the hierarchy captures one.
+extern "C" int pde_op_vcycle(pde_ctx* c, const pde_op_params* p, const pde_solver_opts* o_in, int32_t ncycles,
+                             const double* b, double* z_first, double* z_last, double* bz, pde_mg_info* info) {
+  if (!c || !p || !b || !z_first || !z_last || !info) PDE_FAIL("null argument");
+  if (ncycles < 1) PDE_FAIL("ncycles must be >= 1");
+  if (c->world > 1) PDE_FAIL("pde_op_vcycle runs on one GPU");
+  CUDA_OK(cudaSetDevice(c->device));
+  pde_solver_opts o;
+  if (o_in) o = *o_in; else pde_solver_opts_default(&o);
+  OpGuard G;
+  int nc;
+  PDE_OK(setup_op(c, p, &G.A, &nc));
+  const Grid& g = G.A.g;
+  PDE_OK(G.y.alloc(c, g, nc));  // holds b
+  const long long nloc = (long long)g.nn[0] * g.nn[1] * g.nzl;
+  const size_t bytes = sizeof(double) * nloc * nc;
+  DevMem dense;
+  PDE_OK(dense.alloc(bytes));
+  PDE_OK(h2d(c, dense.p, b, bytes));
+  PDE_OK(launch_unpack(c, g, nc, (const double*)dense.p, G.y.p, 0));
+  PDE_OK(build_hierarchy(c, G, p, o));
+  const int nl = G.mg.levels();
+  if (nl > PDE_MG_MAX_LEVELS) PDE_FAIL("more multigrid levels than pde_mg_info holds");
+  for (int k = 0; k < ncycles; ++k) {
+    double* z = nullptr;
+    bool fused = false;
+    PDE_OK(G.mg.vcycle(c, G.A, G.y.p, &z, S_RHO0, &fused));
+    if (!fused) PDE_OK(launch_dot(c, g, nc, G.y.p, z, S_RHO0));
+    if (k == 0 || k == ncycles - 1) PDE_OK(launch_pack(c, g, nc, z, (double*)dense.p, 0));
+    if (k == 0) PDE_OK(d2h(c, z_first, dense.p, bytes));
+    if (k == ncycles - 1) PDE_OK(d2h(c, z_last, dense.p, bytes));
+  }
+  if (bz) PDE_OK(read_scal(c, S_RHO0, 1, bz));
+  std::memset(info, 0, sizeof(*info));
+  info->levels = nl;
+  info->n_dense = G.mg.lv[nl - 1]->n_dense;
+  info->graph = G.mg.gstate == 2;
+  int ax[3], nax;
+  internal_axes(p->dim, ax, &nax);
+  for (int l = 0; l < nl; ++l) {
+    const MGLevel& L = *G.mg.lv[l];
+    for (int q = 0; q < nax; ++q) info->n[l][q] = L.op.g.nc[ax[q]];
+    info->lmax[l] = L.op.dev.gershgorin;
+    info->paths[l] = L.paths;
+  }
   return 0;
 }
 

@@ -446,6 +446,7 @@ static int smooth(pde_ctx* c, MGLevel& L, const double* b, double** cur, double*
     if (dot_slot >= 0 && sweeps == 2) { a.reduce_slot_xy = dot_slot; if (dot_done) *dot_done = true; }
     if (c->world > 1) PDE_OK(comm_halo_exchange(c, L.op.g, L.op.dev.ncomp, const_cast<double*>(b)));
     PDE_OK(launch_stencil(c, L.op.g, L.op.bc, L.op.dev, a));
+    L.paths |= PDE_MG_FIRST2;
     k0 = 2;
     prev_mode = 3;     // x_1 = s0 D^-1 b
   } else if (zero_guess) {
@@ -468,7 +469,12 @@ static int smooth(pde_ctx* c, MGLevel& L, const double* b, double** cur, double*
       PDE_OK(comm_halo_exchange(c, L.op.g, 1, const_cast<double*>(b), 1));
     }
     PDE_OK(launch_heat_post2(c, L.op.g, L.op.dev, *cur, b, *oth, c2a, c1b, c2b, dot_slot, &handled));
-    if (!handled) PDE_OK(launch_post2(c, L.op.g, L.op.bc, L.op.dev, *cur, b, *oth, c2a, c1b, c2b, dot_slot, &handled));
+    if (handled) {
+      L.paths |= PDE_MG_HEAT_POST2;
+    } else {
+      PDE_OK(launch_post2(c, L.op.g, L.op.bc, L.op.dev, *cur, b, *oth, c2a, c1b, c2b, dot_slot, &handled));
+      if (handled) L.paths |= PDE_MG_POST2_R1;
+    }
     if (handled) {
       std::swap(*cur, *oth);
       if (dot_slot >= 0 && dot_done) *dot_done = true;
@@ -532,6 +538,7 @@ int Hierarchy::vcycle(pde_ctx* c, const Operator& fine, const double* b0, double
     double* bct = window ? Lc.b.p + gc.plane * Lc.gslab.z0 : Lc.b.p;
     bool fused = false;
     if (c->world == 1 || lean[l]) PDE_OK(launch_heat_resid_restrict(c, L.op.g, gct, L.op.dev, cur[l], b, bct, &fused));
+    if (fused) L.paths |= PDE_MG_RESID_RESTRICT;
     if (!fused) {
       StencilArgs a;
       a.x = cur[l]; a.b = b; a.y = L.r.p; a.bscale = 1.0; a.ascale = -1.0;

@@ -35,6 +35,7 @@ struct MGLevel {
   double* Ainv = nullptr;
   long long* idx = nullptr;   // flat local index of global free dof j (-1: owned by another rank)
   double* bglob = nullptr;    // multi-rank: global coarse right-hand side (all-reduced)
+  uint32_t paths = 0;         // PDE_MG_* bits of the fused kernels this level ran (pde_op_vcycle reports them)
 };
 
 struct Hierarchy {

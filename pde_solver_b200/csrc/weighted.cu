@@ -624,3 +624,43 @@ extern "C" int pde_wheat_level_coefs(pde_ctx* c, const pde_wheat_params* p, int 
   if (coef_out) PDE_OK(wmg_level_coefs(c, mg, level, coef_out));
   return 0;
 }
+
+// Test entry: the V-cycle of pde_wheat_solve's GMG path applied ncycles times to one host vector (see the header)
+extern "C" int pde_wheat_vcycle(pde_ctx* c, const pde_wheat_params* p, int32_t ncycles, const double* b, double* z_first,
+                                double* z_last, double* bz, pde_mg_info* info) {
+  if (!c || !p || !b || !z_first || !z_last || !info) PDE_FAIL("null argument");
+  if (ncycles < 1) PDE_FAIL("ncycles must be >= 1");
+  WheatState s;
+  double L[3];
+  PDE_OK(wheat_assemble(c, p, s, L));
+  WHierarchy mg;
+  PDE_OK(mg.build(c, s.g, s.bc, s.coefA.p));
+  const int nl = mg.levels();
+  if (nl < 2) PDE_FAIL("weighted multigrid: the grid does not coarsen");
+  if (nl > PDE_MG_MAX_LEVELS) PDE_FAIL("more multigrid levels than pde_mg_info holds");
+  const Grid& g = s.g;
+  const size_t bytes = sizeof(double) * g.nn[0] * g.nn[1] * g.nzg;
+  double* dense = nullptr;
+  CUDA_OK(cudaMalloc(&dense, bytes));
+  struct DenseRel { double* p; ~DenseRel() { cudaFree(p); } } denserel{dense};
+  PDE_OK(h2d(c, dense, b, bytes));
+  PDE_OK(launch_unpack(c, g, 1, dense, s.r.p, 0));
+  for (int k = 0; k < ncycles; ++k) {
+    double* z = nullptr;
+    PDE_OK(wvcycle(c, mg, s.r.p, &z, S_RHO0));
+    if (k == 0 || k == ncycles - 1) PDE_OK(launch_pack(c, g, 1, z, dense, 0));
+    if (k == 0) PDE_OK(d2h(c, z_first, dense, bytes));
+    if (k == ncycles - 1) PDE_OK(d2h(c, z_last, dense, bytes));
+  }
+  if (bz) PDE_OK(read_scal(c, S_RHO0, 1, bz));
+  std::memset(info, 0, sizeof(*info));
+  info->levels = nl;
+  info->n_dense = mg.lv[nl - 1]->n_dense;
+  int ax[3], nax;
+  internal_axes(p->dim, ax, &nax);
+  for (int l = 0; l < nl; ++l) {
+    for (int q = 0; q < nax; ++q) info->n[l][q] = mg.lv[l]->g.nc[ax[q]];
+    info->lmax[l] = mg.lv[l]->lmax;
+  }
+  return 0;
+}

@@ -377,7 +377,7 @@ static int wsmooth(pde_ctx* c, const WHierarchy& H, WLevel& L, const double* b, 
 }
 
 // z = V(b0); the last level-0 post-sweep leaves sum b0.z in dot_slot
-static int wvcycle(pde_ctx* c, WHierarchy& H, const double* b0, double** z_out, int dot_slot) {
+int wvcycle(pde_ctx* c, WHierarchy& H, const double* b0, double** z_out, int dot_slot) {
   const int nl = H.levels();
   std::vector<double*> cur(nl), oth(nl);
   for (int l = 0; l < nl; ++l) { cur[l] = H.lv[l]->xa.p; oth[l] = H.lv[l]->xb.p; }

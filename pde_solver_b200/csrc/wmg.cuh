@@ -39,5 +39,7 @@ struct WHierarchy {
 // GMG-PCG on A x = b given x (with Dirichlet values) and r = masked(b - A x); p, q: work vectors of level 0's grid
 int wmg_pcg(pde_ctx* c, WHierarchy& h, double* x, double* r, double* p, double* q, double bnorm2,
             const pde_solver_opts& o, pde_stats* st);
+// z = V(b0) (z_out: the level-0 buffer holding it); the last level-0 post-sweep leaves sum b0.z in dot_slot
+int wvcycle(pde_ctx* c, WHierarchy& H, const double* b0, double** z_out, int dot_slot);
 // level `level` expanded to all g.nk offsets (g.kdx order), [nk][nverts] in natural vertex order
 int wmg_level_coefs(pde_ctx* c, const WHierarchy& h, int level, double* out);

@@ -299,6 +299,38 @@ def test_level_coefs_match_galerkin_model(P, name, n):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("name,n", [("2d_spherical", [64, 64]), ("3d_spherical", [16, 16, 16]),
+                                    ("cylinder_core", [32, 32, 32])])
+def test_vcycle_matches_galerkin_model(P, name, n):
+    """pde_wheat_vcycle (the V-cycle of the GMG-PCG) against oracle.gmg_model.vcycle on the Galerkin model, vector by
+    vector: a wrong V-cycle kernel slows the solve down without changing its solution."""
+    if name == "cylinder_core":
+        A, free, _, dim = cylinder_core_system(n)
+        p = _wheat_params(P, 3, n, [0.0, -0.5, -0.5], [1.0, 0.5, 0.5], degree=2, kind=1, core=(0.25, 25.0))
+    else:
+        r_inner = 0.2 if name == "3d_spherical" else 0.1
+        A, free, _, dim = curvi_system(name, n, r_inner)
+        hi = [1.0, np.pi, 2 * np.pi][:dim]
+        p = _wheat_params(P, dim, n, [r_inner, 0.0, 0.0][:dim], hi, rpow=2, wsin=1, degree=2)
+    levels = build_galerkin(A, free, n, dim)
+    b = np.random.default_rng(4).standard_normal(A.shape[0]) * free
+    z1, z3, bz, info = P._lib.wheat_vcycle(P._lib.default_context(), p, b, ncycles=3)
+    assert info["levels"] == len(levels)
+    assert info["n_dense"] == (levels[-1].idx.size if levels[-1].dense is not None else 0)
+    for l, lv in enumerate(levels):
+        assert info["n"][l][:dim] == lv.n
+        assert abs(info["lmax"][l] - lv.lmax) <= 1e-13 * lv.lmax, (l, info["lmax"][l], lv.lmax)
+    ref = gm.vcycle(levels, b)
+    ratio = np.abs(z1 - ref).max() / np.abs(ref).max()
+    print(f"[wvcycle] {name} {n}: max|z-z_model|/max|z_model| = {ratio:.2e}")
+    assert ratio <= 1e-11, ratio
+    assert not z1[~free].any()
+    assert np.array_equal(z3, z1)
+    assert abs(bz - b @ z1) <= 1e-12 * np.abs(b * z1).sum()
+    assert info["paths"] == [0] * len(levels) and info["graph"] == 0
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("name", ["2d_spherical_64", "cylinder_core_32"])
 def test_gmg_iterations_match_model(P, name):
     f_src, Tb = 40.0, 35.0
