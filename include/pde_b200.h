@@ -312,6 +312,25 @@ int pde_op_vcycle(pde_ctx* ctx, const pde_op_params* p, const pde_solver_opts* o
 int pde_wheat_vcycle(pde_ctx* ctx, const pde_wheat_params* p, int32_t ncycles, const double* b, double* z_first,
                      double* z_last, double* bz, pde_mg_info* info);
 
+/* ---- load-vector test entry points ------------------------------------------------------------------------------
+ * The vectors the solvers build on the device before they solve, returned raw, so that tests can compare them with a
+ * reference entry by entry.  Each runs the production launch of its solver on one GPU; natural vertex order. */
+/* b_i = sum over the simplices c that contain vertex i of value_c |c| / (dim + 1), value_c the von Mises stress /
+ * strain (1-D: E u' / u') of the displacement disp [nverts][dim] (the layout of disp_out), with the clamp, Lame
+ * constants and quantity of pde_elasticity_solve.  load_out: [nverts]. */
+int pde_elast_projection_load(pde_ctx* ctx, const pde_elast_params* p, const double* disp, double* load_out);
+/* the P2 load of the cosine / sine initial condition amplitude * prod_q trig(wavenumber x_q) on the box [lo, hi]
+ * (initial_type PDE_IC_COSINE or PDE_IC_SINE): b_i = int I_P2(f) phi_i.  load_out: [nverts]. */
+int pde_trig_ic_load(pde_ctx* ctx, int dim, const int32_t n[3], const double lo[3], const double hi[3],
+                     int initial_type, double amplitude, double wavenumber, double* load_out);
+/* the assembly of pde_wheat_solve: coefA (A = alpha M_w + beta K_w of p, steady: alpha = 0, beta = diffusivity;
+ * transient: alpha = 1, beta = dt diffusivity) and coefM (M_w), each [nk][nverts] with both halves of the stencil,
+ * nk and the offset order as in pde_wheat_level_coefs; no Dirichlet masking.  load: [nverts], m_i = int I(w) phi_i. */
+int pde_wheat_assembly(pde_ctx* ctx, const pde_wheat_params* p, double* coefA, double* coefM, double* load);
+/* y = g (.) m - A x with m_i = int phi_i and component c scaled by g[c], Dirichlet rows 0 (the constant term of the
+ * heat source and the elasticity body force).  x, y: [ncomp][nverts] blocked. */
+int pde_op_load(pde_ctx* ctx, const pde_op_params* p, const double g[3], const double* x, double* y);
+
 #ifdef __cplusplus
 }
 #endif

@@ -299,8 +299,14 @@ def lu_solve(A: sp.csr_matrix, b: np.ndarray) -> np.ndarray:
 # --------------------------------------------------------------------------------------
 
 def project_p2_expression(mesh: Mesh, fn: Callable[[np.ndarray], np.ndarray]) -> np.ndarray:
-    """project(Expression(degree=2), P1): interpolate fn into P2 on every cell (vertices + edge
-    midpoints), integrate exactly against P1, solve the consistent-mass system with LU."""
+    """project(Expression(degree=2), P1): the P2 load of p2_load, then the consistent-mass system with LU."""
+    _, M = assemble_stiffness_mass(mesh)
+    return lu_solve(M, p2_load(mesh, fn))
+
+
+def p2_load(mesh: Mesh, fn: Callable[[np.ndarray], np.ndarray]) -> np.ndarray:
+    """b_i = ∫ I_P2(fn) φ_i: fn interpolated into P2 on every cell (vertices + edge midpoints) and integrated
+    exactly against P1."""
     d = mesh.dim
     vol, _ = _gradients(mesh)
     c = mesh.cells.astype(np.int64)
@@ -322,8 +328,7 @@ def project_p2_expression(mesh: Mesh, fn: Callable[[np.ndarray], np.ndarray]) ->
             fm = fn(0.5 * (X[:, a, :] + X[:, bb, :]))
             contrib += fm * (ein if i in (a, bb) else eout)
         np.add.at(b, c[:, i], contrib * vol)
-    _, M = assemble_stiffness_mass(mesh)
-    return lu_solve(M, b)
+    return b
 
 
 # --------------------------------------------------------------------------------------
@@ -467,12 +472,18 @@ def von_mises_cells(mesh: Mesh, u: np.ndarray, lam: float, mu: float, quantity: 
 
 
 def project_cell_constant(mesh: Mesh, vc: np.ndarray) -> np.ndarray:
-    """project(v, P1) for a cell-wise constant v: M x = Σ_c v_c |c|/(d+1), LU (appendix A.5)."""
+    """project(v, P1) for a cell-wise constant v: M x = cell_constant_load(mesh, v), LU (appendix A.5)."""
+    b = cell_constant_load(mesh, vc)
+    _, M = assemble_stiffness_mass(mesh)
+    return lu_solve(M, b), b
+
+
+def cell_constant_load(mesh: Mesh, vc: np.ndarray) -> np.ndarray:
+    """b_i = Σ_{c ∋ i} v_c |c|/(d+1): the load of project(v, P1) for a cell-wise constant v."""
     vol, _ = _gradients(mesh)
     b = np.zeros(mesh.nv)
     np.add.at(b, mesh.cells.ravel(), np.repeat(vc * vol / (mesh.dim + 1), mesh.dim + 1))
-    _, M = assemble_stiffness_mass(mesh)
-    return lu_solve(M, b), b
+    return b
 
 
 def solve_elasticity(dim: int, L: Sequence[float], n: Sequence[int], E: float, nu: float = 0.3,

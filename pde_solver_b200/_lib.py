@@ -113,7 +113,8 @@ def lib():
                      "pde_heat_close", "pde_elasticity_solve", "pde_op_table", "pde_op_apply", "pde_op_bench", "pde_op_sweep", "pde_op_bench_mode", "pde_comm_info", "pde_device_count",
                      "pde_op_solve", "pde_version", "pde_host_alloc", "pde_host_free", "pde_slab_partition", "pde_op_manufactured", "pde_halo_bench", "pde_wheat_solve", "pde_wheat_level_coefs",
                      "pde_wheat_open", "pde_wheat_set_state", "pde_wheat_step", "pde_wheat_get_state", "pde_wheat_close",
-                     "pde_mesh_coords_box", "pde_op_vcycle", "pde_wheat_vcycle"):
+                     "pde_mesh_coords_box", "pde_op_vcycle", "pde_wheat_vcycle", "pde_elast_projection_load",
+                     "pde_trig_ic_load", "pde_wheat_assembly", "pde_op_load"):
             getattr(L, name).restype = C.c_int
         _lib = L
     return _lib
@@ -324,6 +325,42 @@ def op_vcycle(ctx, p, b, opts=None, ncycles=3):
 def wheat_vcycle(ctx, p, b, ncycles=3):
     """As op_vcycle for the weighted operators of WheatParams and their Galerkin hierarchy."""
     return _vcycle(lambda *a: lib().pde_wheat_vcycle(ctx.handle, C.byref(p), *a), b, ncycles)
+
+
+def op_load(ctx, p, g, x):
+    """y = g (.) m - A x (m_i = int phi_i, component c scaled by g[c], Dirichlet rows 0) through the solvers' stencil
+    launch; x, y [ncomp][nverts] (see pde_op_load in include/pde_b200.h)."""
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    y = np.empty_like(x)
+    check(lib().pde_op_load(ctx.handle, C.byref(p), d3(g, 0.0), ptr(x), ptr(y)))
+    return y
+
+
+def elast_projection_load(ctx, p, disp):
+    """Raw load vector of the projected stress / strain of ElastParams p for a displacement [nverts][dim]."""
+    disp = np.ascontiguousarray(disp, dtype=np.float64)
+    out = np.empty(disp.shape[0])
+    check(lib().pde_elast_projection_load(ctx.handle, C.byref(p), ptr(disp), ptr(out)))
+    return out
+
+
+def trig_ic_load(ctx, dim, n, lo, hi, initial_type, amplitude, wavenumber):
+    """Raw P2 load vector of the cosine / sine initial condition on the box [lo, hi]."""
+    nv, _ = mesh_counts(dim, n)
+    out = np.empty(nv)
+    check(lib().pde_trig_ic_load(ctx.handle, int(dim), i3(n), d3(lo, 0.0), d3(hi, 1.0), IC[initial_type],
+                                 C.c_double(amplitude), C.c_double(wavenumber), ptr(out)))
+    return out
+
+
+def wheat_assembly(ctx, p):
+    """(coefA, coefM [nk][nverts], load [nverts]) as the weighted heat solve assembles them for WheatParams p."""
+    dim = int(p.dim)
+    nv, _ = mesh_counts(dim, [p.n[q] for q in range(dim)])
+    nk = {1: 3, 2: 7, 3: 15}[dim]
+    coefA, coefM, load = np.empty((nk, nv)), np.empty((nk, nv)), np.empty(nv)
+    check(lib().pde_wheat_assembly(ctx.handle, C.byref(p), ptr(coefA), ptr(coefM), ptr(load)))
+    return coefA, coefM, load
 
 
 def comm_info(ctx):

@@ -768,6 +768,60 @@ extern "C" int pde_op_sweep(pde_ctx* c, const pde_op_params* p, int mode, double
   return d2h(c, y, dense.p, sizeof(double) * nloc * nc);
 }
 
+// Test entry: the constant right-hand-side term of the stencil kernels (heat source f m, elasticity body force) on
+// caller data, y = g (.) m - A x through the same launch_stencil call as the solves
+extern "C" int pde_op_load(pde_ctx* c, const pde_op_params* p, const double gconst[3], const double* x, double* y) {
+  if (!c || !p || !gconst || !x || !y) PDE_FAIL("null argument");
+  CUDA_OK(cudaSetDevice(c->device));
+  OpGuard G;
+  int nc;
+  PDE_OK(setup_op(c, p, &G.A, &nc));
+  const Grid& g = G.A.g;
+  PDE_OK(G.x.alloc(c, g, nc));
+  PDE_OK(G.y.alloc(c, g, nc));
+  const long long nloc = (long long)g.nn[0] * g.nn[1] * g.nzl;
+  DevMem dense;
+  PDE_OK(dense.alloc(sizeof(double) * nloc * nc));
+  PDE_OK(h2d(c, dense.p, x, sizeof(double) * nloc * nc));
+  PDE_OK(launch_unpack(c, g, nc, (const double*)dense.p, G.x.p, 0));
+  StencilArgs a;
+  a.x = G.x.p; a.y = G.y.p; a.bscale = 1.0; a.ascale = -1.0; a.variant = p->variant; a.reduce_slot_xy = S_XY;
+  for (int i = 0; i < nc; ++i) a.bconst[i] = gconst[i];
+  if (c->world > 1) PDE_OK(comm_halo_exchange(c, g, nc, G.x.p));
+  PDE_OK(launch_stencil(c, g, G.A.bc, G.A.dev, a));
+  PDE_OK(launch_pack(c, g, nc, G.y.p, (double*)dense.p, 0));
+  return d2h(c, y, dense.p, sizeof(double) * nloc * nc);
+}
+
+// Test entry: the raw P2 load vector of the cosine / sine initial condition on the box [lo, hi] (project_trig_ic's
+// right-hand side, before the mass solve)
+extern "C" int pde_trig_ic_load(pde_ctx* c, int dim, const int32_t n[3], const double lo[3], const double hi[3],
+                                int initial_type, double amplitude, double wavenumber, double* load_out) {
+  if (!c || !n || !lo || !hi || !load_out) PDE_FAIL("null argument");
+  if (c->world > 1) PDE_FAIL("pde_trig_ic_load runs on one GPU");
+  if (dim < 1 || dim > 3) PDE_FAIL("dim must be 1, 2 or 3");
+  if (initial_type != PDE_IC_COSINE && initial_type != PDE_IC_SINE) PDE_FAIL("initial_type must be cosine or sine");
+  CUDA_OK(cudaSetDevice(c->device));
+  double L[3] = {1.0, 1.0, 1.0};
+  for (int k = 0; k < dim; ++k) {
+    L[k] = hi[k] - lo[k];
+    if (!(L[k] > 0)) PDE_FAIL("hi must exceed lo on every axis");
+  }
+  Grid g;
+  PDE_OK(make_grid(dim, n, L, 0, 1, &g));
+  Field rhs;
+  struct Rel { Field* f; ~Rel() { f->release(); } } rel{&rhs};
+  PDE_OK(rhs.alloc(c, g, 1));
+  SimplexGeom sg;
+  build_simplex_geom(dim, g.h, &sg);
+  PDE_OK(launch_p2_load(c, g, sg, amplitude, wavenumber, initial_type == PDE_IC_SINE, n, L, rhs.p, lo));
+  const long long nloc = (long long)g.nn[0] * g.nn[1] * g.nzl;
+  DevMem dense;
+  PDE_OK(dense.alloc(sizeof(double) * nloc));
+  PDE_OK(launch_pack(c, g, 1, rhs.p, (double*)dense.p, 0));
+  return d2h(c, load_out, dense.p, sizeof(double) * nloc);
+}
+
 extern "C" int pde_op_bench_mode(pde_ctx* c, const pde_op_params* p, int mode, int reps, int warmup, double* ms_per_launch,
                                  int64_t* ndofs) {
   if (!c || !p) PDE_FAIL("null argument");
@@ -1001,32 +1055,76 @@ extern "C" int pde_op_manufactured(pde_ctx* c, const pde_op_params* p, const pde
 }
 
 // ---- elasticity -----------------------------------------------------------------------------------------
+// what the elasticity tools solve and project: the operator clamped at x = 0 (1-D: E A u'' on the scalar operator),
+// the Lame constants (2-D plane stress or plane strain) and the launch_cell_rhs mode of the projected quantity
+// (0 / 1: von Mises stress / strain, 2 / 3: axial strain / stress E u')
+struct ElastSetup {
+  pde_op_params op;
+  double lam = 0.0, mu = 0.0;
+  int mode = 0;
+};
+
+static int elast_setup(const pde_elast_params* p, ElastSetup* s) {
+  if (!(p->E > 0)) PDE_FAIL("E must be > 0");
+  const int dim = p->dim;
+  if (dim < 1 || dim > 3) PDE_FAIL("dim must be 1, 2 or 3");
+  pde_op_params& op = s->op;
+  std::memset(&op, 0, sizeof(op));
+  op.dim = dim;
+  for (int k = 0; k < 3; ++k) { op.n[k] = p->n[k]; op.L[k] = p->L[k]; }
+  op.bc.face_on[0] = 1;  // clamp x = 0 (reference :1531-1534, 1681-1684, 1831-1834)
+  s->lam = s->mu = 0.0;
+  if (dim == 1) {
+    op.kind = PDE_OP_HEAT; op.alpha = 0.0; op.beta = p->E * p->area;
+  } else {
+    if (!(p->nu > -1.0 && p->nu < 0.5)) PDE_FAIL("nu must be in (-1, 0.5)");
+    s->mu = p->E / (2.0 * (1.0 + p->nu));
+    s->lam = (dim == 2 && p->plane_stress) ? p->E * p->nu / (1.0 - p->nu * p->nu)
+                                           : p->E * p->nu / ((1.0 + p->nu) * (1.0 - 2.0 * p->nu));
+    op.kind = PDE_OP_ELASTICITY; op.lam = s->lam; op.mu = s->mu;
+  }
+  s->mode = dim == 1 ? (p->quantity == 1 ? 2 : 3) : (p->quantity == 1 ? 1 : 0);
+  return 0;
+}
+
+// Test entry: the raw load vector of the projected stress / strain for a caller's displacement (launch_cell_rhs as
+// pde_elasticity_solve runs it, before the mass solve)
+extern "C" int pde_elast_projection_load(pde_ctx* c, const pde_elast_params* p, const double* disp, double* load_out) {
+  if (!c || !p || !disp || !load_out) PDE_FAIL("null argument");
+  if (c->world > 1) PDE_FAIL("pde_elast_projection_load runs on one GPU");
+  CUDA_OK(cudaSetDevice(c->device));
+  ElastSetup es;
+  PDE_OK(elast_setup(p, &es));
+  const int dim = p->dim, nc = dim == 1 ? 1 : dim;
+  Grid g;
+  PDE_OK(make_grid(dim, p->n, p->L, 0, 1, &g));
+  Field u, rhs;
+  struct Rel { Field* a; Field* b; ~Rel() { a->release(); b->release(); } } rel{&u, &rhs};
+  PDE_OK(u.alloc(c, g, nc));
+  PDE_OK(rhs.alloc(c, g, 1));
+  const long long nloc = (long long)g.nn[0] * g.nn[1] * g.nzl;
+  DevMem dense;
+  PDE_OK(dense.alloc(sizeof(double) * nloc * nc));
+  PDE_OK(h2d(c, dense.p, disp, sizeof(double) * nloc * nc));
+  PDE_OK(launch_unpack(c, g, nc, (const double*)dense.p, u.p, 1));
+  SimplexGeom sg;
+  build_simplex_geom(dim, g.h, &sg);
+  PDE_OK(launch_cell_rhs(c, g, nc, sg, u.p, rhs.p, es.mode, es.lam, es.mu, p->E));
+  PDE_OK(launch_pack(c, g, 1, rhs.p, (double*)dense.p, 0));
+  return d2h(c, load_out, dense.p, sizeof(double) * nloc);
+}
+
 extern "C" int pde_elasticity_solve(pde_ctx* c, const pde_elast_params* p, const pde_solver_opts* o_in,
                                     double* field_out, double* disp_out, pde_stats* st_out, pde_stats* st_proj_out) {
   if (!c || !p || !field_out) PDE_FAIL("null argument");
   CUDA_OK(cudaSetDevice(c->device));
   pde_solver_opts o;
   if (o_in) o = *o_in; else pde_solver_opts_default(&o);
-  if (!(p->E > 0)) PDE_FAIL("E must be > 0");
+  ElastSetup es;
+  PDE_OK(elast_setup(p, &es));
   const int dim = p->dim;
-  pde_bc ubc;
-  std::memset(&ubc, 0, sizeof(ubc));
-  ubc.face_on[0] = 1;  // clamp x = 0 (reference :1531-1534, 1681-1684, 1831-1834)
-  pde_op_params op;
-  std::memset(&op, 0, sizeof(op));
-  op.dim = dim;
-  for (int k = 0; k < 3; ++k) { op.n[k] = p->n[k]; op.L[k] = p->L[k]; }
-  op.bc = ubc;
-  double lam = 0, mu = 0;
-  if (dim == 1) {
-    op.kind = PDE_OP_HEAT; op.alpha = 0.0; op.beta = p->E * p->area;
-  } else {
-    if (!(p->nu > -1.0 && p->nu < 0.5)) PDE_FAIL("nu must be in (-1, 0.5)");
-    mu = p->E / (2.0 * (1.0 + p->nu));
-    lam = (dim == 2 && p->plane_stress) ? p->E * p->nu / (1.0 - p->nu * p->nu)
-                                        : p->E * p->nu / ((1.0 + p->nu) * (1.0 - 2.0 * p->nu));
-    op.kind = PDE_OP_ELASTICITY; op.lam = lam; op.mu = mu;
-  }
+  const pde_op_params& op = es.op;
+  const double lam = es.lam, mu = es.mu;
   OpGuard G;
   int nc;
   PDE_OK(setup_op(c, &op, &G.A, &nc));
@@ -1078,9 +1176,8 @@ extern "C" int pde_elasticity_solve(pde_ctx* c, const pde_elast_params* p, const
   stats_init(&sp, nloc);
   CUDA_OK(cudaEventRecord(c->ev0, c->stream));
   const long long l1 = c->launches;
-  const int mode = dim == 1 ? (p->quantity == 1 ? 2 : 3) : (p->quantity == 1 ? 1 : 0);
   if (c->world > 1) PDE_OK(comm_halo_exchange(c, g, nc, G.x.p));
-  PDE_OK(launch_cell_rhs(c, g, nc, sg, G.x.p, P.r.p, mode, lam, mu, p->E));
+  PDE_OK(launch_cell_rhs(c, g, nc, sg, G.x.p, P.r.p, es.mode, lam, mu, p->E));
   PDE_OK(launch_dot(c, g, 1, P.r.p, P.r.p, S_TMP0));
   if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_TMP0, 1));
   double pn2;

@@ -625,6 +625,25 @@ extern "C" int pde_wheat_level_coefs(pde_ctx* c, const pde_wheat_params* p, int 
   return 0;
 }
 
+// Test entry: what wheat_assemble leaves on the device (full stencils of A and M_w, load m_w), in natural vertex order
+extern "C" int pde_wheat_assembly(pde_ctx* c, const pde_wheat_params* p, double* coefA, double* coefM, double* load) {
+  if (!c || !p || !coefA || !coefM || !load) PDE_FAIL("null argument");
+  WheatState s;
+  double L[3];
+  PDE_OK(wheat_assemble(c, p, s, L));
+  const Grid& g = s.g;
+  const size_t nv = (size_t)g.nn[0] * g.nn[1] * g.nzg;
+  double* dense = nullptr;
+  CUDA_OK(cudaMalloc(&dense, sizeof(double) * nv * g.nk));
+  struct DenseRel { double* p; ~DenseRel() { cudaFree(p); } } denserel{dense};
+  PDE_OK(launch_pack(c, g, g.nk, s.coefA.p, dense, 0));
+  PDE_OK(d2h(c, coefA, dense, sizeof(double) * nv * g.nk));
+  PDE_OK(launch_pack(c, g, g.nk, s.coefM.p, dense, 0));
+  PDE_OK(d2h(c, coefM, dense, sizeof(double) * nv * g.nk));
+  PDE_OK(launch_pack(c, g, 1, s.loadv.p, dense, 0));
+  return d2h(c, load, dense, sizeof(double) * nv);
+}
+
 // Test entry: the V-cycle of pde_wheat_solve's GMG path applied ncycles times to one host vector (see the header)
 extern "C" int pde_wheat_vcycle(pde_ctx* c, const pde_wheat_params* p, int32_t ncycles, const double* b, double* z_first,
                                 double* z_last, double* bz, pde_mg_info* info) {

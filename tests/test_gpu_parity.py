@@ -99,6 +99,20 @@ def test_operator_apply_matches_oracle(P, ctx, kind, dim, n, variant):
         ref[:, dofs] = 0.0                                  # Dirichlet rows are masked
         scale = np.abs(A).max() * np.abs(x).max()
         assert np.abs(y - ref).max() <= 1e-13 * scale * 30
+        # the constant right-hand-side term of the same launch (heat source f m, body force): g (.) m - A x
+        g = np.array([0.7, -1.3, 2.1])
+        yl = P._lib.op_load(ctx, p, g, x)
+        refl = g[:nc, None] * fo.lumped_load(m)[None, :] - (A @ x.ravel()).reshape(nc, m.nv)
+        refl[:, dofs] = 0.0
+        ratio = np.abs(yl - refl).max() / max(scale, np.abs(refl).max())
+        # with x = 0 the load term stands alone (next to A x it is ~1e-12 of the elasticity operator's scale)
+        m0 = np.where(np.isin(np.arange(m.nv), dofs), 0.0, fo.lumped_load(m))
+        y0 = P._lib.op_load(ctx, p, g, np.zeros_like(x))
+        ratio0 = (np.abs(y0 - g[:nc, None] * m0[None, :]).max()
+                  / max(np.abs(g).max() * m0.max(), np.finfo(float).tiny))
+        print(f"[op_load] {kind} {dim}d {n} variant {variant} dirichlet {len(dofs)}: ratio {ratio:.2e}, "
+              f"x = 0 {ratio0:.2e}")
+        assert ratio <= 1e-13 * 30 and ratio0 <= 1e-13 * 30
 
 
 @pytest.mark.parametrize("kind,n", [("elasticity", [66, 20, 12]), ("elasticity", [40, 9, 37]), ("heat", [70, 33, 40])])
@@ -659,16 +673,24 @@ def test_null_spaces_and_volume_at_full_size(P, ctx):
         assert np.abs(r).max() <= 1e-12 * cmax * max(1.0, np.abs(u).max())
 
 
-@pytest.mark.parametrize("precond", ["gmg", "jacobi"])
-def test_steady_heat_with_end_temperatures_is_exactly_linear(P, precond):
+@pytest.mark.parametrize("precond,n,source_value", [
+    ("gmg", [256, 96, 64], 0.0), ("jacobi", [64, 24, 16], 0.0),
+    ("gmg", [256, 96, 64], 40.0), ("jacobi", [64, 24, 16], 40.0),
+    ("gmg", [333, 77, 130], 40.0)],                    # ragged TMA tiles, face rows on the four natural faces
+    ids=["gmg", "jacobi", "gmg-source", "jacobi-source", "gmg-source-ragged"])
+def test_steady_heat_with_end_temperatures_is_exactly_linear(P, precond, n, source_value):
     """Known answer without the oracle: steady conduction between T_left at x = 0 and T_right at x = Lx with
     insulated (natural) side faces is linear in x, and a linear field lies in the P1 space, so the nodal values are
-    exact up to the solver tolerance - on a grid far beyond what the CPU restatement can factorise."""
-    Lx, Ly, Lz, n = 2.0, 0.7, 0.5, ([256, 96, 64] if precond == "gmg" else [64, 24, 16])
-    f = P._solve_heat_3d_raw(Lx, Ly, Lz, n[0], n[1], n[2], 1.7, 0.0, 0.0, 0.01, 1, steady=True, T_left=20.0,
-                             T_right=-5.0, precond=precond, as_arrays=True)
+    exact up to the solver tolerance - on a grid far beyond what the CPU restatement can factorise.  A constant source
+    f adds f x (Lx - x) / (2 kappa): the 1-D P1 solution is exact at the nodes, and the Kuhn split carries that over
+    to the box (test_load_vectors.py checks the formula against the oracle), so the heat source term f m of the
+    stencil kernels is checked here at full size too."""
+    Lx, Ly, Lz, kappa = 2.0, 0.7, 0.5, 1.7
+    f = P._solve_heat_3d_raw(Lx, Ly, Lz, n[0], n[1], n[2], kappa, 0.0, 0.0, 0.01, 1, steady=True, T_left=20.0,
+                             T_right=-5.0, source_type="constant", source_value=source_value, precond=precond,
+                             as_arrays=True)
     x = np.asarray(f.coords)[:, 0]
-    exact = 20.0 + (-5.0 - 20.0) * x / Lx
+    exact = 20.0 + (-5.0 - 20.0) * x / Lx + source_value * x * (Lx - x) / (2.0 * kappa)
     u = np.asarray(f.values)[-1]
     assert np.linalg.norm(u - exact) <= TOL * np.linalg.norm(exact)
     assert P.last_stats()["converged"] == 1
