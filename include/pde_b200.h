@@ -291,8 +291,8 @@ int pde_op_manufactured(pde_ctx* ctx, const pde_op_params* p, const pde_solver_o
  * vector `ncycles` times and return it, so that tests can compare B with a model of it vector by vector. */
 #define PDE_MG_MAX_LEVELS 16
 /* paths bits: fused kernels a level actually ran (k_sweep / generic FIRST2 pass of the first two pre-smoothing
- * sweeps, k_heat_post2, round-1 k_post2, k_heat_post2 residual + restriction) */
-enum { PDE_MG_FIRST2 = 1, PDE_MG_HEAT_POST2 = 2, PDE_MG_POST2_R1 = 4, PDE_MG_RESID_RESTRICT = 8 };
+ * sweeps, k_heat_post2 post-smoothing, k_heat_post2 residual + restriction); bit 4 is unused */
+enum { PDE_MG_FIRST2 = 1, PDE_MG_HEAT_POST2 = 2, PDE_MG_RESID_RESTRICT = 8 };
 typedef struct pde_mg_info {
   int32_t levels, n_dense;
   int32_t graph;                        /* 1: the last cycle replayed a captured CUDA graph */

@@ -249,12 +249,9 @@ struct pde_heat_state {
   bool use_mg = false;
   PcgWork w;
   Field u, r;
-  Field uold, e;          // previous step and increment: x0 = u_n + (u_n - u_{n-1})
   Field un;               // u_n of a verified solve (true-residual check), allocated on first use
-  bool extrap = false;
   DevMem dense;
   long long nloc = 0;
-  long long steps_done = 0;
   double setup_ms = 0;
   // copy pipeline (pde_heat_advance_batch, snapshots of pde_heat_solve): two staging buffers per direction and one
   // stream per direction, so that PCIe traffic in both directions overlaps the solve on the compute stream
@@ -332,7 +329,7 @@ extern "C" int pde_heat_close(pde_heat_state* s) {
   s->A.release(); s->K.release(); s->M.release();
   s->mg.release();
   s->w.release();
-  s->u.release(); s->r.release(); s->uold.release(); s->e.release(); s->un.release();
+  s->u.release(); s->r.release(); s->un.release();
   delete s;
   return 0;
 }
@@ -363,14 +360,6 @@ extern "C" int pde_heat_open(pde_ctx* c, const pde_heat_params* p, const pde_sol
     if ((rc = s->u.alloc(c, s->g, 1))) break;
     if ((rc = s->r.alloc(c, s->g, 1))) break;
     if ((rc = s->w.alloc(c, s->g, 1))) break;
-    {
-      const char* e = getenv("PDE_B200_EXTRAP");
-      s->extrap = !p->steady && (e ? atoi(e) != 0 : false);  // measured: no net gain on config 4, off by default
-      if (s->extrap) {
-        if ((rc = s->uold.alloc(c, s->g, 1))) break;
-        if ((rc = s->e.alloc(c, s->g, 1))) break;
-      }
-    }
     s->nloc = (long long)s->g.nn[0] * s->g.nn[1] * s->g.nzl;
     if ((rc = s->dense.alloc(sizeof(double) * s->nloc))) break;
     long long ndofs = (long long)s->g.nn[0] * s->g.nn[1] * s->g.nzg;
@@ -378,8 +367,6 @@ extern "C" int pde_heat_open(pde_ctx* c, const pde_heat_params* p, const pde_sol
       if ((rc = s->mg.build(c, s->A, PDE_OP_HEAT, alpha, beta))) break;
       s->mg.nu = s->o.cheby_degree > 0 ? s->o.cheby_degree : 2;
       s->mg.ratio = s->o.cheby_ratio > 1 ? s->o.cheby_ratio : 8.0;
-      if (const char* e = getenv("PDE_B200_CHEBY_DEGREE")) s->mg.nu = atoi(e) > 0 ? atoi(e) : s->mg.nu;
-      if (const char* e = getenv("PDE_B200_CHEBY_RATIO")) s->mg.ratio = atof(e) > 1 ? atof(e) : s->mg.ratio;
     }
     s->use_mg = choose_precond(s->o, c, ndofs, s->mg) == PDE_PRECOND_GMG;
     if (!s->use_mg) s->mg.release();
@@ -413,7 +400,6 @@ extern "C" int pde_heat_set_state(pde_heat_state* s, const double* u_host) {
   CUDA_OK(cudaMemcpyAsync(s->dense.p, u_host, sizeof(double) * s->nloc, cudaMemcpyHostToDevice, c->stream));
   PDE_OK(launch_unpack(c, s->g, 1, (const double*)s->dense.p, s->u.p, 0));
   PDE_OK(launch_apply_bc_values(c, s->g, s->bc, s->u.p));
-  s->steps_done = 0;  // a new state has no history: the next step starts from the plain warm start
   return 0;
 }
 
@@ -454,19 +440,6 @@ static int heat_one_solve(pde_heat_state* s, pde_stats* st, bool verify = false)
     PDE_OK(launch_stencil(c, s->g, s->bc, s->M.dev, nb));
     if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_XY, 2));
     PDE_OK(read_scal(c, S_YY, 1, &bn2));
-    if (s->extrap) {
-      // better initial guess (parity-neutral: the stopping rule is relative to ||b||):
-      //   e = u_n - u_{n-1}; x0 = u_n + e; r0 -= A e.   uold keeps u_n for the next step.
-      if (s->steps_done > 0) {
-        PDE_OK(launch_extrapolate(c, s->g, 1, s->u.p, s->uold.p, s->e.p));
-        StencilArgs ea;
-        ea.x = s->e.p; ea.b = s->r.p; ea.y = s->r.p; ea.bscale = 1.0; ea.ascale = -1.0;
-        if (c->world > 1) PDE_OK(comm_halo_exchange(c, s->g, 1, s->e.p));
-        PDE_OK(launch_stencil(c, s->g, s->bc, s->A.dev, ea));
-      } else {
-        PDE_OK(launch_copy(c, s->g, 1, s->uold.p, s->u.p));
-      }
-    }
   }
   PDE_OK(pcg_solve(c, s->A, s->use_mg ? &s->mg : nullptr, s->w, s->u.p, s->r.p, bn2, s->o, st));
   if (verify) {
@@ -509,7 +482,6 @@ extern "C" int pde_heat_step(pde_heat_state* s, int nsteps, pde_stats* st_out) {
   CUDA_OK(cudaEventRecord(c->ev0, c->stream));
   for (int k = 0; k < nsteps; ++k) {
     PDE_OK(heat_one_solve(s, &st, k == nsteps - 1 && s->o.verify_residual >= 0));
-    s->steps_done += 1;
   }
   CUDA_OK(cudaEventRecord(c->ev1, c->stream));
   CUDA_OK(cudaEventSynchronize(c->ev1));
@@ -556,9 +528,7 @@ extern "C" int pde_heat_advance_batch(pde_heat_state* s, int nreq, const double*
     PDE_OK(launch_unpack(c, s->g, 1, q.in[b], s->u.p, 0));
     CUDA_OK(cudaEventRecord(q.in_free[b], c->stream));
     PDE_OK(launch_apply_bc_values(c, s->g, s->bc, s->u.p));
-    s->steps_done = 0;
     PDE_OK(heat_one_solve(s, &st));
-    s->steps_done = 1;
     PDE_OK(pipe_push_snapshot(s, u_out_host[k]));
   }
   PDE_OK(pipe_drain(s));
@@ -854,16 +824,13 @@ extern "C" int pde_op_bench_mode(pde_ctx* c, const pde_op_params* p, int mode, i
   return 0;
 }
 
-// the GMG hierarchy of the operator solves: levels from the operator, smoother degree and ratio from o and the
-// environment
+// the GMG hierarchy of the operator solves: levels from the operator, smoother degree and ratio from o
 static int build_hierarchy(pde_ctx* c, OpGuard& G, const pde_op_params* p, const pde_solver_opts& o) {
   double p0 = p->kind == PDE_OP_ELASTICITY ? p->lam : (p->kind == PDE_OP_MASS ? 1.0 : (p->kind == PDE_OP_STIFFNESS ? 0.0 : p->alpha));
   double p1 = p->kind == PDE_OP_ELASTICITY ? p->mu : (p->kind == PDE_OP_MASS ? 0.0 : (p->kind == PDE_OP_STIFFNESS ? 1.0 : p->beta));
   PDE_OK(G.mg.build(c, G.A, p->kind == PDE_OP_ELASTICITY ? PDE_OP_ELASTICITY : PDE_OP_HEAT, p0, p1));
   G.mg.nu = o.cheby_degree > 0 ? o.cheby_degree : 2;
   G.mg.ratio = o.cheby_ratio > 1 ? o.cheby_ratio : 8.0;
-  if (const char* e = getenv("PDE_B200_CHEBY_DEGREE")) G.mg.nu = atoi(e) > 0 ? atoi(e) : G.mg.nu;
-  if (const char* e = getenv("PDE_B200_CHEBY_RATIO")) G.mg.ratio = atof(e) > 1 ? atof(e) : G.mg.ratio;
   return 0;
 }
 

@@ -213,9 +213,6 @@ struct StencilArgs {
 
 int launch_stencil(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a);
 bool sweep_applicable(const Grid& g, int ncomp);
-// two restart Chebyshev sweeps in one pass (temporal blocking); *handled = false if not applicable
-int launch_post2(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const double* x0, const double* b,
-                 double* y, double c2_0, double c1_1, double c2_1, int dot_slot, bool* handled);
 // rows of the non-Dirichlet nodes on the domain faces (class-table stencil); reductions are ADDED to the slot
 // defer_blocks != nullptr: the kernel only leaves its block sums in c->face_partials (*defer_blocks of them); the
 // sweep kernel launched AFTER it adds them in its own finalize (no fence / atomic ticket per face block)
@@ -231,8 +228,6 @@ int launch_dot(pde_ctx* c, const Grid& g, int ncomp, const double* a, const doub
 int launch_zero(pde_ctx* c, const Grid& g, int ncomp, double* a);
 int launch_copy(pde_ctx* c, const Grid& g, int ncomp, double* dst, const double* src);
 int launch_axpy(pde_ctx* c, const Grid& g, int ncomp, double* y, const double* x, double alpha);
-// e = u - uold ; uold = u ; u = u + e
-int launch_extrapolate(pde_ctx* c, const Grid& g, int ncomp, double* u, double* uold, double* e);
 // first Chebyshev sweep from a zero guess: x = s*dinv*b
 int launch_cheby_first(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const double* b, double* x,
                        double s);

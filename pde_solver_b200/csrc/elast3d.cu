@@ -11,13 +11,12 @@
 //     falls back to the generic kernel if it does not match.
 //   * tile geometry is a compile-time constant (32 x 8 nodes, 128 threads, thread = one column x two rows), so every
 //     shared-memory access is base + immediate.
-//   * the epilogue has no global address arithmetic and no predicates: the right-hand side / previous iterate of the
-//     retiring plane arrive by TMA in the same pipeline stage as the input plane, the output plane is staged in shared
-//     memory and written by a TMA store, which clips at the domain boundary by itself.
+//   * the right-hand side / previous iterate of the retiring plane arrive by TMA in the same pipeline stage as the input
+//     plane; every thread stores its own outputs (a TMA-store epilogue through shared memory measured the same on B200).
 //   * the input components are processed one after the other into the nine accumulators of a row, which keeps the
 //     kernel at <= 128 registers: four CTAs (16 warps) per SM instead of two.
 // Rows with an incomplete element patch (natural faces) are left to k_face_rows, exactly as in k_sweep3d: this kernel
-// stores a value the face kernel never reads there (or, when the output aliases the previous iterate, that iterate).
+// does not store them.
 #include <cuda.h>
 
 #include <cmath>
@@ -45,8 +44,8 @@ constexpr int E_BX = E_TX + 4;                     // input box: origin (x0-2, y
 constexpr int E_STAGES = E_STAGES_;
 static_assert(E_TX % 32 == 0, "strips must not share a warp");
 constexpr int E_NT = E_TX * E_NS;
-template <int YS>
 struct EG {
+  static constexpr int YS = 2;                     // rows per strip
   static constexpr int TY = E_NS * YS;             // rows per tile
   static constexpr int BY = TY + 2;
   static constexpr int XCOMP = E_BX * BY;          // doubles per component of an input box
@@ -155,18 +154,16 @@ __device__ __forceinline__ void e_contrib(const ECoef& C, const double (&V)[YS +
 //                 coefficients arrive with their columns scaled by s0 / diag (so the stencil yields A x1, x1 = s0 D^-1 b),
 //                 y = (1 + c1) x1 + c2 D^-1 (b - A x1).  Valid where every neighbour carries the interior diagonal:
 //                 rows on AND next to natural faces are left to k_face_rows (two layers), which knows the class diagonals
-// TOUT: the output plane is staged in shared memory and written by a TMA store (which clips at the domain boundary);
-//       otherwise every thread stores its own values (no shared-memory traffic, but address arithmetic and predicates).
 #ifndef E_THREADS_PER_SM
 #define E_THREADS_PER_SM 512
 #endif
-template <int MODE, bool PREV, int YS, bool TOUT>
-__global__ void __launch_bounds__(E_NT, (YS <= 2 ? E_THREADS_PER_SM : 384) / E_NT)
+template <int MODE, bool PREV>
+__global__ void __launch_bounds__(E_NT, E_THREADS_PER_SM / E_NT)
 k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmb,
-          const __grid_constant__ CUtensorMap tmp, const __grid_constant__ CUtensorMap tmy,
-          const __grid_constant__ ECoef C, const __grid_constant__ EArgs a, const __grid_constant__ EGeom ge,
-          ReduceBuf red, double* red_out, const double* face_part, int nface_part) {
-  using G = EG<YS>;
+          const __grid_constant__ CUtensorMap tmp, const __grid_constant__ ECoef C, const __grid_constant__ EArgs a,
+          const __grid_constant__ EGeom ge, ReduceBuf red, double* red_out, const double* face_part, int nface_part) {
+  using G = EG;
+  constexpr int YS = G::YS;
   constexpr bool HAS_B = MODE == EM_RESID || MODE == EM_CHEBY;
   constexpr bool CHEBY = MODE == EM_CHEBY;
   constexpr bool FIRST2 = MODE == EM_FIRST2;
@@ -174,8 +171,7 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
   constexpr int STAGE_ELEMS = G::XSTAGE + NAUX * G::TILE;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* const stage0 = reinterpret_cast<double*>(smem_raw);
-  double* const ybuf0 = stage0 + E_STAGES * STAGE_ELEMS;
-  uint64_t* const bars = reinterpret_cast<uint64_t*>(ybuf0 + (TOUT ? 2 * G::TILE : 0));
+  uint64_t* const bars = reinterpret_cast<uint64_t*>(stage0 + E_STAGES * STAGE_ELEMS);
 
   const int t = threadIdx.x;
   const int item = blockIdx.x;
@@ -188,7 +184,6 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
   const int nplanes = zb - za + 2;   // input planes za-1 .. zb
   const uint32_t bar0 = smem_u32(bars);
   const uint32_t stg0 = smem_u32(stage0);
-  const uint32_t yb0 = smem_u32(ybuf0);
   constexpr uint32_t STAGE_BYTES = STAGE_ELEMS * 8;
 
   // step n: input plane za-1+n, and (n >= 2) the right-hand side / previous iterate of output plane za+n-2
@@ -244,7 +239,7 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
     }
   }
   const unsigned fast = fre & ~slow;            // rows this kernel computes on a generic plane
-  double* yrun = a.y + ((long long)ge.PX * iy0 + ix) + ge.plane * za;   // direct stores: column pointer at plane za
+  double* yrun = a.y + ((long long)ge.PX * iy0 + ix) + ge.plane * za;   // output column at plane za
 
   double accA[YS][3], accB[YS][3], accC[YS][3];
 #pragma unroll
@@ -300,12 +295,10 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
       const double* const xo_s = stage0 + ((i - 1) % E_STAGES) * STAGE_ELEMS + xoff + E_BX + 1;
       const double* const bt = sx + G::XSTAGE + toff;
       const double* const pt = bt + G::TILE;
-      double* const yt = ybuf0 + (i & 1) * G::TILE + toff;
-      const unsigned stmask = a.has_y ? (okb & ~keep) : 0u;          // direct stores: rows written by this kernel
+      const unsigned stmask = a.has_y ? (okb & ~keep) : 0u;          // rows written by this kernel
 #pragma unroll
       for (int j = 0; j < YS; ++j) {
         const bool m = (comp >> j) & 1u;
-        const bool k = (keep >> j) & 1u;
 #pragma unroll
         for (int q = 0; q < 3; ++q) {
           const double xo = xo_s[q * G::XCOMP + j * E_BX];
@@ -318,8 +311,6 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
             else dprev = a.prev_mode == 2 ? xo : 0.0;
             const double dn = m ? fma(a.c1, dprev, a.c2d[q] * (Bv - A)) : 0.0;
             yv = xo + dn;
-            // TMA output, PREV: the output may alias x_prev, which k_face_rows still reads on its rows: hand it back
-            if (TOUT && PREV) yv = k ? xo - dprev : yv;
             red_xy = fma(m ? Bv : 0.0, yv, red_xy);
           } else if (FIRST2) {
             // xo is the right-hand side here; A = A x1 (scaled coefficients)
@@ -330,25 +321,13 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
             red_xy = fma(xo, yv, red_xy);
             if (a.need_yy) red_yy = fma(yv, yv, red_yy);
           }
-          if (TOUT) yt[q * G::TCOMP + j * E_TX] = yv;
-          else if ((stmask >> j) & 1u) yrun[q * ge.comp_stride + j * (long long)ge.PX] = yv;
+          if ((stmask >> j) & 1u) yrun[q * ge.comp_stride + j * (long long)ge.PX] = yv;
         }
       }
-      if (TOUT) {
-        if (t == 0) tma_store_wait_read0();   // the store of the step before has released the other output buffer
-        fence_proxy_async();
-      } else {
-        yrun += ge.plane;
-      }
+      yrun += ge.plane;
     }
-    __syncthreads();   // stage (i-1) and the tiles of stage i are consumed; the output tile is complete
-    if (t == 0) {
-      if (TOUT && FIN && a.has_y) {
-        tma_store_4d(&tmy, yb0 + (i & 1) * (G::TILE * 8), x0, y0, zout + PDE_NG, 0);
-        tma_store_commit();
-      }
-      if (i + E_STAGES - 1 < nplanes) issue(i + E_STAGES - 1);
-    }
+    __syncthreads();   // stage (i-1) and the tiles of stage i are consumed
+    if (t == 0 && i + E_STAGES - 1 < nplanes) issue(i + E_STAGES - 1);
   };
 
   using T_ = std::true_type;
@@ -360,7 +339,6 @@ k_elast3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUten
     if (i + 1 < nplanes) body(T_{}, i + 1, accA, accB, accC);
     if (i + 2 < nplanes) body(T_{}, i + 2, accB, accC, accA);
   }
-  if (TOUT && t == 0) tma_store_wait_all();
 
   if (a.do_reduce) {
     if (CHEBY) {
@@ -406,17 +384,9 @@ bool extract_coef(const OpDev& op, ECoef* C) {
   return true;
 }
 
-struct ETune {
-  int ys, tout, zc;
-};
-const ETune& etune() {
-  static ETune t = {env_int("PDE_B200_E_YS", 2), env_int("PDE_B200_E_TOUT", 0), env_int("PDE_B200_E_ZC", 64)};
-  return t;
-}
-
-template <int MODE, bool PREV, int YS, bool TOUT>
+template <int MODE, bool PREV>
 int launch_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a, const ECoef& C) {
-  using G = EG<YS>;
+  using G = EG;
   constexpr int NAUX = ((MODE == EM_RESID || MODE == EM_CHEBY) ? 1 : 0) + (PREV ? 1 : 0);
   EGeom ge;
   ge.nn0 = g.nn[0]; ge.nn1 = g.nn[1]; ge.nzl = g.nzl; ge.z0 = g.z0; ge.nzg = g.nzg;
@@ -425,28 +395,26 @@ int launch_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const 
   ge.PX = g.PX; ge.plane = g.plane; ge.comp_stride = g.comp_stride;
   ge.ntx = (g.nn[0] + E_TX - 1) / E_TX;
   ge.nty = (g.nn[1] + G::TY - 1) / G::TY;
-  int zc = etune().zc < 2 ? 2 : etune().zc;
+  int zc = 64;
   while (zc > 4 && (long long)ge.ntx * ge.nty * ((g.nzl + zc - 1) / zc) < 8LL * c->sm_count) zc /= 2;
   ge.nzc = (g.nzl + zc - 1) / zc;
   ge.zc = (g.nzl + ge.nzc - 1) / ge.nzc;
   ge.nzc = (g.nzl + ge.zc - 1) / ge.zc;
   const long long items = (long long)ge.ntx * ge.nty * ge.nzc;
   if (items > RED_MAX_BLOCKS) PDE_FAIL("elasticity sweep grid exceeds the reduction buffer");
-  const size_t smem = ((size_t)E_STAGES * (G::XSTAGE + NAUX * G::TILE) + (TOUT ? 2 * G::TILE : 0)) * sizeof(double) +
-                      E_STAGES * sizeof(uint64_t);
-  auto kern = k_elast3d<MODE, PREV, YS, TOUT>;
+  const size_t smem = (size_t)E_STAGES * (G::XSTAGE + NAUX * G::TILE) * sizeof(double) + E_STAGES * sizeof(uint64_t);
+  auto kern = k_elast3d<MODE, PREV>;
   static bool attr_set = false;
   if (!attr_set) {
     CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     attr_set = true;
   }
-  CUtensorMap tmx, tmb, tmp, tmy;
+  CUtensorMap tmx, tmb, tmp;
   PDE_OK(field_tensor_map(a.x, g, 3, E_BX, G::BY, &tmx));
-  tmb = tmp = tmy = tmx;   // unused maps still have to be valid kernel parameters
+  tmb = tmp = tmx;   // unused maps still have to be valid kernel parameters
   if (MODE == EM_RESID || MODE == EM_CHEBY) PDE_OK(field_tensor_map(a.b, g, 3, E_TX, G::TY, &tmb));
   if (PREV) PDE_OK(field_tensor_map(a.xprev, g, 3, E_TX, G::TY, &tmp));
-  if (TOUT && a.y) PDE_OK(field_tensor_map(a.y, g, 3, E_TX, G::TY, &tmy));
   EArgs ea;
   ea.y = a.y;
   ECoef Cs = C;
@@ -467,25 +435,14 @@ int launch_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const 
   ea.has_y = a.y != nullptr;
   ea.need_yy = ea.do_reduce && !a.skip_yy;
   double* out = ea.do_reduce ? c->scal + a.reduce_slot_xy : nullptr;
-  // Natural faces.  Direct stores never touch the rows of k_face_rows, so that kernel can run FIRST and leave its
-  // block sums for this kernel's finalize (no fence + atomic ticket in each of its ~5000 latency-bound blocks).  With
-  // the TMA output path this kernel writes whole tiles, so the face rows have to be written after it.
+  // Natural faces.  This kernel never stores the rows of k_face_rows, so that kernel can run FIRST and leave its
+  // block sums for this kernel's finalize (no fence + atomic ticket in each of its ~5000 latency-bound blocks).
   int nfp = 0;
-  if (!TOUT && !op.uniform_diag) PDE_OK(launch_face_rows(c, g, bc, op, a, &nfp));
-  kern<<<(unsigned)items, E_NT, smem, c->stream>>>(tmx, tmb, tmp, tmy, Cs, ea, ge, c->red, out, c->face_partials, nfp);
+  if (!op.uniform_diag) PDE_OK(launch_face_rows(c, g, bc, op, a, &nfp));
+  kern<<<(unsigned)items, E_NT, smem, c->stream>>>(tmx, tmb, tmp, Cs, ea, ge, c->red, out, c->face_partials, nfp);
   c->launches++;
   CUDA_OK(cudaGetLastError());
-  if (TOUT && !op.uniform_diag) PDE_OK(launch_face_rows(c, g, bc, op, a));
   return 0;
-}
-
-template <int YS, bool TOUT>
-int launch_mode(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a, const ECoef& C) {
-  if (a.cheby == 2) return launch_t<EM_FIRST2, false, YS, TOUT>(c, g, bc, op, a, C);
-  if (a.cheby)
-    return a.prev_mode == 1 ? launch_t<EM_CHEBY, true, YS, TOUT>(c, g, bc, op, a, C)
-                            : launch_t<EM_CHEBY, false, YS, TOUT>(c, g, bc, op, a, C);
-  return a.b ? launch_t<EM_RESID, false, YS, TOUT>(c, g, bc, op, a, C) : launch_t<EM_APPLY, false, YS, TOUT>(c, g, bc, op, a, C);
 }
 
 }  // namespace
@@ -494,33 +451,23 @@ int launch_mode(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, con
 // the kernel implements; otherwise *handled stays false and the generic vector sweep runs.
 int launch_elast3d(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a, bool* handled) {
   *handled = false;
-  static const int off = env_int("PDE_B200_NO_ELAST3D", 0);
-  if (off || op.ncomp != 3 || g.dim != 3 || g.nk != PDE_NOFF) return 0;
+  if (op.ncomp != 3 || g.dim != 3 || g.nk != PDE_NOFF) return 0;
   if (a.ghost_out || (a.cheby == 1 && (a.prev_mode == 3 || !a.b))) return 0;
-  if (a.cheby == 2 && (bc.side_excl || a.reduce_slot_xy >= 0 || !env_int("PDE_B200_E_FIRST2", 1))) return 0;
+  if (a.cheby == 2 && (bc.side_excl || a.reduce_slot_xy >= 0)) return 0;
   if (a.cheby && a.prev_mode == 1 && !a.xprev) return 0;
   ECoef C;
   if (!extract_coef(op, &C)) return 0;
   *handled = true;
-  const int ys = etune().ys;
-  const bool tout = etune().tout != 0;
-#define E_DISPATCH(YS_)                                                \
-  do {                                                                 \
-    if (tout) return launch_mode<YS_, true>(c, g, bc, op, a, C);       \
-    return launch_mode<YS_, false>(c, g, bc, op, a, C);                \
-  } while (0)
-  if (ys == 3) E_DISPATCH(3);
-  if (ys == 4) E_DISPATCH(4);
-  E_DISPATCH(2);
-#undef E_DISPATCH
+  if (a.cheby == 2) return launch_t<EM_FIRST2, false>(c, g, bc, op, a, C);
+  if (a.cheby)
+    return a.prev_mode == 1 ? launch_t<EM_CHEBY, true>(c, g, bc, op, a, C) : launch_t<EM_CHEBY, false>(c, g, bc, op, a, C);
+  return a.b ? launch_t<EM_RESID, false>(c, g, bc, op, a, C) : launch_t<EM_APPLY, false>(c, g, bc, op, a, C);
 }
 
 // can the smoother use the fused first-two-sweeps mode on this level?  (the caller must know before it decides between
 // one fused launch and cheby_first + sweep)
 bool elast3d_first2_ok(const Grid& g, const BcDev& bc, const OpDev& op) {
-  static const int off = env_int("PDE_B200_NO_ELAST3D", 0);
-  static const int on = env_int("PDE_B200_E_FIRST2", 1);
-  if (off || !on || op.ncomp != 3 || g.dim != 3 || g.nk != PDE_NOFF || bc.side_excl) return false;
+  if (op.ncomp != 3 || g.dim != 3 || g.nk != PDE_NOFF || bc.side_excl) return false;
   if (!sweep_applicable(g, 3)) return false;
   ECoef C;
   return extract_coef(op, &C);

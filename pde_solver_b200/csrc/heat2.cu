@@ -1,6 +1,5 @@
 // k_heat_post2: the TWO post-smoothing Chebyshev-Jacobi sweeps of the scalar (heat / mass) multigrid levels in ONE pass
-// over the data (temporal blocking), for uniform-diagonal operators (every face Dirichlet).  Replaces k_post2 (round 1:
-// 0.39 of the measured HBM peak at 168 registers, 151 static instructions per node of which 47 FP64).
+// over the data (temporal blocking), for uniform-diagonal operators (every face Dirichlet).
 //
 //     d0 = m a0 (b - A x0)                         x1 = x0 + d0           (a_k = c2_k / diag, m = 0 on Dirichlet rows)
 //     x2 = x1 + m (c1 d0 + a1 (b - A x1))
@@ -10,9 +9,9 @@
 // shared-memory ring between the two stages; x1 is never formed and b is read once per stage-A node.
 //
 // Layout (compile time, so that every shared-memory access is base + immediate):
-//   tile TX x TY = (CW-2) x 2*YSB nodes, grown tile CW x (TY+2); a warp covers one row of the grown tile (CW = 32 or 64),
-//   thread = column c of the grown tile x strip s in {0, 1}: stage A owns rows s*YSA + j (YSA = YSB + 1) of the grown tile,
-//   stage B rows s*YSB + j of the tile.  Input planes arrive by TMA: x0 as a (TX+4) x (TY+4) box at (x0-2, y0-2), b of the
+//   tile TX x TY = (CW-2) x 2*YSB nodes (YSB = 4), grown tile CW x (TY+2); a warp covers one row of the grown tile
+//   (CW = 64 from 128 nodes in x, else 32), thread = column c of the grown tile x strip s in {0, 1}: stage A owns rows
+//   s*YSA + j (YSA = YSB + 1) of the grown tile, stage B rows s*YSB + j of the tile.  Input planes arrive by TMA: x0 as a (TX+4) x (TY+4) box at (x0-2, y0-2), b of the
 //   plane stage A retires as a (TX+4) x (TY+2) box at (x0-2, y0-1) in the same pipeline stage (the TMA start coordinate
 //   must be 16-byte aligned, hence x0-2).  Stage B runs one plane behind stage A on a three-slot ring of d0 planes and
 //   retires x2 one plane later; input planes za-2 .. zb+1 give outputs za .. zb-1 (fields carry PDE_NG = 2 ghost planes).
@@ -34,8 +33,9 @@ namespace {
 template <bool RR>
 struct HS { static constexpr int N = RR ? H_RR_STAGES : 4; };
 
-template <int CW, int YSB>
+template <int CW>
 struct HG {
+  static constexpr int YSB = 4;
   static constexpr int TX = CW - 2, YSA = YSB + 1, TY = 2 * YSB, RA = TY + 2;
   static constexpr int BX = TX + 4, BYX = TY + 4, BYB = TY + 2;
   static constexpr int XBOX = BX * BYX, BBOX = BX * BYB;              // doubles per TMA box
@@ -95,13 +95,13 @@ __device__ __forceinline__ void h2_contrib(const H2Coef& C, const double (&V)[YS
 //   nothing of it goes to HBM; on every even global plane stage B forms the coarse right-hand side at the even nodes of the
 //   tile, r(2X,2Y,2Z) + 1/2 (its 14 Kuhn neighbours), from the three ring planes around it: 17 B per fine dof (x, b in, 1/8
 //   out) instead of 24 (residual) + 9 (restriction).  Four ring slots: stage B reads the plane stage A wrote two steps ago.
-template <int CW, int YSB, bool RR>
-__global__ void __launch_bounds__(2 * CW, CW == 64 ? ((RR && H_RR_STAGES == 3) ? 4 : (YSB >= 4 ? 3 : (YSB == 3 ? 4 : 5))) : 6)
+template <int CW, bool RR>
+__global__ void __launch_bounds__(2 * CW, CW == 64 ? ((RR && H_RR_STAGES == 3) ? 4 : 3) : 6)
 k_heat_post2(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmb,
              const __grid_constant__ H2Coef C, const __grid_constant__ H2Args a, const __grid_constant__ H2Geom ge,
              ReduceBuf red, double* red_out) {
-  using G = HG<CW, YSB>;
-  constexpr int YSA = G::YSA;
+  using G = HG<CW>;
+  constexpr int YSA = G::YSA, YSB = G::YSB;
   constexpr int H_STAGES = HS<RR>::N;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* const stage0 = reinterpret_cast<double*>(smem_raw);
@@ -269,22 +269,24 @@ k_heat_post2(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CU
   }
 }
 
-template <int CW, int YSB, bool RR>
+template <int CW, bool RR>
 int launch_t(pde_ctx* c, const Grid& g, const OpDev& op, const double* x0, const double* b, const H2Args& ha_in) {
-  using G = HG<CW, YSB>;
+  using G = HG<CW>;
   H2Geom ge;
   ge.nn0 = g.nn[0]; ge.nn1 = g.nn[1]; ge.nzl = g.nzl; ge.z0 = g.z0; ge.nzg = g.nzg; ge.PX = g.PX; ge.plane = g.plane;
   ge.ntx = (g.nn[0] + G::TX - 1) / G::TX;
   ge.nty = (g.nn[1] + G::TY - 1) / G::TY;
-  static const int zc_env = env_int("PDE_B200_P2_ZC", 64);
-  int zc = zc_env < 4 ? 4 : zc_env;
+  int zc = 64;
   while (zc > 8 && (long long)ge.ntx * ge.nty * ((g.nzl + zc - 1) / zc) < 6LL * c->sm_count) zc /= 2;
+  // grids thin in x have many tiles per plane (33 x 4097 x 4097 nodes: 1026): longer z chunks keep the grid within the
+  // reduction buffer
+  while (zc < g.nzl && (long long)ge.ntx * ge.nty * ((g.nzl + zc - 1) / zc) > RED_MAX_BLOCKS) zc *= 2;
   ge.nzc = (g.nzl + zc - 1) / zc;
   ge.zc = (g.nzl + ge.nzc - 1) / ge.nzc;
   ge.nzc = (g.nzl + ge.zc - 1) / ge.zc;
   const long long items = (long long)ge.ntx * ge.nty * ge.nzc;
-  if (items > RED_MAX_BLOCKS) return 2;   // not applicable: the caller falls back
-  auto kern = k_heat_post2<CW, YSB, RR>;
+  if (items > RED_MAX_BLOCKS) return 2;   // the tiles of one plane alone exceed it: the caller falls back
+  auto kern = k_heat_post2<CW, RR>;
   static bool attr_set = false;
   if (!attr_set) {
     CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G::smem(HS<RR>::N)));
@@ -304,30 +306,18 @@ int launch_t(pde_ctx* c, const Grid& g, const OpDev& op, const double* x0, const
   return 0;
 }
 
-bool heat2_applicable(const Grid& g, const OpDev& op) {
-  static const int off = env_int("PDE_B200_NO_HEAT2", 0);
-  if (off) return false;
-  if (g.dim != 3 || g.nk != PDE_NOFF || op.ncomp != 1 || !op.uniform_diag) return false;
-  return g.nn[0] >= 32 && g.nn[1] >= 8 && g.nzl >= 8;
-}
-
 template <bool RR>
 int dispatch(pde_ctx* c, const Grid& g, const OpDev& op, const double* x0, const double* b, const H2Args& ha) {
-  static const int cw_env = env_int("PDE_B200_P2_CW", 0);
-  static const int ysb = env_int("PDE_B200_P2_YSB", 4);
-  const int cw = cw_env ? cw_env : (g.nn[0] >= 128 ? 64 : 32);
-  if (cw == 64 && ysb == 3) return launch_t<64, 3, RR>(c, g, op, x0, b, ha);
-  if (cw == 64) return launch_t<64, 4, RR>(c, g, op, x0, b, ha);
-  return launch_t<32, 4, RR>(c, g, op, x0, b, ha);
+  if (g.nn[0] >= 128) return launch_t<64, RR>(c, g, op, x0, b, ha);
+  return launch_t<32, RR>(c, g, op, x0, b, ha);
 }
 
 }  // namespace
 
-// does one of the fused post-smoothing kernels (k_heat_post2, or k_post2 of round 1) take this level?
-bool post2_applicable(const Grid& g, const OpDev& op) {
+// does k_heat_post2 (both post-smoothing sweeps, or residual + restriction) take this level?
+bool heat2_applicable(const Grid& g, const OpDev& op) {
   if (g.dim != 3 || g.nk != PDE_NOFF || op.ncomp != 1 || !op.uniform_diag) return false;
-  if (g.nn[0] < 32 || g.nn[1] < 8 || g.nzl < 8) return false;
-  return !env_int("PDE_B200_NO_HEAT2", 0) || !env_int("PDE_B200_NO_POST2", 0);
+  return g.nn[0] >= 32 && g.nn[1] >= 8 && g.nzl >= 8;
 }
 
 // Two restart Chebyshev sweeps in one pass; *handled = false if the kernel does not apply (the caller falls back).
@@ -352,8 +342,7 @@ int launch_heat_post2(pde_ctx* c, const Grid& g, const OpDev& op, const double* 
 int launch_heat_resid_restrict(pde_ctx* c, const Grid& gf, const Grid& gc, const OpDev& op, const double* x, const double* b,
                                double* bcoarse, bool* handled) {
   *handled = false;
-  static const int off = env_int("PDE_B200_NO_RR", 0);
-  if (off || !heat2_applicable(gf, op)) return 0;
+  if (!heat2_applicable(gf, op)) return 0;
   // nested grids, slab windows that nest too (rank r owns coarse planes z0/2 ...)
   if (gf.nc[0] != 2 * gc.nc[0] || gf.nc[1] != 2 * gc.nc[1] || gf.nc[2] != 2 * gc.nc[2] || gf.z0 != 2 * gc.z0) return 0;
   H2Args ha{};

@@ -411,8 +411,10 @@ k_face_rows(const __grid_constant__ Grid g, const __grid_constant__ BcDev bc, co
           const double yv = fma(1.0 + a.c1, xv[0][i], a.c2 * s_dinv[cls * NC + i] * (xo[i] - acc[i]));
           (a.y + i * g.comp_stride)[idxl] = yv;
         } else if (CHEBY) {
-          const double dprev = a.prev_mode == 1 ? xo[i] - pv[i] : (a.prev_mode == 2 ? xo[i] : 0.0);
-          const double dn = a.c1 * dprev + a.c2 * __ldg(dinv + cls * NC + i) * (B - acc[i]);
+          const double di = __ldg(dinv + cls * NC + i);
+          const double dprev = a.prev_mode == 1 ? xo[i] - pv[i]
+                             : (a.prev_mode == 2 ? xo[i] : (a.prev_mode == 3 ? xo[i] - a.s0 * di * B : 0.0));
+          const double dn = a.c1 * dprev + a.c2 * di * (B - acc[i]);
           const double yv = xo[i] + dn;
           (a.y + i * g.comp_stride)[idxl] = yv;
           acc_xy = fma(B, yv, acc_xy);
@@ -579,8 +581,10 @@ k_face_tile(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUt
         const double x1 = a.s0 * s_dinv[cls * NC + i] * xo;
         (a.y + i * g.comp_stride)[idxl] = fma(1.0 + a.c1, x1, a.c2 * s_dinv[cls * NC + i] * (xo - acc[i]));
       } else if (CHEBY) {
-        const double dprev = a.prev_mode == 1 ? xo - pv[i] : (a.prev_mode == 2 ? xo : 0.0);
-        const double dn = a.c1 * dprev + a.c2 * __ldg(dinv + cls * NC + i) * (B - acc[i]);
+        const double di = __ldg(dinv + cls * NC + i);
+        const double dprev = a.prev_mode == 1 ? xo - pv[i]
+                           : (a.prev_mode == 2 ? xo : (a.prev_mode == 3 ? xo - a.s0 * di * B : 0.0));
+        const double dn = a.c1 * dprev + a.c2 * di * (B - acc[i]);
         const double yv = xo + dn;
         (a.y + i * g.comp_stride)[idxl] = yv;
         acc_xy = fma(B, yv, acc_xy);
@@ -678,8 +682,7 @@ int launch_face_rows(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op
   for (int k = 0; full && k < PDE_NOFF; ++k) full = g.kidx[k] == k;
   if (layers == 2 && !full) PDE_FAIL("fused first sweeps on natural faces: grid too large for the 3-D face kernel");
   double* out = sd.do_reduce ? c->scal + a.reduce_slot_xy : nullptr;
-  static const int face_tma = getenv("PDE_B200_FACE_TMA") ? atoi(getenv("PDE_B200_FACE_TMA")) : 1;
-  if (face_tma && full && op.ncomp == 3) {
+  if (full && op.ncomp == 3) {
     CUtensorMap t0, t1, t2;
     PDE_OK(field_tensor_map(a.x, g, 3, 4, FACE_TU + 2, &t0, FACE_TV + 2));
     PDE_OK(field_tensor_map(a.x, g, 3, FACE_TU + 4, 3, &t1, FACE_TV + 2));
@@ -880,31 +883,6 @@ k_axpy(double* __restrict__ y, const double* __restrict__ x, double alpha, long 
       }
     }
   }
-}
-
-__global__ void __launch_bounds__(256)
-k_extrapolate(double* __restrict__ u, double* __restrict__ uold, double* __restrict__ e, long long n, int ncomp,
-              long long cs) {
-  const long long n2 = n >> 1;
-  for (int cidx = 0; cidx < ncomp; ++cidx) {
-    double2* u2 = reinterpret_cast<double2*>(u + cidx * cs);
-    double2* o2 = reinterpret_cast<double2*>(uold + cidx * cs);
-    double2* e2 = reinterpret_cast<double2*>(e + cidx * cs);
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (long long)gridDim.x * blockDim.x) {
-      const double2 a = u2[i], b = o2[i];
-      const double2 d = make_double2(a.x - b.x, a.y - b.y);
-      e2[i] = d;
-      o2[i] = a;
-      u2[i] = make_double2(a.x + d.x, a.y + d.y);
-    }
-  }
-}
-int launch_extrapolate(pde_ctx* c, const Grid& g, int ncomp, double* u, double* uold, double* e) {
-  int blocks = flat_blocks(c, g.total / 2, 256 * 4);
-  k_extrapolate<<<blocks, 256, 0, c->stream>>>(u, uold, e, g.total, ncomp, g.comp_stride);
-  c->launches++;
-  CUDA_OK(cudaGetLastError());
-  return 0;
 }
 
 int launch_dot(pde_ctx* c, const Grid& g, int ncomp, const double* a, const double* b, int slot) {

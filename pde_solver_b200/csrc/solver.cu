@@ -4,7 +4,6 @@
 // (fenics_mcp_server.py:265,311,397,440,661,709,1538,1688,1838: assemble AIJ + sparse LU every call)
 // with a matrix-free preconditioned CG whose operator is never stored.
 #include <cmath>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 
@@ -15,7 +14,7 @@ int launch_stencil_fast(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev&
 int launch_heat_post2(pde_ctx* c, const Grid& g, const OpDev& op, const double* x0, const double* b, double* y, double c2_0,
                       double c1_1, double c2_1, int dot_slot, bool* handled);
 bool elast3d_first2_ok(const Grid& g, const BcDev& bc, const OpDev& op);
-bool post2_applicable(const Grid& g, const OpDev& op);
+bool heat2_applicable(const Grid& g, const OpDev& op);
 int launch_heat_resid_restrict(pde_ctx* c, const Grid& gf, const Grid& gc, const OpDev& op, const double* x, const double* b,
                                double* bcoarse, bool* handled);
 
@@ -338,13 +337,11 @@ int Hierarchy::build(pde_ctx* c, const Operator& fine, int kind, double p0, doub
     lv.push_back(std::move(L));
     // can we coarsen further?
     bool can = true;
-    if (const char* ml = getenv("PDE_B200_MAX_LEVELS")) can = can && (level + 1 < atoi(ml));
     int32_t nc2[3] = {0, 0, 0};
     // vector (elasticity) operators: re-discretised P1 operators on grids with a single cell across the body are
     // far too stiff in bending (locking), which spoils the coarse correction (33 -> ~20 PCG iterations on the
     // cantilever when the hierarchy stops at two cells across); scalar operators coarsen down to one cell
-    static const int env_min = getenv("PDE_B200_MIN_COARSE_CELLS") ? atoi(getenv("PDE_B200_MIN_COARSE_CELLS")) : 0;
-    const int min_cells = env_min > 0 ? env_min : (ncomp > 1 ? 2 : 1);
+    const int min_cells = ncomp > 1 ? 2 : 1;
     for (int q = 0; q < nax; ++q) {
       if (n[q] % 2 != 0 || n[q] < 2) can = false;
       nc2[q] = n[q] / 2;
@@ -373,7 +370,7 @@ int Hierarchy::build(pde_ctx* c, const Operator& fine, int kind, double p0, doub
     long long nfree = count_free_and_index(gg, Lc.op.bc, ncomp, nullptr, nullptr);
     if (nfree > 0 && nfree <= PDE_DENSE_MAX) PDE_OK(build_dense_coarse(c, Lc, dim, n, Lu));
   }
-  if (ncomp > 1 && !getenv("PDE_B200_NO_LMAX_EST"))
+  if (ncomp > 1)
     for (auto& L : lv) PDE_OK(estimate_lmax(c, *L, 12));
   return 0;
 }
@@ -392,35 +389,6 @@ void Hierarchy::release() {
   }
   lv.clear();
 }
-
-struct Cheby {
-  double theta, delta, sigma, rho, lmax_;
-  int kind = 1;  // 1: first-kind Chebyshev on [lmax/ratio, lmax]; 4: fourth-kind (Lottes), needs lmax only
-  void init(double lmax, double ratio) {
-    static const int env_kind = getenv("PDE_B200_CHEBY_KIND") ? atoi(getenv("PDE_B200_CHEBY_KIND")) : 1;
-    kind = env_kind == 4 ? 4 : 1;
-    lmax_ = lmax;
-    const double lmin = lmax / ratio;
-    theta = 0.5 * (lmax + lmin);
-    delta = 0.5 * (lmax - lmin);
-    sigma = theta / delta;
-    rho = 1.0 / sigma;
-  }
-  // coefficients of sweep k (k = 0 restarts the recurrence): d = c1 d + c2 Dinv r
-  void coef(int k, double* c1, double* c2) {
-    if (kind == 4) {
-      if (k == 0) { *c1 = 0.0; *c2 = 4.0 / (3.0 * lmax_); return; }
-      *c1 = (2.0 * k - 1.0) / (2.0 * k + 3.0);
-      *c2 = (8.0 * k + 4.0) / ((2.0 * k + 3.0) * lmax_);
-      return;
-    }
-    if (k == 0) { rho = 1.0 / sigma; *c1 = 0.0; *c2 = 1.0 / theta; return; }
-    const double rn = 1.0 / (2.0 * sigma - rho);
-    *c1 = rn * rho;
-    *c2 = 2.0 * rn / delta;
-    rho = rn;
-  }
-};
 
 // Chebyshev(Jacobi) smoothing.  dot_slot >= 0: the LAST sweep also leaves sum b.x_new in that scalar slot
 // (*dot_done tells whether a sweep could do it).
@@ -458,7 +426,7 @@ static int smooth(pde_ctx* c, MGLevel& L, const double* b, double** cur, double*
   }
   // (the applicability test comes first: on slab levels too small for the fused kernels the two halo exchanges below
   // would be thrown away and repeated by the sweep loop)
-  if (!zero_guess && sweeps == 2 && post2_applicable(L.op.g, L.op.dev) && (c->world == 1 || L.op.g.nzl >= PDE_NG)) {
+  if (!zero_guess && sweeps == 2 && heat2_applicable(L.op.g, L.op.dev) && (c->world == 1 || L.op.g.nzl >= PDE_NG)) {
     // both sweeps in one pass over the data (needs two halo planes of the iterate and one of the rhs)
     double c1a, c2a, c1b, c2b;
     ch.coef(0, &c1a, &c2a);
@@ -471,11 +439,6 @@ static int smooth(pde_ctx* c, MGLevel& L, const double* b, double** cur, double*
     PDE_OK(launch_heat_post2(c, L.op.g, L.op.dev, *cur, b, *oth, c2a, c1b, c2b, dot_slot, &handled));
     if (handled) {
       L.paths |= PDE_MG_HEAT_POST2;
-    } else {
-      PDE_OK(launch_post2(c, L.op.g, L.op.bc, L.op.dev, *cur, b, *oth, c2a, c1b, c2b, dot_slot, &handled));
-      if (handled) L.paths |= PDE_MG_POST2_R1;
-    }
-    if (handled) {
       std::swap(*cur, *oth);
       if (dot_slot >= 0 && dot_done) *dot_done = true;
       return 0;
@@ -513,7 +476,7 @@ int Hierarchy::vcycle(pde_ctx* c, const Operator& fine, const double* b0, double
   for (int l = 0; l + 1 < nl; ++l)
     lean[l] = c->world > 1 && !lv[l]->replicated && nu == 2 && lv[l]->op.dev.uniform_diag && lv[l]->op.dev.ncomp == 1 && lv[l]->op.g.dim == 3 &&
               lv[l]->op.g.nzl >= 8 && lv[l + 1]->op.g.nzl >= PDE_NG && sweep_applicable(lv[l]->op.g, 1) &&
-              !getenv("PDE_B200_NO_POST2") && !getenv("PDE_B200_NO_LEAN_HALO");
+              !getenv("PDE_B200_NO_LEAN_HALO");
   // down: pre-smoothing and residual of level l, restriction into level l+1
   auto down = [&](int l) -> int {
     MGLevel& L = *lv[l];
@@ -637,8 +600,7 @@ int Hierarchy::vcycle(pde_ctx* c, const Operator& fine, const double* b0, double
     *z_out = cur[0];
     return 0;
   }
-  static const int graph_env = getenv("PDE_B200_MG_GRAPH") ? atoi(getenv("PDE_B200_MG_GRAPH")) : 1;
-  if (gstate == 0 && !(graph_env && (solo ? nl >= 3 : nl - R >= 2))) gstate = -1;
+  if (gstate == 0 && !(solo ? nl >= 3 : nl - R >= 2)) gstate = -1;
   PDE_OK(down(0));
   if (solo) {
     PDE_OK(run_graph_part());
@@ -703,13 +665,6 @@ int pcg_solve(pde_ctx* c, const Operator& A, Hierarchy* mg, PcgWork& w, double* 
     PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, z, S_RHO0, S_RHO0, 1, 0));
   }
   PDE_OK(read_scal(c, S_RHO0 + 1, 1, &rr));
-  const bool trace = getenv("PDE_B200_TRACE") != nullptr;
-  if (trace) {
-    double v[2];
-    PDE_OK(read_scal(c, S_RHO0, 2, v));
-    fprintf(stderr, "[pcg] n=%lld gmg=%d levels=%d bnorm2=%.6e rho0=%.6e rr0=%.6e\n", (long long)g.total, (int)gmg,
-            gmg ? mg->levels() : 1, bnorm2, v[0], v[1]);
-  }
   int it = 0;
   bool conv = rr <= tol2;
   const int check = gmg ? 1 : (o.check_every > 0 ? o.check_every : 10);
@@ -734,12 +689,6 @@ int pcg_solve(pde_ctx* c, const Operator& A, Hierarchy* mg, PcgWork& w, double* 
     }
     PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, gmg ? z : r, sr, sn, 0, !gmg, gmg ? x : nullptr, S_XY));
     ++it;
-    if (trace && (it <= 30 || it % 50 == 0)) {
-      double v[2], pap;
-      PDE_OK(read_scal(c, sn, 2, v));
-      PDE_OK(read_scal(c, S_XY, 1, &pap));
-      fprintf(stderr, "[pcg] it=%d pAp=%.6e rho=%.6e rr=%.6e\n", it, pap, v[0], v[1]);
-    }
     if (it % check == 0 || it >= o.max_iters) {
       PDE_OK(read_scal(c, sn + 1, 1, &rr));
       if (!(rr == rr)) PDE_FAIL("PCG broke down (NaN residual)");

@@ -59,6 +59,26 @@ struct Hierarchy {
   long long gnodes = 0;      // kernels inside the graph (for the launch count)
 };
 
+// First-kind Chebyshev(Jacobi) smoother on [lmax/ratio, lmax]: the recurrence d = c1 d + c2 Dinv r of sweep k
+struct Cheby {
+  double theta, delta, sigma, rho;
+  void init(double lmax, double ratio) {
+    const double lmin = lmax / ratio;
+    theta = 0.5 * (lmax + lmin);
+    delta = 0.5 * (lmax - lmin);
+    sigma = theta / delta;
+    rho = 1.0 / sigma;
+  }
+  // coefficients of sweep k (k = 0 restarts the recurrence)
+  void coef(int k, double* c1, double* c2) {
+    if (k == 0) { rho = 1.0 / sigma; *c1 = 0.0; *c2 = 1.0 / theta; return; }
+    const double rn = 1.0 / (2.0 * sigma - rho);
+    *c1 = rn * rho;
+    *c2 = 2.0 * rn / delta;
+    rho = rn;
+  }
+};
+
 struct PcgWork {
   Field p, q;
   int alloc(pde_ctx* c, const Grid& g, int ncomp);

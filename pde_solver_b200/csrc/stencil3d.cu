@@ -18,6 +18,7 @@
 
 #include <cmath>
 
+#include <algorithm>
 #include <map>
 #include <mutex>
 #include <type_traits>
@@ -34,7 +35,6 @@ struct SweepGeom {
   int zc;             // planes per chunk
   int ns;             // strips (of YS rows) per tile
   int stage_elems;    // doubles per stage (all components), multiple of 16
-  int spec;           // 1: the last warp is a dedicated TMA producer (empty/full mbarriers, no CTA barrier)
   int zlo, zhi;       // output plane range [zlo, zhi): [0, nzl), or [-1, nzl+1) when the ghost planes are computed too
 };
 
@@ -145,7 +145,7 @@ enum { M_APPLY = 0, M_RESID = 1, M_CHEBY = 2, M_FIRST2 = 3 };
 #ifndef SW_MINB3
 #define SW_MINB3 1
 #endif
-template <int NC, int YS, int MODE, bool SPEC>
+template <int NC, int YS, int MODE>
 __global__ void __launch_bounds__(NC == 1 ? SW_MAXT1 : SW_MAXT3, NC == 1 ? SW_MINB1 : SW_MINB3)
 k_sweep3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ Grid g, const __grid_constant__ BcDev bc,
           const __grid_constant__ Coef<NC> C, const __grid_constant__ SweepArgs a, const __grid_constant__ SweepGeom sw,
@@ -172,44 +172,21 @@ k_sweep3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ Grid 
   const uint32_t stg0 = smem_u32(stage0);
   const uint32_t stage_stride = (uint32_t)(sw.stage_elems * sizeof(double));
 
-  // warp specialisation: the LAST warp of the CTA only feeds the TMA ring; the others compute.
-  //   full[s]  : TMA transaction barrier of stage s (1 arrival + bytes)
-  //   empty[s] : one arrival per compute warp once it has read stage s
-  constexpr bool spec = SPEC;
-  const int ncw = (int)(blockDim.x >> 5) - (spec ? 1 : 0);  // compute warps
-  const uint32_t ebar0 = bar0 + 8 * SW_STAGES;
+  // full[s]: TMA transaction barrier of stage s (1 arrival + bytes); thread 0 refills a stage after the CTA barrier
+  // that follows its last read
   if (t == 0) {
 #pragma unroll
-    for (int s = 0; s < SW_STAGES; ++s) {
-      mbar_init(bar0 + 8 * s, 1);
-      mbar_init(ebar0 + 8 * s, (uint32_t)ncw);
-    }
+    for (int s = 0; s < SW_STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-  if (!spec && t == 0) {
+  if (t == 0) {
     for (int i = 0; i < SW_STAGES && i < nplanes; ++i) {
       mbar_expect_tx(bar0 + 8 * i, stage_bytes);
+      // tensor z coordinate: local plane lz is z = lz + PDE_NG (the ghost planes come first).  The box starts at x0-2: TMA needs
+      // the inner start coordinate 16-byte aligned (even for FP64); x0-1 raises an illegal-instruction fault
       tma_load_4d(stg0 + i * stage_stride, &tmx, x0 - 2, y0 - 1, za + i - 1 + PDE_NG, 0, bar0 + 8 * i);
     }
-  }
-  if (spec && (t >> 5) == ncw) {
-    // ---- producer warp ----
-    if ((t & 31) == 0) {
-      for (int i = 0; i < nplanes; ++i) {
-        const int stage = i % SW_STAGES;
-        if (i >= SW_STAGES) mbar_wait(ebar0 + 8 * stage, (uint32_t)(((i / SW_STAGES) - 1) & 1));
-        mbar_expect_tx(bar0 + 8 * stage, stage_bytes);
-        // tensor z coordinate: local plane lz is z = lz + PDE_NG (the ghost planes come first).  The box starts at x0-2: TMA needs
-        // the inner start coordinate 16-byte aligned (even for FP64); x0-1 raises an illegal-instruction fault
-        tma_load_4d(stg0 + stage * stage_stride, &tmx, x0 - 2, y0 - 1, za + i - 1 + PDE_NG, 0, bar0 + 8 * stage);
-      }
-    }
-    if (a.do_reduce) {  // the block reduction below is CTA-wide
-      if (MODE >= M_CHEBY) { double v[1] = {0.0}; block_reduce_finalize<1>(v, red, red_out); }
-      else { double v[2] = {0.0, 0.0}; block_reduce_finalize<2>(v, red, red_out); }
-    }
-    return;
   }
 
   const int lx = t % sw.tx;
@@ -336,15 +313,10 @@ k_sweep3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ Grid 
       }
       plane_contrib<NC, YS>(C, V, aP, a0, aM);
     }
-    if (spec) {
-      __syncwarp();  // this warp has consumed the stage: hand it back to the producer
-      if ((t & 31) == 0) mbar_arrive(ebar0 + 8 * stage);
-    } else {
-      __syncthreads();  // every thread has consumed this stage
-      if (t == 0 && i + SW_STAGES < nplanes) {
-        mbar_expect_tx(bar0 + 8 * stage, stage_bytes);
-        tma_load_4d(stg0 + stage * stage_stride, &tmx, x0 - 2, y0 - 1, za + i + SW_STAGES - 1 + PDE_NG, 0, bar0 + 8 * stage);
-      }
+    __syncthreads();  // every thread has consumed this stage
+    if (t == 0 && i + SW_STAGES < nplanes) {
+      mbar_expect_tx(bar0 + 8 * stage, stage_bytes);
+      tma_load_4d(stg0 + stage * stage_stride, &tmx, x0 - 2, y0 - 1, za + i + SW_STAGES - 1 + PDE_NG, 0, bar0 + 8 * stage);
     }
     if (FIN) {
       const int gz = zout + g.z0;
@@ -418,220 +390,6 @@ k_sweep3d(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ Grid 
   }
 }
 
-// ----------------------------------------------------------------------------------------------------
-// k_post2: TWO Chebyshev-Jacobi sweeps in ONE pass over the data (temporal blocking), for scalar operators
-// whose free nodes all carry the interior stencil (every face Dirichlet):
-//     d0 = a0 (b - A x0),  x1 = x0 + d0 ;   d1 = c1 d0 + a1 (b - A x1),  x2 = x1 + d1        (a_k = c2_k / diag)
-// reads x0 and b, writes x2: 24 B/dof instead of 24 + 32 for two separate sweeps.
-//   Stage A runs the plane sweep on the output tile grown by one node in x and y (and one plane in z) and
-//   leaves x1, d0 of the plane it retires in a 3-slot shared-memory ring; stage B runs the same plane sweep on
-//   that ring, one plane behind, and retires x2.  A thread owns column c of the grown tile in both stages, a
-//   strip of YSB+1 rows in stage A and YSB rows in stage B; TY = 2*YSB rows of output per tile.
-//   Input planes za-2 .. zb+1 are needed for outputs za .. zb-1: fields carry PDE_NG = 2 ghost planes.
-// ----------------------------------------------------------------------------------------------------
-// tuned on B200 by A/B builds (heat 512^3 step, ms): YSB/threads/minBlocks 3/192/2 68.4, 4/192/2 66.7, 4/128/3 66.4,
-// 2/192/3 71.5, 5/192/2 76.6, 6/192/1 72.9
-#ifndef P2_MAXT
-#define P2_MAXT 128
-#endif
-#ifndef P2_MINB
-#define P2_MINB 3
-#endif
-#ifndef P2_YSB
-#define P2_YSB 4
-#endif
-
-struct Post2Geom {
-  int tx, ty;          // output tile
-  int cw, ra;          // grown tile: tx+2 columns, ty+2 rows
-  int bx, by;          // TMA box (tx+4, ty+4), origin (x0-2, y0-2)
-  int ntx, nty, nzc, zc;
-  int stage_elems;     // doubles per TMA stage (multiple of 16)
-  int ring_elems;      // doubles per ring slot (cw*ra rounded up)
-};
-struct Post2Args {
-  const double* b;
-  double* y;
-  double a0, c1, a1;
-  int do_reduce;
-};
-
-template <int YSB>
-__global__ void __launch_bounds__(P2_MAXT, P2_MINB)
-k_post2(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ Grid g, const __grid_constant__ Coef<1> C,
-        const __grid_constant__ Post2Args a, const __grid_constant__ Post2Geom pg, ReduceBuf red, double* red_out) {
-  constexpr int YSA = YSB + 1;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  double* stage0 = reinterpret_cast<double*>(smem_raw);
-  double* x1ring = stage0 + (size_t)SW_STAGES * pg.stage_elems;
-  double* d0ring = x1ring + 3 * (size_t)pg.ring_elems;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(d0ring + 3 * (size_t)pg.ring_elems);
-
-  const int t = threadIdx.x;
-  const int item = blockIdx.x;
-  const int itx = item % pg.ntx;
-  const int ity = (item / pg.ntx) % pg.nty;
-  const int izc = item / (pg.ntx * pg.nty);
-  const int x0 = itx * pg.tx, y0 = ity * pg.ty;
-  const int za = izc * pg.zc;
-  const int zb = min(za + pg.zc, g.nzl);
-  const int nplanes = zb - za + 4;  // input planes za-2 .. zb+1
-  const uint32_t stage_bytes = (uint32_t)(pg.bx * pg.by * sizeof(double));
-  const uint32_t bar0 = smem_u32(bars);
-  const uint32_t stg0 = smem_u32(stage0);
-  const uint32_t stage_stride = (uint32_t)(pg.stage_elems * sizeof(double));
-
-  if (t == 0) {
-#pragma unroll
-    for (int s = 0; s < SW_STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  if (t == 0) {
-    for (int i = 0; i < SW_STAGES && i < nplanes; ++i) {
-      mbar_expect_tx(bar0 + 8 * i, stage_bytes);
-      tma_load_4d(stg0 + i * stage_stride, &tmx, x0 - 2, y0 - 2, za - 2 + i + PDE_NG, 0, bar0 + 8 * i);
-    }
-  }
-
-  const int c = t % pg.cw;           // column of the grown tile: x = x0 - 1 + c
-  int s = t / pg.cw;
-  const bool active = s < 2;
-  if (!active) s = 0;                // surplus threads shadow strip 0 and never store
-  const int ixA = x0 - 1 + c;
-  const int cB = min(max(c, 1), pg.cw - 2);  // stage-B column used for addressing (clamped for the two edge columns)
-  const bool colB = active && c >= 1 && c <= pg.tx && ixA < g.nn[0];
-  // stage A: rows rA = s*YSA + j of the grown tile (y = y0 - 1 + rA); stage B: rows rB = s*YSB + j (y = y0 + rB)
-  double mA[YSA], mB[YSB];
-  unsigned loadA = 0, validB = 0;
-  const bool xfree = ixA >= 1 && ixA <= g.nn[0] - 2;
-#pragma unroll
-  for (int j = 0; j < YSA; ++j) {
-    const int iy = y0 - 1 + s * YSA + j;
-    const bool f = active && xfree && iy >= 1 && iy <= g.nn[1] - 2;
-    mA[j] = f ? 1.0 : 0.0;
-    if (f) loadA |= 1u << j;
-  }
-#pragma unroll
-  for (int j = 0; j < YSB; ++j) {
-    const int iy = y0 + s * YSB + j;
-    const bool v = colB && iy < g.nn[1];
-    if (v) validB |= 1u << j;
-    mB[j] = (v && xfree && iy >= 1 && iy <= g.nn[1] - 2) ? 1.0 : 0.0;
-  }
-  const double* sbaseA = stage0 + (s * YSA) * pg.bx + c;                 // V[r][cc] = sbaseA[r*bx + cc]
-  const int ringA = (s * YSA) * pg.cw + c;                               // ring offset of stage-A row j: + j*cw
-  const int ringB = (s * YSB) * pg.cw + cB - 1;                          // VB[r][cc] = ring[ringB + r*cw + cc]
-  const int ringOwn = (s * YSB + 1) * pg.cw + cB;                        // own node of stage-B row j: + j*cw
-  const unsigned colA0 = (unsigned)((long long)g.PX * (y0 - 1 + s * YSA) + ixA);  // only used where loadA is set
-  const unsigned colB0 = (unsigned)((long long)g.PX * (y0 + s * YSB) + ixA);
-
-  double aA[YSA][1], aB[YSA][1], aC[YSA][1];     // stage-A accumulators (three planes in flight)
-  double bA_[YSB][1], bB_[YSB][1], bC_[YSB][1];  // stage-B accumulators
-  double xA[YSA], xB[YSA], xC[YSA];              // own-column x0 values of the resident / previous plane
-#pragma unroll
-  for (int j = 0; j < YSA; ++j) aA[j][0] = aB[j][0] = aC[j][0] = xA[j] = xB[j] = xC[j] = 0.0;
-#pragma unroll
-  for (int j = 0; j < YSB; ++j) bA_[j][0] = bB_[j][0] = bC_[j][0] = 0.0;
-  double red_xy = 0.0;
-
-  auto body = [&](int i, double (&aP)[YSA][1], double (&a0)[YSA][1], double (&aM)[YSA][1], double (&bP)[YSB][1],
-                  double (&b0)[YSB][1], double (&bM)[YSB][1], double (&xprev)[YSA], double (&xcur)[YSA]) {
-    const int stage = i % SW_STAGES;
-    const uint32_t parity = (uint32_t)((i / SW_STAGES) & 1);
-    const int q = za - 2 + i;        // resident input plane
-    const int pA = q - 1;            // plane stage A retires (x1, d0)
-    const int pB = q - 2;            // plane stage B retires (x2)
-    const bool finA = i >= 2, finB = i >= 4;
-    // early global loads of the right-hand side for the two retiring planes
-    double rhsA[YSA], rhsB[YSB];
-    if (finA) {
-      const double* bp = a.b + (long long)g.plane * pA;
-#pragma unroll
-      for (int j = 0; j < YSA; ++j) rhsA[j] = ((loadA >> j) & 1u) ? bp[colA0 + (unsigned)j * (unsigned)g.PX] : 0.0;
-    }
-    if (finB) {
-      const double* bp = a.b + (long long)g.plane * pB;
-#pragma unroll
-      for (int j = 0; j < YSB; ++j) rhsB[j] = ((validB >> j) & 1u) ? bp[colB0 + (unsigned)j * (unsigned)g.PX] : 0.0;
-    }
-    mbar_wait(bar0 + 8 * stage, parity);
-    {  // ---- stage A: plane q of x0 ----
-      double V[YSA + 2][3][1];
-      const double* sp = sbaseA + (size_t)stage * pg.stage_elems;
-#pragma unroll
-      for (int r = 0; r < YSA + 2; ++r)
-#pragma unroll
-        for (int cc = 0; cc < 3; ++cc) {
-          if ((r == 0 && cc == 2) || (r == YSA + 1 && cc == 0)) V[r][cc][0] = 0.0;  // never used
-          else V[r][cc][0] = sp[r * pg.bx + cc];
-        }
-#pragma unroll
-      for (int j = 0; j < YSA; ++j) xcur[j] = V[j + 1][1][0];
-      plane_contrib<1, YSA>(C, V, aP, a0, aM);
-    }
-    const int slotA = (pA + 3) % 3;
-    if (finA) {
-      const int gz = pA + g.z0;
-      const double mz = (gz >= 1 && gz <= g.nzg - 2) ? 1.0 : 0.0;
-      double* x1s = x1ring + (size_t)slotA * pg.ring_elems + ringA;
-      double* d0s = d0ring + (size_t)slotA * pg.ring_elems + ringA;
-      if (active) {
-#pragma unroll
-        for (int j = 0; j < YSA; ++j) {
-          const double d0 = mA[j] * mz * a.a0 * (rhsA[j] - aP[j][0]);
-          x1s[j * pg.cw] = xprev[j] + d0;
-          d0s[j * pg.cw] = d0;
-        }
-      }
-    }
-    __syncthreads();  // the TMA stage is consumed and plane pA of x1 / d0 is visible
-    if (t == 0 && i + SW_STAGES < nplanes) {
-      mbar_expect_tx(bar0 + 8 * stage, stage_bytes);
-      tma_load_4d(stg0 + stage * stage_stride, &tmx, x0 - 2, y0 - 2, za - 2 + i + SW_STAGES + PDE_NG, 0, bar0 + 8 * stage);
-    }
-    if (finA) {  // ---- stage B: plane pA of x1 ----
-      double V[YSB + 2][3][1];
-      const double* rp = x1ring + (size_t)slotA * pg.ring_elems + ringB;
-#pragma unroll
-      for (int r = 0; r < YSB + 2; ++r)
-#pragma unroll
-        for (int cc = 0; cc < 3; ++cc) {
-          if ((r == 0 && cc == 2) || (r == YSB + 1 && cc == 0)) V[r][cc][0] = 0.0;
-          else V[r][cc][0] = rp[r * pg.cw + cc];
-        }
-      plane_contrib<1, YSB>(C, V, bP, b0, bM);
-    }
-    if (finB) {
-      const int slotB = (pB + 3) % 3;
-      const int gz = pB + g.z0;
-      const double mz = (gz >= 1 && gz <= g.nzg - 2) ? 1.0 : 0.0;
-      const double* x1o = x1ring + (size_t)slotB * pg.ring_elems + ringOwn;
-      const double* d0o = d0ring + (size_t)slotB * pg.ring_elems + ringOwn;
-      double* yp = a.y + (long long)g.plane * pB;
-#pragma unroll
-      for (int j = 0; j < YSB; ++j) {
-        const double x1 = x1o[j * pg.cw], d0 = d0o[j * pg.cw];
-        const double d1 = mB[j] * mz * fma(a.c1, d0, a.a1 * (rhsB[j] - bP[j][0]));
-        const double x2 = x1 + d1;
-        if ((validB >> j) & 1u) yp[colB0 + (unsigned)j * (unsigned)g.PX] = x2;
-        red_xy = fma(mB[j] * mz * rhsB[j], x2, red_xy);
-      }
-    }
-  };
-
-  // stage-A roles rotate from step 0, stage-B roles from step 2 (its first plane): phase (i+1) mod 3
-  for (int i = 0; i < nplanes; i += 3) {
-    body(i, aA, aB, aC, bB_, bC_, bA_, xC, xA);
-    if (i + 1 < nplanes) body(i + 1, aB, aC, aA, bC_, bA_, bB_, xA, xB);
-    if (i + 2 < nplanes) body(i + 2, aC, aA, aB, bA_, bB_, bC_, xB, xC);
-  }
-  if (a.do_reduce) {
-    double v[1] = {red_xy};
-    block_reduce_finalize<1>(v, red, red_out);
-  }
-}
-
 // ---- host side: tensor maps, tile geometry, launch ---------------------------------------------------
 typedef CUresult (*PFN_tmEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                       const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -693,33 +451,18 @@ int field_tensor_map(const double* field, const Grid& g, int nc, int bx, int by,
 }
 
 
-struct SweepTune {
-  int nt, zc, ys, txmax, spec;
-};
-static const SweepTune& sweep_tune() {
-  static SweepTune t = {env_int("PDE_B200_SW_NT", 0), env_int("PDE_B200_SW_ZC", 64), env_int("PDE_B200_SW_YS", 0),
-                        env_int("PDE_B200_SW_TXMAX", 0), env_int("PDE_B200_SW_SPEC", -1)};
-  return t;
-}
-
-template <int NC, int YS, int MODE, bool SPEC>
+template <int NC, int YS, int MODE>
 static int launch_sweep_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a) {
-  const SweepTune& tu = sweep_tune();
   SweepGeom sw;
-  sw.spec = SPEC ? 1 : 0;
-  int txmax = tu.txmax > 0 ? tu.txmax : (NC == 1 ? 192 : 64);  // tuned on B200: heat 512^3, elasticity 1280x256x256
-  txmax = txmax < 32 ? 32 : (txmax > 254 ? 254 : txmax);
-  // room for the producer warp of the warp-specialised variant (and the even rounding of tx)
-  static const int txmargin = env_int("PDE_B200_SW_TXMARGIN", 2);   // 513 nodes: 3 tiles of 172 on 192 threads (A/B: apply 0.397 -> 0.375 ms)
-  const int margin = SPEC ? 34 : (txmargin < 2 ? 2 : txmargin);
-  if (txmax > (NC == 1 ? SW_MAXT1 : SW_MAXT3) - margin) txmax = (NC == 1 ? SW_MAXT1 : SW_MAXT3) - margin;
+  constexpr int maxnt = NC == 1 ? SW_MAXT1 : SW_MAXT3;
+  // tile width and threads per CTA tuned on B200 (heat 512^3, elasticity 1280x256x256); two columns of margin for the
+  // even rounding of tx (513 nodes: 3 tiles of 172 on 192 threads, A/B: apply 0.397 -> 0.375 ms)
+  const int txmax = std::min(NC == 1 ? 192 : 64, maxnt - 2);
+  const int nt_target = std::min(NC == 1 ? 192 : 128, maxnt);
   sw.ntx = (g.nn[0] + txmax - 1) / txmax;
   sw.tx = (g.nn[0] + sw.ntx - 1) / sw.ntx;
   sw.tx += sw.tx & 1;  // even: the TMA box row must be a multiple of 16 bytes
   sw.ntx = (g.nn[0] + sw.tx - 1) / sw.tx;
-  const int maxnt = (NC == 1 ? SW_MAXT1 : SW_MAXT3) - (SPEC ? 32 : 0);  // a producer warp is extra
-  int nt_target = tu.nt > 0 ? tu.nt : (NC == 1 ? 192 : 128);
-  nt_target = nt_target < 64 ? 64 : (nt_target > maxnt ? maxnt : nt_target);
   sw.ns = nt_target / sw.tx;
   if (sw.ns < 1) sw.ns = 1;
   const int max_ns = (g.nn[1] + YS - 1) / YS;
@@ -731,7 +474,7 @@ static int launch_sweep_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDe
   sw.bx = sw.tx + 4;
   sw.by = sw.ty + 2;
   if (sw.bx > 256 || sw.by > 256) PDE_FAIL("sweep TMA box exceeds 256");
-  int zc = tu.zc < 2 ? 2 : tu.zc;
+  int zc = 64;
   // small grids (coarse multigrid levels): shorter z chunks so that the grid still covers the SMs
   while (zc > 4 && (long long)sw.ntx * sw.nty * ((g.nzl + zc - 1) / zc) < 4LL * c->sm_count) zc /= 2;
   // ghost_out: also produce the two ghost planes next to the slab (needs two valid halo planes of x and one of b),
@@ -746,8 +489,8 @@ static int launch_sweep_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDe
   sw.stage_elems = ((sw.bx * sw.by * NC + 15) / 16) * 16;
   const long long items = (long long)sw.ntx * sw.nty * sw.nzc;
   if (items > RED_MAX_BLOCKS) PDE_FAIL("sweep grid exceeds the reduction buffer");
-  const size_t smem = (size_t)SW_STAGES * sw.stage_elems * sizeof(double) + 2 * SW_STAGES * sizeof(uint64_t);
-  auto kern = k_sweep3d<NC, YS, MODE, SPEC>;
+  const size_t smem = (size_t)SW_STAGES * sw.stage_elems * sizeof(double) + SW_STAGES * sizeof(uint64_t);
+  auto kern = k_sweep3d<NC, YS, MODE>;
   static size_t smem_set = 0;
   if (smem > smem_set) {
     CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -766,7 +509,7 @@ static int launch_sweep_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDe
   for (int i = 0; i < 3; ++i) sa.dinv_int[i] = i < NC ? op.h_dinv_int[i] : 0.0;
   sa.do_reduce = a.reduce_slot_xy >= 0;
   double* out = sa.do_reduce ? c->scal + a.reduce_slot_xy : nullptr;
-  kern<<<(unsigned)items, nt + (sw.spec ? 32 : 0), smem, c->stream>>>(tm, g, bc, C, sa, sw, c->red, out);
+  kern<<<(unsigned)items, nt, smem, c->stream>>>(tm, g, bc, C, sa, sw, c->red, out);
   c->launches++;
   CUDA_OK(cudaGetLastError());
   // natural (non-Dirichlet) faces: their rows have incomplete element patches and come from the class table
@@ -774,70 +517,8 @@ static int launch_sweep_t(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDe
   return 0;
 }
 
-// Two Chebyshev sweeps (restart k = 0, 1) in one pass; returns *handled = false if the kernel does not apply.
-int launch_post2(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const double* x0, const double* b,
-                 double* y, double c2_0, double c1_1, double c2_1, int dot_slot, bool* handled) {
-  (void)bc;
-  *handled = false;
-  if (env_int("PDE_B200_NO_POST2", 0)) return 0;
-  if (g.dim != 3 || g.nk != PDE_NOFF || op.ncomp != 1 || !op.uniform_diag) return 0;
-  if (g.nn[0] < 32 || g.nn[1] < 8 || g.nzl < 8) return 0;
-  constexpr int YSB = P2_YSB;
-  static const int txmax_env = env_int("PDE_B200_P2_TXMAX", 94);
-  static const int zc_env = env_int("PDE_B200_P2_ZC", 64);
-  Post2Geom pg;
-  int txmax = txmax_env < 30 ? 30 : (txmax_env > P2_MAXT / 2 - 2 ? P2_MAXT / 2 - 2 : txmax_env);
-  pg.ntx = (g.nn[0] + txmax - 1) / txmax;
-  pg.tx = (g.nn[0] + pg.ntx - 1) / pg.ntx;
-  pg.tx += pg.tx & 1;
-  if (pg.tx > txmax) pg.tx = txmax - (txmax & 1);
-  pg.ntx = (g.nn[0] + pg.tx - 1) / pg.tx;
-  pg.ty = 2 * YSB;
-  pg.nty = (g.nn[1] + pg.ty - 1) / pg.ty;
-  pg.cw = pg.tx + 2;
-  pg.ra = pg.ty + 2;
-  pg.bx = pg.tx + 4;
-  pg.by = pg.ty + 4;
-  const int nt = ((2 * pg.cw + 31) / 32) * 32;
-  if (nt > P2_MAXT) PDE_FAIL("post2 tile exceeds the thread limit");
-  int zc = zc_env < 4 ? 4 : zc_env;
-  while (zc > 8 && (long long)pg.ntx * pg.nty * ((g.nzl + zc - 1) / zc) < 4LL * c->sm_count) zc /= 2;
-  pg.nzc = (g.nzl + zc - 1) / zc;
-  pg.zc = (g.nzl + pg.nzc - 1) / pg.nzc;
-  pg.nzc = (g.nzl + pg.zc - 1) / pg.zc;
-  pg.stage_elems = ((pg.bx * pg.by + 15) / 16) * 16;
-  pg.ring_elems = ((pg.cw * pg.ra + 15) / 16) * 16;
-  const long long items = (long long)pg.ntx * pg.nty * pg.nzc;
-  if (items > RED_MAX_BLOCKS) return 0;
-  const size_t smem = ((size_t)SW_STAGES * pg.stage_elems + 6 * (size_t)pg.ring_elems) * sizeof(double) +
-                      SW_STAGES * sizeof(uint64_t);
-  auto kern = k_post2<YSB>;
-  static size_t smem_set = 0;
-  if (smem > smem_set) {
-    CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_set = smem;
-  }
-  CUtensorMap tm;
-  PDE_OK(field_tensor_map(x0, g, 1, pg.bx, pg.by, &tm));
-  Coef<1> C;
-  for (int k = 0; k < PDE_NOFF; ++k) C.c[k][0] = op.h_int[k];
-  Post2Args pa;
-  pa.b = b; pa.y = y;
-  pa.a0 = c2_0 * op.h_dinv_int[0];
-  pa.c1 = c1_1;
-  pa.a1 = c2_1 * op.h_dinv_int[0];
-  pa.do_reduce = dot_slot >= 0;
-  kern<<<(unsigned)items, nt, smem, c->stream>>>(tm, g, C, pa, pg, c->red, pa.do_reduce ? c->scal + dot_slot : nullptr);
-  c->launches++;
-  CUDA_OK(cudaGetLastError());
-  *handled = true;
-  return 0;
-}
-
 // does the TMA plane-sweep kernel take this grid?  (callers that rely on its ghost-plane outputs must ask)
 bool sweep_applicable(const Grid& g, int ncomp) {
-  static const int off = env_int("PDE_B200_NO_SWEEP", 0);
-  if (off) return false;
   if (g.dim != 3 || g.nk != PDE_NOFF) return false;
   if (ncomp != 1 && ncomp != 3) return false;
   // small grids (coarse multigrid levels) stay on the generic kernel: they are launch-latency bound
@@ -938,8 +619,6 @@ k_sweep2d(const __grid_constant__ Grid g, const __grid_constant__ Coef2d C, cons
 }
 
 static bool sweep2d_applicable(const Grid& g, const OpDev& op, const StencilArgs& a) {
-  static const int off = env_int("PDE_B200_NO_SWEEP2D", 0);
-  if (off) return false;
   if (g.dim != 2 || g.nk != 7 || op.ncomp != 1 || !op.uniform_diag) return false;
   if (g.nn[0] < 128 || g.nzl < 8) return false;           // small levels stay on the table kernel (launch bound anyway)
   if (a.ghost_out) return false;
@@ -960,8 +639,7 @@ static int launch_sweep2d_t(pde_ctx* c, const Grid& g, const OpDev& op, const St
   for (int i = 0; i < 3; ++i) sa.dinv_int[i] = i < 1 ? op.h_dinv_int[i] : 0.0;
   sa.do_reduce = a.reduce_slot_xy >= 0;
   const int nbx = (g.nn[0] + 255) / 256;
-  int zc = env_int("PDE_B200_SW2D_ZC", 64);
-  zc = zc < 4 ? 4 : zc;
+  int zc = 64;
   while (zc > 8 && (long long)nbx * ((g.nzl + zc - 1) / zc) < 4LL * c->sm_count) zc /= 2;
   const int nbz = (g.nzl + zc - 1) / zc;
   if ((long long)nbx * nbz > RED_MAX_BLOCKS) PDE_FAIL("2-D sweep grid exceeds the reduction buffer");
@@ -974,6 +652,14 @@ static int launch_sweep2d_t(pde_ctx* c, const Grid& g, const OpDev& op, const St
 
 int launch_elast3d(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a, bool* handled);
 
+// strips of YS = 4 rows for the scalar operators, 2 for the vector ones
+template <int NC, int YS>
+static int launch_sweep(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a) {
+  if (a.cheby == 2) return launch_sweep_t<NC, YS, M_FIRST2>(c, g, bc, op, a);
+  if (a.cheby) return launch_sweep_t<NC, YS, M_CHEBY>(c, g, bc, op, a);
+  return a.b ? launch_sweep_t<NC, YS, M_RESID>(c, g, bc, op, a) : launch_sweep_t<NC, YS, M_APPLY>(c, g, bc, op, a);
+}
+
 int launch_stencil_fast(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op, const StencilArgs& a,
                         bool* handled) {
   *handled = false;
@@ -984,27 +670,9 @@ int launch_stencil_fast(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev&
     return a.b ? launch_sweep2d_t<M_RESID>(c, g, op, a) : launch_sweep2d_t<M_APPLY>(c, g, op, a);
   }
   if (!sweep_applicable(g, op.ncomp)) return 0;
-  const int ys = sweep_tune().ys;
   *handled = true;
-#define SWEEP_DISPATCH_S(NC_, YS_, SP_)                                                   \
-  do {                                                                                   \
-    if (a.cheby == 2) return launch_sweep_t<NC_, YS_, M_FIRST2, SP_>(c, g, bc, op, a);   \
-    if (a.cheby) return launch_sweep_t<NC_, YS_, M_CHEBY, SP_>(c, g, bc, op, a);         \
-    return a.b ? launch_sweep_t<NC_, YS_, M_RESID, SP_>(c, g, bc, op, a)                 \
-               : launch_sweep_t<NC_, YS_, M_APPLY, SP_>(c, g, bc, op, a);                \
-  } while (0)
-  // PDE_B200_SW_SPEC=1: dedicated TMA producer warp (measured slower than the CTA-barrier ring for both
-  // operators on B200, kept selectable)
-#define SWEEP_DISPATCH(NC_, YS_)                              \
-  do {                                                       \
-    if (sweep_tune().spec > 0) SWEEP_DISPATCH_S(NC_, YS_, true); \
-    SWEEP_DISPATCH_S(NC_, YS_, false);                       \
-  } while (0)
   if (a.cheby == 1 && !a.b) { *handled = false; return 0; }  // smoother sweeps always carry a rhs field
-  if (op.ncomp == 1) {
-    if (ys == 2) SWEEP_DISPATCH(1, 2);
-    SWEEP_DISPATCH(1, 4);
-  }
+  if (op.ncomp == 1) return launch_sweep<1, 4>(c, g, bc, op, a);
   if (op.ncomp == 3) {
     // the dedicated elasticity kernel (elast3d.cu) takes the launch when the table has the Kuhn-mesh pattern
     {
@@ -1023,8 +691,7 @@ int launch_stencil_fast(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev&
     for (int k = 7; k < PDE_NOFF; ++k)
       for (int i = 0; i < 3; ++i) ok = ok && fabs(op.h_int[k * 9 + i * 3 + i]) <= 1e-12 * mx;
     if (!ok) { *handled = false; return 0; }
-    if (ys == 1) SWEEP_DISPATCH(3, 1);
-    SWEEP_DISPATCH(3, 2);
+    return launch_sweep<3, 2>(c, g, bc, op, a);
   }
   *handled = false;
   return 0;

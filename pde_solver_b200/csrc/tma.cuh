@@ -1,7 +1,6 @@
 // TMA / mbarrier PTX wrappers and the tensor-map helper shared by the plane-sweep kernels (sm_100a).
 #pragma once
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "device.cuh"
 
@@ -12,9 +11,6 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok;
@@ -34,24 +30,8 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* tm,
       : "memory");
 }
 
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* tm, uint32_t src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(tm), "r"(src),
-               "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// the committed bulk stores have finished READING shared memory (the source buffer may be overwritten)
-__device__ __forceinline__ void tma_store_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// generic-proxy writes to shared memory become visible to the async proxy (TMA store source)
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// Tensor map of a padded field: (x, y, z incl. the ghost planes, component); out-of-range x/y read as 0 and are
-// clipped on stores.  Cached per (base, grid, box).
+// Tensor map of a padded field: (x, y, z incl. the ghost planes, component); out-of-range x/y read as 0.
+// Cached per (base, grid, box).
 // bz: planes per box (the sweeps load one plane at a time; the face kernel loads a whole neighbourhood).
 int field_tensor_map(const double* field, const Grid& g, int nc, int bx, int by, CUtensorMap* out, int bz = 1);
 
-static inline int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}

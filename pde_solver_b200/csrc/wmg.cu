@@ -348,26 +348,22 @@ void WHierarchy::release() {
   lv.clear();
 }
 
-// Chebyshev(Jacobi) on [lmax/ratio, lmax], the recurrence of solver.cu's first-kind smoother.  x lives in *cur on
-// entry and exit.  dot_slot >= 0: the last sweep also leaves sum b.x_new there (it must be a general sweep).
+// Chebyshev(Jacobi) on [lmax/ratio, lmax] (Cheby, solver.cuh).  x lives in *cur on entry and exit.  dot_slot >= 0: the
+// last sweep also leaves sum b.x_new there (it must be a general sweep).
 static int wsmooth(pde_ctx* c, const WHierarchy& H, WLevel& L, const double* b, double** cur, double** oth,
                    int sweeps, bool zero_guess, double ratio, int dot_slot) {
-  const double lmin = L.lmax / ratio;
-  const double theta = 0.5 * (L.lmax + lmin), delta = 0.5 * (L.lmax - lmin), sigma = theta / delta;
-  double rho = 1.0 / sigma;
+  Cheby ch;
+  ch.init(L.lmax, ratio);
   int k0 = 0;
   if (zero_guess) {
-    PDE_OK(wsweep(c, L, H.bc, W_FIRST, nullptr, b, nullptr, *cur, 0.0, 1.0 / theta, -1));
+    double c1, c2;
+    ch.coef(0, &c1, &c2);
+    PDE_OK(wsweep(c, L, H.bc, W_FIRST, nullptr, b, nullptr, *cur, 0.0, c2, -1));
     k0 = 1;
   }
   for (int k = k0; k < sweeps; ++k) {
-    double c1 = 0.0, c2 = 1.0 / theta;
-    if (k > 0) {
-      const double rn = 1.0 / (2.0 * sigma - rho);
-      c1 = rn * rho;
-      c2 = 2.0 * rn / delta;
-      rho = rn;
-    }
+    double c1, c2;
+    ch.coef(k, &c1, &c2);
     // x_{k-1}: none on a restart, zero after the first sweep from a zero guess, else the other buffer
     const double* xprev = (k == 0 || (zero_guess && k == 1)) ? nullptr : *oth;
     PDE_OK(wsweep(c, L, H.bc, W_CHEBY, *cur, b, xprev, *oth, c1, c2, k == sweeps - 1 ? dot_slot : -1));

@@ -121,6 +121,18 @@ def test_product_path_does_not_import_the_oracle():
                 assert "oracle" not in src.replace("# oracle", ""), fn
 
 
+def test_library_reads_only_the_multi_gpu_and_cell_rhs_switches():
+    # kernel variants are compared as separate library builds, not switched at run time: the CUDA library reads the
+    # environment only for the multi-GPU halo / hierarchy settings and the cell right-hand-side pass count
+    csrc = os.path.join(ROOT, "pde_solver_b200", "csrc")
+    read = set()
+    for fn in os.listdir(csrc):
+        src = open(os.path.join(csrc, fn)).read()
+        read |= set(re.findall(r"\b(?:getenv|env_int)\s*\(\s*\"(PDE_B200_\w+)\"", src))
+    assert read == {"PDE_B200_HALO", "PDE_B200_HALO_BLOCKS", "PDE_B200_HALO_DEBUG", "PDE_B200_REP_NODES",
+                    "PDE_B200_NO_LEAN_HALO", "PDE_B200_CELL_2PASS"}
+
+
 # ------------------------------------------------------------------ GPU: through MCP
 @pytest.mark.gpu
 def test_call_tool_in_process(server, tmp_path):

@@ -5,15 +5,10 @@ fixed linear map z = B b; pde_op_vcycle applies the solver's own hierarchy to a 
 
 CPU part: the model itself (B symmetric and positive, P^T equal to the restriction formula of k_restrict and the
 residual-restriction mode of k_heat_post2).  GPU part: B b against the model at every size the model can build, with
-info.paths pinning which fused kernels each case runs; the kernel variants behind the environment switches (each in a
-subprocess: the switches are read once per process); the PCG iteration count against the model; symmetry,
-positivity and graph-replay repeatability at the benchmark sizes."""
+info.paths pinning which fused kernels each case runs, and at other smoother degrees; the PCG iteration count against
+the model; symmetry, positivity and graph-replay repeatability at the benchmark sizes."""
 import copy
 import functools
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -21,12 +16,11 @@ import pytest
 from oracle import fem_oracle as fo
 from oracle import gmg_model as gm
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ALPHA, BETA = 1.0, 0.013
 LAME = fo.lame(210e9, 0.3, 3)
 # max|z - z_model| <= BAR * max|z_model|; worst measured on a B200: 1.7e-13 (elasticity 64x16x16), heat <= 3.6e-15
 BAR = 2e-11
-FIRST2, HEAT_POST2, POST2_R1, RR = 1, 2, 4, 8
+FIRST2, HEAT_POST2, RR = 1, 2, 8
 
 
 def dirichlet_pred(L, faces, side_excl=False):
@@ -50,7 +44,10 @@ CASES = {
     # level 0: 129 x 65 x 65 nodes, CW = 64 tiles (last x tile 5 columns, last y tile one row); levels 1-2: CW = 32
     # post2 + RR; then the generic kernels, dense coarsest level, graph
     "heat3d_128": dict(kind="heat", dim=3, n=(128, 64, 64), faces=ALL(3)),
-    # 121 / 61 nodes: CW = 32 with a one-column last x tile; coarsest 31 x 11 x 10 nodes, smoothed; graph
+    # 121 / 61 nodes: CW = 32 with a one-column last x tile; coarsest 31 x 11 x 10 nodes, smoothed; graph.
+    # Level 1 (61 x 21 x 19 nodes, 3 x 3 tiles) halves its z chunk from 64 to 8 to cover 6 x 148 SMs, then evens it out
+    # to ceil(19 / 3) = 7: chunks start at planes 0, 7 and 14, odd starts in both the post-smoothing and the
+    # residual-restriction mode of k_heat_post2
     "heat3d_120": dict(kind="heat", dim=3, n=(120, 40, 36), faces=ALL(3)),
     # two levels, smoothed coarsest, no graph
     "heat3d_130": dict(kind="heat", dim=3, n=(130, 40, 36), faces=ALL(3)),
@@ -201,7 +198,7 @@ def gpu_vcycle(P, ctx, name, nu=2):
     return _GPU[key]
 
 
-def check_against_model(name, b, z1, z3, bz, info, nu=2, graph=True):
+def check_against_model(name, b, z1, z3, bz, info, nu=2):
     """The checks every V-cycle case makes; returns max|z - z_model| / max|z_model|."""
     levels, free = model(name)
     nl = len(levels)
@@ -223,7 +220,7 @@ def check_against_model(name, b, z1, z3, bz, info, nu=2, graph=True):
     assert ratio <= BAR, ratio
     assert not z1[~free].any()
     assert np.array_equal(z3, z1)
-    assert info["graph"] == (1 if graph and nl >= 3 else 0)
+    assert info["graph"] == (1 if nl >= 3 else 0)
     assert abs(bz - b @ z1) <= 1e-12 * np.abs(b * z1).sum()
     return ratio
 
@@ -237,73 +234,14 @@ def test_vcycle_matches_model(P, ctx, name):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("nu", [1, 3])
-def test_vcycle_other_smoother_degrees_match_model(P, ctx, nu):
-    """nu = 1: no fused first sweeps, no post2; nu = 3: the sweep that rebuilds d from x1 = s0 D^-1 b (prev_mode 3)."""
-    name = "heat3d_128"
+@pytest.mark.parametrize("name,nu", [("heat3d_128", 1), ("heat3d_128", 3), ("elast3d_64", 3)],
+                         ids=["1", "3", "elast3d_64-3"])
+def test_vcycle_other_smoother_degrees_match_model(P, ctx, name, nu):
+    """nu = 1: no fused first sweeps, separate post sweeps; nu = 3: the sweep that rebuilds d from x1 = s0 D^-1 b
+    (prev_mode 3).  k_elast3d declines that sweep, so on elast3d_64 it runs the generic k_sweep3d<3, 2, CHEBY>."""
     b, z1, z3, bz, info = gpu_vcycle(P, ctx, name, nu)
     check_against_model(name, b, z1, z3, bz, info, nu=nu)
     assert info["paths"] == expected_paths(name, info["levels"], info["n_dense"], nu), info["paths"]
-
-
-_SUB = r"""
-import json, sys
-import numpy as np
-sys.path[:0] = [sys.argv[1], sys.argv[1] + "/tests"]
-import pde_solver_b200 as P
-from test_vcycle_parity import op_params, ncomp
-ctx = P._lib.default_context()
-out = sys.argv[2]
-for name in sys.argv[3:]:
-    b = np.load(f"{out}/{name}_b.npy")
-    z1, z3, bz, info = P._lib.op_vcycle(ctx, op_params(P, name), b.reshape(ncomp(name), -1),
-                                        P._lib.make_opts(precond="gmg"), ncycles=3)
-    np.save(f"{out}/{name}_z1.npy", z1.ravel())
-    np.save(f"{out}/{name}_z3.npy", z3.ravel())
-    with open(f"{out}/{name}_info.json", "w") as f:
-        json.dump(dict(info, bz=bz), f)
-"""
-
-VARIANTS = {
-    "no_rr": {"PDE_B200_NO_RR": "1"},
-    "no_heat2": {"PDE_B200_NO_HEAT2": "1"},                    # k_post2 + separate residual and restriction
-    "no_post2": {"PDE_B200_NO_HEAT2": "1", "PDE_B200_NO_POST2": "1"},
-    "cw32": {"PDE_B200_P2_CW": "32"},
-    "cw64_ysb3": {"PDE_B200_P2_CW": "64", "PDE_B200_P2_YSB": "3"},
-    "zc5": {"PDE_B200_P2_ZC": "5"},                            # odd z-chunk starts
-    "no_graph": {"PDE_B200_MG_GRAPH": "0"},
-    "no_sweep": {"PDE_B200_NO_SWEEP": "1"},
-}
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("variant", list(VARIANTS))
-def test_kernel_variants_match_model_and_default(P, ctx, variant, tmp_path):
-    names = ["heat3d_128", "heat3d_120"]
-    for name in names:
-        np.save(tmp_path / f"{name}_b.npy", rhs(name))
-    env = dict(os.environ, **VARIANTS[variant])
-    r = subprocess.run([sys.executable, "-c", _SUB, ROOT, str(tmp_path)] + names, env=env, cwd=ROOT,
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-4000:]
-    for name in names:
-        b = rhs(name)
-        z1, z3 = np.load(tmp_path / f"{name}_z1.npy"), np.load(tmp_path / f"{name}_z3.npy")
-        with open(tmp_path / f"{name}_info.json") as f:
-            info = json.load(f)
-        check_against_model(name, b, z1, z3, info["bz"], info, graph=variant != "no_graph")
-        _, z_def, _, _, info_def = gpu_vcycle(P, ctx, name)
-        assert np.abs(z1 - z_def).max() <= 1e-12 * np.abs(z_def).max()
-        p, p_def = info["paths"], info_def["paths"]
-        post = HEAT_POST2 | POST2_R1
-        if variant == "no_rr":
-            assert p[0] == p_def[0] & ~RR and p_def[0] & RR
-        elif variant == "no_heat2":
-            assert p[0] == (p_def[0] & ~(RR | post)) | POST2_R1 and p_def[0] & HEAT_POST2
-        elif variant == "no_post2":
-            assert p[0] == p_def[0] & ~(RR | post)
-        else:
-            assert p == p_def
 
 
 @pytest.mark.gpu
@@ -325,14 +263,16 @@ def test_pcg_iterations_match_model(P, ctx, name):
 
 FULL = [("heat", 3, [512, 512, 512], [1.0, 1.0, 1.0], None),
         ("heat", 2, [4096, 4096], [1.0, 1.0], None),
-        ("elasticity", 3, [640, 128, 128], [1.0, 0.2, 0.2], {0: 0.0})]
+        ("elasticity", 3, [640, 128, 128], [1.0, 0.2, 0.2], {0: 0.0}),
+        # thin in x: 1026 k_heat_post2 tiles per plane, whose z chunks must grow past 64 planes to fit the reduction buffer
+        ("heat", 3, [32, 4096, 4096], [1.0 / 128, 1.0, 1.0], None)]
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind,dim,n,L,faces", FULL)
 def test_vcycle_symmetric_positive_repeatable_at_full_size(P, ctx, kind, dim, n, L, faces):
-    """The bench.py workloads, where the model cannot run: u.Bv = v.Bu, u.Bu > 0, the replayed graph cycle repeats the
-    live one bit for bit; on 512^3 level 0 runs the fused kernels the benchmark times."""
+    """The bench.py workloads and a grid thin in x, where the model cannot run: u.Bv = v.Bu, u.Bu > 0, the replayed graph
+    cycle repeats the live one bit for bit; on the 3-D heat grids level 0 runs the fused kernels the benchmark times."""
     faces = faces if faces is not None else {f: 0.0 for f in range(2 * dim)}
     lam, mu = LAME
     p = P._lib.op_params(kind, dim, n, L, ALPHA, BETA, lam, mu, bc=P._lib.make_bc(faces))
