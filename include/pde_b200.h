@@ -117,7 +117,8 @@ typedef struct pde_stats {
   int32_t solves;        /* linear solves performed */
   int32_t converged;     /* 1 if every solve reached rtol */
   int32_t levels;        /* multigrid levels used (1 = Jacobi) */
-  int32_t reserved;
+  int32_t precond_applies; /* multigrid preconditioner applications (V-cycles) over all solves of the call: one per
+                              PCG iteration (iters_total), none for a start that already meets rtol; 0 for Jacobi */
   double final_relres;   /* last solve: ||r||/||b|| (recurrence) */
   double true_relres;    /* last solve: ||b - A x||/||b|| recomputed */
   double solve_ms;       /* device time of the solver region (CUDA events) */

@@ -25,12 +25,14 @@ class SolverOpts(C.Structure):
 
 class Stats(C.Structure):
     _fields_ = [("ndofs", C.c_int64), ("iters_total", C.c_int64), ("solves", C.c_int32),
-                ("converged", C.c_int32), ("levels", C.c_int32), ("reserved", C.c_int32),
+                ("converged", C.c_int32), ("levels", C.c_int32), ("precond_applies", C.c_int32),
                 ("final_relres", C.c_double), ("true_relres", C.c_double), ("solve_ms", C.c_double),
                 ("setup_ms", C.c_double), ("launches", C.c_int64)]
 
     def as_dict(self):
-        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+        """The published statistics (what last_stats() and the steppers report).  precond_applies, a check of the
+        solver loop, is read from the structure itself."""
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "precond_applies"}
 
 
 class HeatParams(C.Structure):

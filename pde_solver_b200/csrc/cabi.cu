@@ -421,27 +421,34 @@ static int heat_one_solve(pde_heat_state* s, pde_stats* st, bool verify = false)
     if (!s->un.p) PDE_OK(s->un.alloc(c, s->g, 1));
     PDE_OK(launch_copy(c, s->g, 1, s->un.p, s->u.p));
   }
+  // r0.r0 (for pcg_solve's first convergence test) comes from the pass that writes r0, into S_RHO1; ||b||^2 goes to
+  // S_RR, so one all-reduce and one poll carry both.  Slots S_RHO0 .. S_RR are free until PCG writes them.
   StencilArgs a;
-  a.x = s->u.p; a.y = s->r.p; a.bconst[0] = f; a.reduce_slot_xy = S_XY;
+  a.x = s->u.p; a.y = s->r.p; a.bconst[0] = f; a.reduce_slot_xy = S_RHO0;
   if (c->world > 1) PDE_OK(comm_halo_exchange(c, s->g, 1, s->u.p));
-  double bn2;
+  double rr0, bn2;
   if (p.steady) {
-    // r0 = f m - kappa K u0 (u0 = Dirichlet lift): this IS the reduced right-hand side
+    // r0 = f m - kappa K u0 (u0 = Dirichlet lift): this IS the reduced right-hand side, ||b||^2 = r0.r0
     a.bscale = 1.0; a.ascale = -1.0;
     PDE_OK(launch_stencil(c, s->g, s->bc, s->A.dev, a));
-    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_XY, 2));
-    PDE_OK(read_scal(c, S_YY, 1, &bn2));
+    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO1, 1));
+    PDE_OK(read_scal(c, S_RHO1, 1, &rr0));
+    bn2 = rr0;
   } else {
     // warm start x0 = u_n  =>  r0 = b - A u_n = dt (f m - kappa K u_n)   (b = M u_n + dt f m)
     a.bscale = p.dt; a.ascale = -p.dt * kappa;
     PDE_OK(launch_stencil(c, s->g, s->bc, s->K.dev, a));
-    StencilArgs nb;
-    nb.x = s->u.p; nb.y = nullptr; nb.bconst[0] = f; nb.bscale = p.dt; nb.ascale = 1.0; nb.reduce_slot_xy = S_XY;
+    StencilArgs nb;   // b: u.b into S_PAP, ||b||^2 into S_RR
+    nb.x = s->u.p; nb.y = nullptr; nb.bconst[0] = f; nb.bscale = p.dt; nb.ascale = 1.0; nb.reduce_slot_xy = S_PAP;
     PDE_OK(launch_stencil(c, s->g, s->bc, s->M.dev, nb));
-    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_XY, 2));
-    PDE_OK(read_scal(c, S_YY, 1, &bn2));
+    static_assert(S_RR == S_RHO1 + 2, "r0.r0 and ||b||^2 are read in one call");
+    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO1, 3));
+    double v[3];
+    PDE_OK(read_scal(c, S_RHO1, 3, v));
+    rr0 = v[0];
+    bn2 = v[2];
   }
-  PDE_OK(pcg_solve(c, s->A, s->use_mg ? &s->mg : nullptr, s->w, s->u.p, s->r.p, bn2, s->o, st));
+  PDE_OK(pcg_solve(c, s->A, s->use_mg ? &s->mg : nullptr, s->w, s->u.p, s->r.p, bn2, s->o, st, &rr0));
   if (verify) {
     StencilArgs t;
     t.y = s->r.p; t.reduce_slot_xy = S_XY;
@@ -579,6 +586,7 @@ extern "C" int pde_heat_solve(pde_ctx* c, const pde_heat_params* p, const pde_so
       if ((rc = pde_heat_step(s, 1, &st))) break;
       acc.true_relres = st.true_relres;
       acc.iters_total += st.iters_total;
+      acc.precond_applies += st.precond_applies;
       acc.solves += st.solves;
       acc.converged &= st.converged;
       acc.levels = st.levels;

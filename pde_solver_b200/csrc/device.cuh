@@ -221,7 +221,8 @@ int launch_face_rows(pde_ctx* c, const Grid& g, const BcDev& bc, const OpDev& op
 // Jacobi-PCG fused update: x += a p, r -= a q, rho_new = r.dinv r, rr = r.r  (a = rho/pAp from scal)
 int launch_cg_update(pde_ctx* c, const Grid& g, const OpDev& op, double* x, double* r, const double* p,
                      const double* q, int slot_rho, int slot_pap, int slot_rho_new, int slot_rr, int jacobi);
-// p = z + beta p with z = dinv r (jacobi) or z given; beta = rho_new/rho (first: beta = 0)
+// p = z + beta p with z = dinv r (jacobi) or z given; beta = rho_new/rho (first: beta = 0).  x_deferred (not jacobi):
+// also x += alpha p_old with alpha = rho/pAp from slot_pap; with r_or_z null ONLY that x update runs and p is left as is
 int launch_cg_pupdate(pde_ctx* c, const Grid& g, const OpDev& op, double* p, const double* r_or_z,
                       int slot_rho, int slot_rho_new, int first, int jacobi, double* x_deferred = nullptr, int slot_pap = 0);
 int launch_dot(pde_ctx* c, const Grid& g, int ncomp, const double* a, const double* b, int slot);

@@ -776,6 +776,16 @@ k_cg_pupdate_flat(double* __restrict__ p, const double* __restrict__ z, long lon
     for (int cidx = 0; cidx < ncomp; ++cidx) {
       double2* p2 = reinterpret_cast<double2*>(p + cidx * cs);
       double2* x2 = reinterpret_cast<double2*>(x + cidx * cs);
+      if (z == nullptr) {   // the converged iteration: x += alpha p alone, p is not needed any more
+        for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (long long)gridDim.x * blockDim.x) {
+          const double2 pv = p2[i];
+          double2 xv = x2[i];
+          xv.x = fma(alpha, pv.x, xv.x);
+          xv.y = fma(alpha, pv.y, xv.y);
+          x2[i] = xv;
+        }
+        continue;
+      }
       const double2* z2 = reinterpret_cast<const double2*>(z + cidx * cs);
       for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (long long)gridDim.x * blockDim.x) {
         const double2 zv = z2[i];

@@ -637,57 +637,100 @@ int PcgWork::alloc(pde_ctx* c, const Grid& g, int ncomp) {
 }
 void PcgWork::release() { p.release(); q.release(); }
 
+int mg_pcg(pde_ctx* c, const Grid& g, int ncomp, double* x, double* r, double* p, double* q, double bnorm2,
+           const double* rr0, const pde_solver_opts& o, pde_stats* st, const std::function<int()>& apply,
+           const std::function<int(int, double**)>& vcycle) {
+  OpDev flat;          // the flat vector kernels read nothing but the component count
+  flat.ncomp = ncomp;
+  const double tol2 = o.rtol * o.rtol * bnorm2;
+  double rr;
+  if (rr0) {
+    rr = *rr0;
+  } else {
+    PDE_OK(launch_dot(c, g, ncomp, r, r, S_RHO1));
+    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO1, 1));
+    PDE_OK(read_scal(c, S_RHO1, 1, &rr));
+  }
+  int it = 0;
+  bool conv = rr <= tol2;
+  if (!conv && o.max_iters > 0) {
+    double* z = nullptr;
+    PDE_OK(vcycle(S_RHO0, &z));
+    st->precond_applies++;
+    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO0, 1));
+    PDE_OK(launch_cg_pupdate(c, g, flat, p, z, S_RHO0, S_RHO0, 1, 0));
+    for (;;) {
+      const int sr = 2 * (it & 1), sn = 2 * (1 - (it & 1));
+      PDE_OK(apply());
+      PDE_OK(launch_cg_update(c, g, flat, nullptr, r, p, q, sr, S_XY, sn, sn + 1, 0));   // r -= alpha q, r.r
+      if (c->world > 1) PDE_OK(comm_allreduce_scal(c, sn + 1, 1));
+      ++it;
+      PDE_OK(read_scal(c, sn + 1, 1, &rr));
+      if (!(rr == rr)) PDE_FAIL("PCG broke down (NaN residual)");
+      conv = rr <= tol2;
+      if (conv || it >= o.max_iters) {
+        PDE_OK(launch_cg_pupdate(c, g, flat, p, nullptr, sr, sn, 0, 0, x, S_XY));   // x += alpha p
+        break;
+      }
+      PDE_OK(vcycle(sn, &z));
+      st->precond_applies++;
+      if (c->world > 1) PDE_OK(comm_allreduce_scal(c, sn, 1));
+      PDE_OK(launch_cg_pupdate(c, g, flat, p, z, sr, sn, 0, 0, x, S_XY));          // x += alpha p_old, p = z + beta p
+    }
+  }
+  st->iters_total += it;
+  st->final_relres = std::sqrt(rr / bnorm2);
+  if (!conv) st->converged = 0;
+  return 0;
+}
+
 int pcg_solve(pde_ctx* c, const Operator& A, Hierarchy* mg, PcgWork& w, double* x, double* r, double bnorm2,
-              const pde_solver_opts& o, pde_stats* st) {
+              const pde_solver_opts& o, pde_stats* st, const double* rr0) {
   const Grid& g = A.g;
   const int nc = A.dev.ncomp;
-  const bool gmg = mg != nullptr;
-  const double tol2 = o.rtol * o.rtol * bnorm2;
   st->solves += 1;
-  st->levels = gmg ? mg->levels() : 1;
+  st->levels = mg ? mg->levels() : 1;
   if (!(bnorm2 > 0.0)) {  // zero right-hand side: the initial guess (Dirichlet lift) is the solution
     st->final_relres = 0.0;
     return 0;
   }
-  double* z = nullptr;
-  double rr;
-  if (!gmg) {
-    CUDA_OK(cudaMemsetAsync(c->scal + S_XY, 0, 2 * sizeof(double), c->stream));
-    PDE_OK(launch_cg_update(c, g, A.dev, x, r, w.p.p, w.q.p, S_RHO0, S_XY, S_RHO0, S_RHO0 + 1, 1));
-    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO0, 2));
-    PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, r, S_RHO0, S_RHO0, 1, 1));
-  } else {
-    bool fused = false;
-    PDE_OK(mg->vcycle(c, A, r, &z, S_RHO0, &fused));
-    if (!fused) PDE_OK(launch_dot(c, g, nc, r, z, S_RHO0));
-    PDE_OK(launch_dot(c, g, nc, r, r, S_RHO0 + 1));
-    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO0, 2));
-    PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, z, S_RHO0, S_RHO0, 1, 0));
-  }
-  PDE_OK(read_scal(c, S_RHO0 + 1, 1, &rr));
-  int it = 0;
-  bool conv = rr <= tol2;
-  const int check = gmg ? 1 : (o.check_every > 0 ? o.check_every : 10);
-  while (!conv && it < o.max_iters) {
-    const int sr = 2 * (it & 1), sn = 2 * (1 - (it & 1));
+  // q = A p, p.q in S_XY
+  auto apply = [&]() -> int {
     StencilArgs a;
     a.x = w.p.p; a.y = w.q.p; a.reduce_slot_xy = S_XY;
     a.skip_yy = 1;   // only p.Ap is needed
     if (c->world > 1) PDE_OK(comm_halo_exchange(c, g, nc, w.p.p));
     PDE_OK(launch_stencil(c, g, A.bc, A.dev, a));
     if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_XY, 1));
-    // GMG path: x += alpha p is deferred to the p update below (p is read there anyway)
-    PDE_OK(launch_cg_update(c, g, A.dev, gmg ? nullptr : x, r, w.p.p, w.q.p, sr, S_XY, sn, sn + 1, !gmg));
-    // slots (sn, sn+1) = (r.z, r.r): Jacobi fills both in the update kernel; with multigrid r.z only exists after
-    // the V-cycle, so the two partial sums travel in ONE all-reduce there (r.r is only needed by the poll below)
-    if (c->world > 1 && !gmg) PDE_OK(comm_allreduce_scal(c, sn, 2));
-    if (gmg) {
+    return 0;
+  };
+  if (mg) {
+    // z = V(r); r.z from the last smoother sweep where it can fuse it
+    auto vcycle = [&](int slot, double** z) -> int {
       bool fused = false;
-      PDE_OK(mg->vcycle(c, A, r, &z, sn, &fused));
-      if (!fused) PDE_OK(launch_dot(c, g, nc, r, z, sn));
-      if (c->world > 1) PDE_OK(comm_allreduce_scal(c, sn, 2));
-    }
-    PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, gmg ? z : r, sr, sn, 0, !gmg, gmg ? x : nullptr, S_XY));
+      PDE_OK(mg->vcycle(c, A, r, z, slot, &fused));
+      if (!fused) PDE_OK(launch_dot(c, g, nc, r, *z, slot));
+      return 0;
+    };
+    return mg_pcg(c, g, nc, x, r, w.p.p, w.q.p, bnorm2, rr0, o, st, apply, vcycle);
+  }
+  const double tol2 = o.rtol * o.rtol * bnorm2;
+  double rr;
+  CUDA_OK(cudaMemsetAsync(c->scal + S_XY, 0, 2 * sizeof(double), c->stream));
+  PDE_OK(launch_cg_update(c, g, A.dev, x, r, w.p.p, w.q.p, S_RHO0, S_XY, S_RHO0, S_RHO0 + 1, 1));
+  if (c->world > 1) PDE_OK(comm_allreduce_scal(c, S_RHO0, 2));
+  PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, r, S_RHO0, S_RHO0, 1, 1));
+  PDE_OK(read_scal(c, S_RHO0 + 1, 1, &rr));
+  int it = 0;
+  bool conv = rr <= tol2;
+  const int check = o.check_every > 0 ? o.check_every : 10;
+  while (!conv && it < o.max_iters) {
+    const int sr = 2 * (it & 1), sn = 2 * (1 - (it & 1));
+    PDE_OK(apply());
+    // slots (sn, sn+1) = (r.z, r.r), both from the update kernel
+    PDE_OK(launch_cg_update(c, g, A.dev, x, r, w.p.p, w.q.p, sr, S_XY, sn, sn + 1, 1));
+    if (c->world > 1) PDE_OK(comm_allreduce_scal(c, sn, 2));
+    PDE_OK(launch_cg_pupdate(c, g, A.dev, w.p.p, r, sr, sn, 0, 1));
     ++it;
     if (it % check == 0 || it >= o.max_iters) {
       PDE_OK(read_scal(c, sn + 1, 1, &rr));

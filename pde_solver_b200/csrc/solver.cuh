@@ -1,5 +1,6 @@
 // Solver-layer objects: device fields, operators, multigrid hierarchy, PCG.
 #pragma once
+#include <functional>
 #include <memory>
 
 #include "device.cuh"
@@ -86,9 +87,19 @@ struct PcgWork {
 };
 
 // Solves A x = b given x (initial guess incl. Dirichlet values) and r = masked(b - A x).
-// bnorm2 = ||b||^2 for the stopping rule ||r|| <= rtol ||b||.
+// bnorm2 = ||b||^2 for the stopping rule ||r|| <= rtol ||b||.  rr0: r.r over all ranks when the caller's
+// right-hand-side pass has already formed it (multigrid only; null: computed here).
 int pcg_solve(pde_ctx* c, const Operator& A, Hierarchy* mg, PcgWork& w, double* x, double* r, double bnorm2,
-              const pde_solver_opts& o, pde_stats* st);
+              const pde_solver_opts& o, pde_stats* st, const double* rr0 = nullptr);
+
+// The GMG-PCG loop of pcg_solve and wmg_pcg, in the order of oracle/gmg_model.pcg: r -= alpha q is followed by the
+// convergence poll, and only an iteration that goes on runs the V-cycle, so a solve of k iterations runs k V-cycles.
+// The x update of an iteration rides on its p update (x += alpha p_old, p = z + beta p); the last iteration runs it
+// alone.  apply(): q = A p with p.q in S_XY (all-reduced); vcycle(slot, &z): z = V(r) with this rank's r.z in slot.
+// rr0 as in pcg_solve.  p, q: work vectors of g.
+int mg_pcg(pde_ctx* c, const Grid& g, int ncomp, double* x, double* r, double* p, double* q, double bnorm2,
+           const double* rr0, const pde_solver_opts& o, pde_stats* st, const std::function<int()>& apply,
+           const std::function<int(int, double**)>& vcycle);
 
 int project_trig_ic(pde_ctx* c, const Grid& g, const BcDev& bc, int dim, const int32_t n_user[3], const double L_user[3],
                     const double* lo_user, double amp, double kw, int use_sin, const pde_solver_opts& o, double* u,

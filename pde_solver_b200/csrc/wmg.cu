@@ -396,42 +396,17 @@ int wvcycle(pde_ctx* c, WHierarchy& H, const double* b0, double** z_out, int dot
   return 0;
 }
 
-// The recurrence of pcg_solve (GMG branch): device scalars, the x update deferred into the p update, a poll per
-// iteration.  The flat vector kernels only use ncomp from the operator description.
+// The GMG-PCG loop of pcg_solve (mg_pcg) with this hierarchy's level-0 operator and V-cycle (one GPU only)
 int wmg_pcg(pde_ctx* c, WHierarchy& h, double* x, double* r, double* p, double* q, double bnorm2,
             const pde_solver_opts& o, pde_stats* st) {
   if (h.levels() < 2) PDE_FAIL("weighted multigrid needs at least two levels");
   WLevel& L0 = *h.lv[0];
-  const Grid& g = L0.g;
-  OpDev one;
-  one.ncomp = 1;
   st->solves += 1;
   st->levels = h.levels();
   if (!(bnorm2 > 0.0)) { st->final_relres = 0.0; return 0; }
-  const double tol2 = o.rtol * o.rtol * bnorm2;
-  double* z = nullptr;
-  PDE_OK(wvcycle(c, h, r, &z, S_RHO0));
-  PDE_OK(launch_dot(c, g, 1, r, r, S_RHO0 + 1));
-  PDE_OK(launch_cg_pupdate(c, g, one, p, z, S_RHO0, S_RHO0, 1, 0));
-  double rr;
-  PDE_OK(read_scal(c, S_RHO0 + 1, 1, &rr));
-  int it = 0;
-  bool conv = rr <= tol2;
-  while (!conv && it < o.max_iters) {
-    const int sr = 2 * (it & 1), sn = 2 * (1 - (it & 1));
-    PDE_OK(wsweep(c, L0, h.bc, W_APPLY, p, nullptr, nullptr, q, 0.0, 0.0, S_XY));     // q = A p, p.q
-    PDE_OK(launch_cg_update(c, g, one, nullptr, r, p, q, sr, S_XY, sn, sn + 1, 0));  // r -= a q, r.r
-    PDE_OK(wvcycle(c, h, r, &z, sn));                                                // z = V(r), r.z
-    PDE_OK(launch_cg_pupdate(c, g, one, p, z, sr, sn, 0, 0, x, S_XY));               // x += a p, p = z + b p
-    ++it;
-    PDE_OK(read_scal(c, sn + 1, 1, &rr));
-    if (!(rr == rr)) PDE_FAIL("weighted GMG-PCG broke down (NaN residual)");
-    conv = rr <= tol2;
-  }
-  st->iters_total += it;
-  st->final_relres = std::sqrt(rr / bnorm2);
-  if (!conv) st->converged = 0;
-  return 0;
+  auto apply = [&]() { return wsweep(c, L0, h.bc, W_APPLY, p, nullptr, nullptr, q, 0.0, 0.0, S_XY); };   // q = A p, p.q
+  auto vcycle = [&](int slot, double** z) { return wvcycle(c, h, r, z, slot); };                          // z = V(r), r.z
+  return mg_pcg(c, L0.g, 1, x, r, p, q, bnorm2, nullptr, o, st, apply, vcycle);
 }
 
 int wmg_level_coefs(pde_ctx* c, const WHierarchy& h, int level, double* out) {
